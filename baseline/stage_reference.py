@@ -1,6 +1,6 @@
 """Stage the reference's model files next to the repo so that they can travel to the GPU box.
 
-    python baseline/stage_reference.py            # /root/reference -> baseline/_ref/
+    python baseline/stage_reference.py [CHECKOUT]  # CHECKOUT (default $PO2_REFERENCE) -> baseline/_ref/
 
 The reference (mschoenb97/po2_quantization) is a flat script repo without setup.py / pyproject, so
 `pip install --target baseline/_ref /root/reference` has nothing to install; what the GPU-side tests and
@@ -8,7 +8,7 @@ The reference (mschoenb97/po2_quantization) is a flat script repo without setup.
 MobileNetV2, MobileViT, the factory, the reference QuantizedConv2d) and `utils/quantizers.py`.  They are
 copied verbatim into baseline/_ref/ (git-ignored: reference sources never enter this repo's history;
 not gpurun-ignored: the directory ships with the snapshot like the built .so).  Nothing is edited.
-`__graft_entry__.build()` runs this when /root/reference is present.
+`__graft_entry__.build()` runs this; without a checkout it stages nothing.
 """
 import filecmp
 import os
@@ -21,10 +21,11 @@ FILES = ["models/__init__.py", "models/model.py", "models/resnet.py", "models/mo
          "models/quantized_conv.py", "utils/__init__.py", "utils/quantizers.py"]
 
 
-def stage(src: str = "/root/reference", verbose: bool = True) -> bool:
-    if not os.path.isdir(os.path.join(src, "models")):
+def stage(src: str = None, verbose: bool = True) -> bool:
+    src = src or os.environ.get("PO2_REFERENCE")
+    if not src or not os.path.isdir(os.path.join(src, "models")):
         if verbose:
-            print(f"[stage_reference] {src} not present: nothing staged")
+            print(f"[stage_reference] no reference checkout ({src or '$PO2_REFERENCE unset'}): nothing staged")
         return False
     n = 0
     for rel in FILES:
@@ -39,4 +40,4 @@ def stage(src: str = "/root/reference", verbose: bool = True) -> bool:
 
 
 if __name__ == "__main__":
-    stage(sys.argv[1] if len(sys.argv) > 1 else "/root/reference")
+    stage(sys.argv[1] if len(sys.argv) > 1 else None)

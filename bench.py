@@ -4,6 +4,7 @@ PO2 4-bit QAT forward + STE backward + SGD, batch 128 per GPU) and quantizer GB/
 
     python bench.py --gpus N --steps K --warmup W            # our arm (N>1 under torchrun)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as DIR/*.npy
 
 One JSON line on rank 0.
   value      whole-job images/s of the QAT step with inputs resident in HBM (CUDA-graph replay)
@@ -30,6 +31,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 import torch.nn as nn
 
@@ -296,6 +298,31 @@ class StepHarness:
         torch.cuda.empty_cache()
 
 
+DUMP_LIMIT_BYTES = 64 * 2 ** 20
+
+
+def step_outputs(model, loss_buf):
+    """What a training step leaves its caller: the loss of the last step, the parameters after its SGD update and
+    the norms' running statistics (floating-point tensors only; the integer batch counters are left out)."""
+    out = {"loss": loss_buf.detach().float().cpu().numpy()}
+    with torch.no_grad():
+        for name, t in list(model.named_parameters()) + list(model.named_buffers()):
+            if t.is_floating_point():
+                out[name] = t.detach().float().cpu().numpy()
+    return out
+
+
+def dump_outputs(arrays, directory):
+    """Write each array as <directory>/<name>.npy (float32), so that two builds run with the same arguments
+    (hence the same seeded inputs) can be compared output for output."""
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: outputs of {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte dump limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), v)
+
+
 def run_ours(a):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -434,6 +461,7 @@ def _run_ours_on_stream(a, ops, world, rank, local_rank, device):
     timeouts = _exchange_timeouts()
     if rank != 0:
         return
+    outputs = step_outputs(h.model, h.loss_buf) if a.dump_outputs else None
     mode = ops.get_conv_mode()
     ms_step = ms_total / a.steps
     out = {
@@ -483,6 +511,8 @@ def _run_ours_on_stream(a, ops, world, rank, local_rank, device):
         if not a.no_cpu_baseline:
             out["cpu_baseline"] = cpu_baseline(B, steps=2)
     print(json.dumps(out), flush=True)
+    if outputs is not None:
+        dump_outputs(outputs, a.dump_outputs)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -551,7 +581,7 @@ def _reference_training_step(device, batch, seed_rank=0):
         loss.backward()
         opt.step()
         loss_buf.copy_(loss.detach())
-    return step, loss_buf, kind, what
+    return step, loss_buf, kind, what, model
 
 
 def _time_loop(fn, iters):
@@ -570,7 +600,7 @@ def gpu_oracle_step(a, device, ms_main):
     quantizer ops, cuDNN convolutions (allow_tf32 at torch's default, True), stock BatchNorm -- eager (how
     train.py runs it) and CUDA-graph captured (launch overhead removed: the strongest same-box baseline)."""
     try:
-        step, loss_buf, kind, what = _reference_training_step(device, a.batch)
+        step, loss_buf, kind, what, _ = _reference_training_step(device, a.batch)
         for _ in range(5):
             step()
         iters = min(a.steps, 10)
@@ -910,12 +940,11 @@ def cpu_training_step_fn(batch):
     """The reference's training step on host cores: the one place bench.py executes the oracle / the
     staged reference files (as the baseline being timed, never as the product)."""
     torch.set_num_threads(os.cpu_count() or 1)
-    step, loss_buf, kind, what = _reference_training_step(torch.device("cpu"), batch)
-    return step, loss_buf, kind, what
+    return _reference_training_step(torch.device("cpu"), batch)
 
 
 def cpu_baseline(batch, steps=2):
-    step, loss_buf, kind, what = cpu_training_step_fn(batch)
+    step, loss_buf, kind, what, _ = cpu_training_step_fn(batch)
     step(); step()                          # first step: oneDNN primitive creation, thread-pool start-up
     t0 = time.perf_counter()
     for _ in range(steps):
@@ -931,31 +960,23 @@ def run_reference(a):
     """--impl reference: the reference's own CPU implementation of the step on all host threads -- the
     unmodified reference files when baseline/_ref is staged, else the oracle's op-for-op torch port
     (pinned bit-exactly to the reference by tests/test_oracle_golden.py).  Same batch, same warm-up
-    count and same config keys as our arm; only the NUMBER of timed steps is bounded (and reported) so
-    that a slow host still finishes within minutes."""
+    count, same number of timed steps and same config keys as our arm."""
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if rank != 0:
         return
     B = a.batch
-    step, loss_buf, kind, what = cpu_training_step_fn(B)
+    step, loss_buf, kind, what, model = cpu_training_step_fn(B)
     warm = max(a.warmup, 3)
-    step()                                   # cold step (library initialisation), never timed or probed
-    t0 = time.perf_counter()
-    step()
-    probe = time.perf_counter() - t0         # the SECOND step is the probe
-    budget = 240.0
-    steps = max(1, min(a.steps, int((budget - probe * warm) / max(probe, 1e-3))))
-    for _ in range(max(0, warm - 2)):
+    for _ in range(warm):                    # the first one initialises the libraries
         step()
+    steps = a.steps
     t0 = time.perf_counter()
     for _ in range(steps):
         step()
     dt = time.perf_counter() - t0
     v = B * steps / dt
-    sample = (f"{steps} training steps at the full batch {B} after {warm} warm-up steps" +
-              ("" if steps == a.steps else f" (fewer than the requested {a.steps}: a step takes {probe:.1f} s on this host)") +
-              f"; {what}")
+    sample = f"{steps} training steps at the full batch {B} after {warm} warm-up steps; {what}"
     out = {"impl": "reference", "metric": METRIC, "value": v, "unit": "images/s", "n_gpus": world,
            "steps": steps, "warmup": warm, "ms_per_step": dt / steps * 1e3, "higher_is_better": True,
            "scaling": "weak", "vs_baseline": None, "dtype": "f32 (torch CPU kernels)",
@@ -970,6 +991,8 @@ def run_reference(a):
            "e2e": {"value": v, "unit": "images/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
            "gpu_launches": 0}
     print(json.dumps(out), flush=True)
+    if a.dump_outputs:
+        dump_outputs(step_outputs(model, loss_buf), a.dump_outputs)
 
 
 def main():
@@ -988,7 +1011,12 @@ def main():
     ap.add_argument("--torch-profile", default=None, help="write a torch.profiler kernel table of eager steps and exit")
     ap.add_argument("--graph-timeline", default=None, help="write the device timeline of graph replays (torch.profiler) and exit")
     ap.add_argument("--profile-step", action="store_true", help="run one eager step inside cudaProfilerStart/Stop and exit")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the loss of the last step and the model's parameters and running "
+                         "statistics after it as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.impl == "reference":
         run_reference(a)
     else:

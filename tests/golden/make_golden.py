@@ -1,6 +1,6 @@
 """Generate golden input/output vectors from the UNMODIFIED reference (run in the build container).
 
-    python tests/golden/make_golden.py          # needs /root/reference; writes tests/golden/*.npz
+    PO2_REFERENCE=<checkout> python tests/golden/make_golden.py      # writes tests/golden/*.npz
 
 The reference is Python and cannot travel to the GPU box, so its outputs on seeded inputs are
 committed as fixtures.  Tensors are stored as raw bit patterns (uint32 for fp32, uint16 for
@@ -12,7 +12,7 @@ import sys
 import numpy as np
 import torch
 
-REF = os.environ.get("PO2_REFERENCE", "/root/reference")
+REF = os.environ.get("PO2_REFERENCE") or sys.exit("make_golden.py: set PO2_REFERENCE to a checkout of the reference")
 sys.path.insert(0, REF)
 from utils.quantizers import (PowerOfTwoPlusQuantizer, PowerOfTwoQuantizer,  # noqa: E402
                               LinearPowerOfTwoQuantizer, LinearPowerOfTwoPlusQuantizer,
@@ -55,6 +55,22 @@ def boundary_inputs(plus: bool, scale: float) -> torch.Tensor:
     x = torch.cat([x * sgn, s.reshape(1)])       # plant the max so that scale == s
     assert torch.max(torch.abs(x)).item() == s.item()
     return x
+
+
+def save_quantizer_cases(path, cases):
+    """{"<case>|x": bits, "<case>|y": bits} -> the layout tests/golden_util.quantizer_cases() reads: each distinct
+    input once, flattened and stored as differences of consecutive bit patterns (the file stays under 1 MB)."""
+    keys = sorted(k[:-2] for k in cases if k.endswith("|x"))
+    inputs, index, out = {}, [], {}
+    for k in keys:
+        x = cases[k + "|x"]
+        i = inputs.setdefault((x.dtype.str, x.shape, x.tobytes()), len(inputs))
+        if f"input|{i}" not in out:
+            f = x.ravel()
+            out[f"input|{i}"] = np.diff(f, prepend=f.dtype.type(0)).astype(f.dtype)
+        index.append(i)
+        out[k + "|y"] = cases[k + "|y"]
+    np.savez_compressed(path, cases=np.array(keys), input_of_case=np.array(index, dtype=np.int32), **out)
 
 
 def main():
@@ -102,7 +118,7 @@ def main():
             y = qc.forward(None, x, bits=4, fsr=fsr)
             cases[f"fsr{fsr}|f32|{qn}|4|x"] = bits_of(x)
             cases[f"fsr{fsr}|f32|{qn}|4|y"] = bits_of(y)
-    np.savez_compressed(os.path.join(HERE, "quantizer_golden.npz"), **cases)
+    save_quantizer_cases(os.path.join(HERE, "quantizer_golden.npz"), cases)
     print("quantizer cases:", len(cases) // 2)
 
     # statistical known answer (SURVEY.md section 4): po2 -> po2+ MSE change on randn(2^20)

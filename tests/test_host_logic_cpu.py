@@ -187,7 +187,7 @@ def test_reference_file_loader_variants():
     import sys
     from workloads import reference_files as RF
     if RF.find_reference() is None:
-        pytest.skip("no reference checkout (baseline/_ref or /root/reference)")
+        pytest.skip("no reference checkout ($PO2_REFERENCE or baseline/_ref)")
     d, s = RF.load("dropin"), RF.load("stock")
     assert d.QuantizedConv2d is P.QuantizedConv2d and s.QuantizedConv2d is not P.QuantizedConv2d
     assert d.quantizers.quantizer_dict["po2+"] is P.PowerOfTwoPlusQuantizer

@@ -104,7 +104,7 @@ def _ref_ns():
     from workloads import reference_files as RF
     d, s = RF.load("dropin"), RF.load("stock")
     if d is None or s is None:
-        pytest.skip("no reference checkout staged (baseline/_ref; run baseline/stage_reference.py in the build container)")
+        pytest.skip("no reference checkout ($PO2_REFERENCE or baseline/_ref)")
     return RF, d, s
 
 
@@ -379,7 +379,7 @@ def test_fuse_batchnorm_on_the_reference_model_files():
     from workloads import reference_files as RF
     ns = RF.load("dropin")
     if ns is None:
-        pytest.skip("no reference checkout (baseline/_ref)")
+        pytest.skip("no reference checkout ($PO2_REFERENCE or baseline/_ref)")
     torch.manual_seed(5)
     a = ns.get_model("resnet20", 10, P.PowerOfTwoQuantizer, 4, (32, 32)).cuda().train()
     b = copy.deepcopy(a)

@@ -1,6 +1,5 @@
-"""Import the reference's OWN model files, unmodified, from wherever a checkout is available:
-$PO2_REFERENCE, baseline/_ref/ (staged by baseline/stage_reference.py; ships to the GPU box) or
-/root/reference (the build container).
+"""Import the reference's OWN model files, unmodified, from a checkout named by $PO2_REFERENCE or staged
+into baseline/_ref/ by baseline/stage_reference.py.  The repository does not contain them.
 
 Two variants of the same files:
   * ``load("dropin")`` -- `models.quantized_conv` and `utils.quantizers` replaced by this repo's drop-in
@@ -23,7 +22,7 @@ _cache = {}
 
 
 def find_reference():
-    for p in (os.environ.get("PO2_REFERENCE"), os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
+    for p in (os.environ.get("PO2_REFERENCE"), os.path.join(ROOT, "baseline", "_ref")):
         if p and os.path.isfile(os.path.join(p, "models", "model.py")) and os.path.isfile(os.path.join(p, "utils", "quantizers.py")):
             return p
     return None
