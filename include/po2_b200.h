@@ -253,6 +253,33 @@ int po2_lin_max_channel_elems(void);
 int po2_lin_quantize(const void* w, void* y, int K, int C, int RS, int bits, int num_iters, int plus, int flavor,
                      void* stream);
 
+/* lin / lin+ weights on the tensor-core conv: after num_iters >= 1 rounds every weight is n * 2^k (one power-of-two
+ * step per input channel, |n| <= 2^(bits-1) - 1), which is exact as a bf16 operand for bits <= 9 (compute 0) and as
+ * a tf32 operand for bits <= 12 (compute 2).  So the packed operand holds y itself and every consumer of
+ * (packed, scale) -- po2_conv2d_fwd_packed(_ep / _stats), po2_conv2d_dgrad_packed, po2_conv2d_dgrad -- takes it with a
+ * scale of 1.0f.
+ * po2_lin_quantize_pack: po2_lin_quantize (y_out bit-identical) that also writes the operand of conv2d(x of shape
+ * (B, C, H, W), y) into `packed` (po2_conv2d_pack_bytes bytes) and, if packed_dgrad != NULL, the data-gradient operand
+ * (po2_conv2d_dgrad_pack_bytes bytes; stride-1 dense layers).  One launch; two (quantizer + po2_conv2d_pack) when the
+ * operand needs channel padding.  PO2_E_UNSUPPORTED: no tensor-core operand for this geometry / compute, bits not
+ * exact in it, num_iters < 1, or a channel above po2_lin_max_channel_elems().
+ * Multi-tensor form: ONE launch for many lin weights, one CTA per (tensor, input channel).  po2_lin_multi_desc_fill
+ * writes entry `index` of a HOST table of po2_lin_multi_desc_bytes()-sized entries (same arguments as
+ * po2_lin_quantize_pack; fill in index order 0, 1, ...) and returns the tensor's CTA count C (> 0), or
+ * PO2_E_UNSUPPORTED when the layer must take po2_lin_quantize_pack (channel padding).  The caller copies the table
+ * to the device once and calls po2_lin_quantize_pack_multi with total_ctas = the sum of the returned counts and
+ * max_channel_elems = the largest K*R*S of the table. */
+int po2_lin_quantize_pack(const void* w, void* y_out, void* packed, size_t packed_bytes, void* packed_dgrad,
+                          size_t packed_dgrad_bytes, int B, int C, int H, int W, int K, int R, int S, int stride, int pad,
+                          int groups, int bits, int num_iters, int plus, int flavor, int compute, void* stream);
+size_t po2_lin_multi_desc_bytes(void);
+int po2_lin_multi_desc_fill(void* host_table, int index, const void* w, void* y_out, void* packed, size_t packed_bytes,
+                            void* packed_dgrad, size_t packed_dgrad_bytes, int B, int C, int H, int W, int K, int R,
+                            int S, int stride, int pad, int groups, int bits, int num_iters, int plus, int flavor,
+                            int compute);
+int po2_lin_quantize_pack_multi(const void* device_table, int ntensors, int total_ctas, int max_channel_elems,
+                                void* stream);
+
 /* ---- batch normalisation around the quantized convs (SURVEY.md section 8f "next" #3) -----------------
  * The reference models follow every QuantizedConv2d with nn.SyncBatchNorm (+ ReLU, + the residual add):
  * models/resnet.py:38-61, models/mobilenet.py:29-33.  x, y, dy, dx are fp32 [B][C][HW] (NCHW), parameters

@@ -66,6 +66,10 @@ SIGNATURES = {
     "po2_conv2d_wgrad": (_i, [_vp, _vp, _vp] + [_i] * 11 + [_vp, _sz, _vp]),
     "po2_lin_max_channel_elems": (_i, []),
     "po2_lin_quantize": (_i, [_vp, _vp] + [_i] * 7 + [_vp]),
+    "po2_lin_quantize_pack": (_i, [_vp, _vp, _vp, _sz, _vp, _sz] + [_i] * 15 + [_vp]),
+    "po2_lin_multi_desc_bytes": (_sz, []),
+    "po2_lin_multi_desc_fill": (_i, [_vp, _i, _vp, _vp, _vp, _sz, _vp, _sz] + [_i] * 15),
+    "po2_lin_quantize_pack_multi": (_i, [_vp, _i, _i, _i, _vp]),
     "po2_bn_workspace_bytes": (_sz, [_i]),
     "po2_bn_mailbox_bytes": (_sz, []),
     "po2_bn_stats": (_i, [_vp, _i, _i, _i, _vp, _vp, _sz, _vp, _i, _i, _vp]),

@@ -28,6 +28,7 @@ import torch
 
 from . import ops
 from .quantized_conv import QuantizedConv2d
+from .quantizers import quantizer_family
 
 FORMAT = "po2-packed-v1"
 
@@ -38,12 +39,13 @@ def _qconv_weight_names(model: torch.nn.Module) -> Dict[str, QuantizedConv2d]:
 
 def _layer_quantizer(m: QuantizedConv2d, quantizer, bits):
     """(bits, plus) this layer's weight is quantized with, or None if it is a full-precision layer"""
+    # lin / lin+ weights have no PO2 codes: stored as fp32 (their PTQ tag is _po2_lin_ptq, not read here)
     if quantizer is not None:
-        plus = getattr(quantizer, "_PLUS", None)
-        return (int(bits), bool(plus)) if plus is not None else None
+        fam = quantizer_family(quantizer)
+        return (int(bits), fam[1]) if fam is not None and fam[0] == "po2" else None
     if m.quantize_fn is not None:
-        plus = getattr(m.quantize_fn, "_PLUS", None)
-        return (int(m.bits), bool(plus)) if plus is not None else None
+        fam = quantizer_family(m.quantize_fn)
+        return (int(m.bits), fam[1]) if fam is not None and fam[0] == "po2" else None
     tag = m.__dict__.get("_po2_ptq")
     if tag is not None and tag[0] == m.weight._version and len(tag) >= 4:
         return int(tag[2]), bool(tag[3])

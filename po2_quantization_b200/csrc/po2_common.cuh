@@ -121,6 +121,31 @@ struct PackArgs {
   FastDiv div_nt2;
 };
 
+// The packed layout in one place: store r, the operand value of weight element (k, c, tap) of a (K, C, taps) tensor,
+// into Bp (and, when on, its data-gradient twin Bp2).  r must be exact in the operand type (bf16 / tf32).
+__device__ __forceinline__ void pack_store(const PackArgs& pk, int k, int c, int tap, float r) {
+  const int nt = fdiv(k, pk.div_nt);
+  const int n = k - nt * pk.NT;
+  const int cg = pk.G == 8 ? (c >> 3) : (c >> 2), cj = c & (pk.G - 1);
+  const size_t idx = pk.tapminor
+      ? (((((size_t)nt * 3 + tap / 3) * pk.ncg + cg) * 3 + tap % 3) * pk.NT + n) * pk.G + cj
+      : ((((size_t)nt * pk.taps + tap) * pk.ncg + cg) * pk.NT + n) * pk.G + cj;
+  if (pk.G == 8) reinterpret_cast<__nv_bfloat16*>(pk.Bp)[idx] = __float2bfloat16_rn(r);
+  else reinterpret_cast<float*>(pk.Bp)[idx] = r;
+  if (pk.Bp2) {
+    // data-gradient operand: out channel = c, in channel = k, tap rotated (csrc/po2_conv.cu, transpose)
+    const int tap2 = pk.taps - 1 - tap;
+    const int nt2 = fdiv(c, pk.div_nt2);
+    const int n2 = c - nt2 * pk.NT2;
+    const int cg2 = pk.G == 8 ? (k >> 3) : (k >> 2), cj2 = k & (pk.G - 1);
+    const size_t idx2 = pk.tapminor2
+        ? (((((size_t)nt2 * 3 + tap2 / 3) * pk.ncg2 + cg2) * 3 + tap2 % 3) * pk.NT2 + n2) * pk.G + cj2
+        : ((((size_t)nt2 * pk.taps + tap2) * pk.ncg2 + cg2) * pk.NT2 + n2) * pk.G + cj2;
+    if (pk.G == 8) reinterpret_cast<__nv_bfloat16*>(pk.Bp2)[idx2] = __float2bfloat16_rn(r);
+    else reinterpret_cast<float*>(pk.Bp2)[idx2] = r;
+  }
+}
+
 // quantize w (fp32, n = K*C*taps elements) into y + scale AND the packed operand, one launch
 int fused_quantize_pack(const void* w, void* y, float* scale_out, int64_t n, int bits, int fsr, int mode,
                         int flavor, void* workspace, const PackArgs& pk, cudaStream_t st);
@@ -136,6 +161,18 @@ struct MultiDesc {
 int multi_fused_capacity();
 int multi_fused_launch(const MultiDesc* descs_dev, int ntensors, int csize, cudaStream_t st);
 int check_quant_args(int bits, int fsr, int mode, int flavor);
+
+// csrc/po2_lin.cu: lin / lin+ quantizer with optional operand emission.  A lin weight is n * 2^k (|n| <= 2^(bits-1) - 1,
+// one power-of-two step per input channel), so the packed operand holds y itself (the conv's scale is 1.0).
+struct LinDesc {             // one tensor of the multi-tensor launch
+  const float* w; float* y;
+  int K, C, RS, bits, iters, plus, flavor;
+  int cta0;                  // first CTA of this tensor: the tensors' CTAs are consecutive, one per input channel
+  PackArgs pk;
+};
+int lin_check_args(int K, int C, int RS, int bits, int num_iters, int flavor);
+int lin_launch(const float* w, float* y, int K, int C, int RS, int bits, int iters, int plus, int flavor,
+               const PackArgs& pk, cudaStream_t st);
 
 // ---- optional conv epilogue: eval-mode BatchNorm folded into the conv (per-out-channel affine), the residual add
 // and the activation of the block -- y = act(conv * a[k] + b[k] + res) -- models/resnet.py:55-71 at inference.

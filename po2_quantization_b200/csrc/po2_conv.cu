@@ -1743,6 +1743,83 @@ int po2_multi_desc_fill_dgrad(void* host_table, int index, void* packed_dgrad, s
   return 0;
 }
 
+// ---- lin / lin+ weights on the tensor-core kernels ----------------------------------------------------------------
+// A lin weight is n * 2^k per input channel, |n| <= 2^(bits-1) - 1: exact as a bf16 operand for bits <= 9 and as a
+// tf32 operand for bits <= 12, so the packed operand holds y itself and the conv runs with scale = 1.0.  The
+// quantizer kernel writes it (and the stride-1 data-gradient operand) from the CTA that owns the input channel.
+// Fills pk for conv2d(x of shape (B, C, H, W), w (K, C/groups, R, S)); PO2_E_UNSUPPORTED when the geometry has no
+// tensor-core operand, needs channel padding (the per-channel emitter writes no padding) or bits is not exact.
+static int lin_pack_args(PackArgs& pk, ConvGeom& g, void* packed, size_t packed_bytes, void* packed_dgrad,
+                         size_t dgrad_bytes, int B, int C, int H, int W, int K, int R, int S, int stride, int pad,
+                         int groups, int bits, int num_iters, int compute) {
+  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
+  if (compute == 1 || !umma_eligible(g) || !plan_umma(g, compute == 2)) return PO2_E_UNSUPPORTED;
+  if (num_iters < 1 || bits > (g.tf32 ? 12 : 9)) return PO2_E_UNSUPPORTED;      // step not a power of two / not exact
+  if (packed_bytes < umma_pack_bytes(g)) return PO2_E_WORKSPACE;
+  pk = PackArgs{};
+  pk.Bp = packed;
+  pk.G = g.G; pk.C = C; pk.K = K; pk.taps = g.ntaps; pk.NT = g.NT; pk.ncg = C / g.G; pk.tapminor = g.tapminor;
+  pk.div_ct = make_fastdiv((uint32_t)(C * g.ntaps));
+  pk.div_t = make_fastdiv((uint32_t)g.ntaps);
+  pk.div_nt = make_fastdiv((uint32_t)g.NT);
+  if (packed_dgrad) {
+    ConvGeom gd;
+    if (stride != 1 || groups != 1 || !dgrad_geom(gd, B, C, H, W, K, R, S, pad, compute)) return PO2_E_UNSUPPORTED;
+    if (!(gd.Cpad == K && gd.ntiles_n * gd.NT == C) || gd.G != g.G || gd.ntaps != g.ntaps) return PO2_E_UNSUPPORTED;
+    if (dgrad_bytes < umma_pack_bytes(gd)) return PO2_E_WORKSPACE;
+    pk.Bp2 = packed_dgrad;
+    pk.NT2 = gd.NT; pk.ncg2 = K / gd.G; pk.tapminor2 = gd.tapminor;
+    pk.div_nt2 = make_fastdiv((uint32_t)gd.NT);
+  }
+  return 0;
+}
+
+// y = lin(w) and the packed operand(s) of conv2d(x of shape (B, C, H, W), y): one launch, or two (quantizer + pack)
+// when the operand needs channel padding.
+int po2_lin_quantize_pack(const void* w, void* y_out, void* packed, size_t packed_bytes, void* packed_dgrad,
+                          size_t packed_dgrad_bytes, int B, int C, int H, int W, int K, int R, int S, int stride, int pad,
+                          int groups, int bits, int num_iters, int plus, int flavor, int compute, void* stream) {
+  if (!w || !y_out || !packed) return PO2_E_NULL;
+  const int Cg = groups > 0 ? C / groups : 0;
+  if (int e = lin_check_args(K, Cg, R * S, bits, num_iters, flavor)) return e;
+  PackArgs pk;
+  ConvGeom g;
+  if (int e = lin_pack_args(pk, g, packed, packed_bytes, packed_dgrad, packed_dgrad_bytes, B, C, H, W, K, R, S, stride,
+                            pad, groups, bits, num_iters, compute)) return e;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (g.Cpad == C && g.ntiles_n * g.NT == K)
+    return lin_launch((const float*)w, (float*)y_out, K, C, R * S, bits, num_iters, plus, flavor, pk, st);
+  if (packed_dgrad) return PO2_E_UNSUPPORTED;
+  if (int e = lin_launch((const float*)w, (float*)y_out, K, Cg, R * S, bits, num_iters, plus, flavor, PackArgs{}, st))
+    return e;
+  return po2_conv2d_pack(y_out, nullptr, packed, packed_bytes, B, C, H, W, K, R, S, stride, pad, groups, PO2_W_F32_PO2,
+                         bits, 1, compute, stream);
+}
+
+// entry `index` of a LinDesc table (host memory, filled in index order 0, 1, ...: the entry starts its CTAs behind
+// those of entry index - 1).  Returns this tensor's CTA count (C) or a PO2_E_* code.
+int po2_lin_multi_desc_fill(void* host_table, int index, const void* w, void* y_out, void* packed, size_t packed_bytes,
+                            void* packed_dgrad, size_t packed_dgrad_bytes, int B, int C, int H, int W, int K, int R,
+                            int S, int stride, int pad, int groups, int bits, int num_iters, int plus, int flavor,
+                            int compute) {
+  if (!host_table || index < 0 || !w || !y_out || !packed) return PO2_E_NULL;
+  const int Cg = groups > 0 ? C / groups : 0;
+  if (int e = lin_check_args(K, Cg, R * S, bits, num_iters, flavor)) return e;
+  PackArgs pk;
+  ConvGeom g;
+  if (int e = lin_pack_args(pk, g, packed, packed_bytes, packed_dgrad, packed_dgrad_bytes, B, C, H, W, K, R, S, stride,
+                            pad, groups, bits, num_iters, compute)) return e;
+  if (!(g.Cpad == C && g.ntiles_n * g.NT == K)) return PO2_E_UNSUPPORTED;
+  LinDesc* t = reinterpret_cast<LinDesc*>(host_table);
+  LinDesc d = {};
+  d.w = (const float*)w; d.y = (float*)y_out;
+  d.K = K; d.C = C; d.RS = R * S; d.bits = bits; d.iters = num_iters; d.plus = plus; d.flavor = flavor;
+  d.cta0 = index == 0 ? 0 : t[index - 1].cta0 + t[index - 1].C;
+  d.pk = pk;
+  t[index] = d;
+  return C;
+}
+
 // gx = dL/dx from g = dL/dout and the pre-packed data-gradient operand: one launch
 int po2_conv2d_dgrad_packed(const void* g_out, const void* packed, const float* scale, void* gx, int B, int C, int H,
                             int W, int K, int R, int S, int pad, int compute, void* stream) {

@@ -44,13 +44,15 @@ __device__ __forceinline__ float lin_pow2_round_log2(float step, int flavor) {
   return exp2f(rintf(log2f(step)));
 }
 
-__global__ void __launch_bounds__(LIN_THREADS) lin_quantize_kernel(const float* __restrict__ w, float* __restrict__ y,
-                                                                   int K, int C, int RS, int bits, int iters,
-                                                                   int plus, int flavor) {
+// input channel c of w (K, C, RS) -> y; with pk.Bp set, also the channel's entries of the conv's packed operand(s)
+// (the operand value is y itself: n * 2^k with |n| <= 2^(bits-1) - 1 -- exact in bf16 for bits <= 9, in tf32 for
+// bits <= 12 -- once at least one refinement round has made the step a power of two)
+__device__ __forceinline__ void lin_channel(const float* __restrict__ w, float* __restrict__ y, int K, int C, int RS,
+                                            int bits, int iters, int plus, int flavor, int c, const PackArgs& pk) {
   extern __shared__ float sw[];
   __shared__ double red[LIN_THREADS / 32][2];
   __shared__ float bc[2];
-  const int c = blockIdx.x, n = K * RS;
+  const int n = K * RS;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   // ---- stage the channel, min / max (torch.amax / amin propagate NaN)
   float hi = -INFINITY, lo = INFINITY;
@@ -115,9 +117,46 @@ __global__ void __launch_bounds__(LIN_THREADS) lin_quantize_kernel(const float* 
   for (int i = tid; i < n; i += LIN_THREADS) {
     const int k = i / RS, j = i - k * RS;
     const float q = LIN_Q(sw[i], step);
-    y[((size_t)k * C + c) * RS + j] = __fmul_rn(q, step);
+    const float yv = __fmul_rn(q, step);
+    y[((size_t)k * C + c) * RS + j] = yv;
+    if (pk.Bp) pack_store(pk, k, c, j, yv);
   }
 #undef LIN_Q
+}
+
+__global__ void __launch_bounds__(LIN_THREADS) lin_quantize_kernel(const float* __restrict__ w, float* __restrict__ y,
+                                                                   int K, int C, int RS, int bits, int iters,
+                                                                   int plus, int flavor, PackArgs pk) {
+  lin_channel(w, y, K, C, RS, bits, iters, plus, flavor, blockIdx.x, pk);
+}
+
+// Multi-tensor form: ONE launch for the lin layers of a model, one CTA per (tensor, input channel).  The tensor of a
+// CTA is found by binary search over the descriptors' first CTAs (ascending by construction).
+__global__ void __launch_bounds__(LIN_THREADS) lin_multi_kernel(const LinDesc* __restrict__ descs, int ntensors) {
+  const int b = blockIdx.x;
+  int lo = 0, hi = ntensors - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (descs[mid].cta0 <= b) lo = mid; else hi = mid - 1;
+  }
+  const LinDesc& d = descs[lo];
+  lin_channel(d.w, d.y, d.K, d.C, d.RS, d.bits, d.iters, d.plus, d.flavor, b - d.cta0, d.pk);
+}
+
+int lin_check_args(int K, int C, int RS, int bits, int num_iters, int flavor) {
+  if (K <= 0 || C <= 0 || RS <= 0 || (int64_t)K * C * RS >= (1ll << 31)) return PO2_E_SIZE;
+  if (bits < 2 || bits > 16 || num_iters < 0) return PO2_E_BITS;
+  if (flavor < 0 || flavor >= PO2_NUM_FLAVORS) return PO2_E_FLAVOR;
+  if (flavor == PO2_FLAVOR_TORCH_CUDA && !PO2_HAVE_TORCH_CUDA_TABLE) return PO2_E_FLAVOR;
+  if ((int64_t)K * RS > LIN_MAX_ELEMS) return PO2_E_UNSUPPORTED;
+  return 0;
+}
+
+int lin_launch(const float* w, float* y, int K, int C, int RS, int bits, int iters, int plus, int flavor,
+               const PackArgs& pk, cudaStream_t st) {
+  const size_t smem = (size_t)K * RS * sizeof(float);
+  lin_quantize_kernel<<<C, LIN_THREADS, smem, st>>>(w, y, K, C, RS, bits, iters, plus, flavor, pk);
+  return (int)cudaGetLastError();
 }
 
 }  // namespace po2
@@ -131,14 +170,21 @@ int po2_lin_max_channel_elems(void) { return LIN_MAX_ELEMS; }
 int po2_lin_quantize(const void* w, void* y, int K, int C, int RS, int bits, int num_iters, int plus, int flavor,
                      void* stream) {
   if (!w || !y) return PO2_E_NULL;
-  if (K <= 0 || C <= 0 || RS <= 0 || (int64_t)K * C * RS >= (1ll << 31)) return PO2_E_SIZE;
-  if (bits < 2 || bits > 16 || num_iters < 0) return PO2_E_BITS;
-  if (flavor < 0 || flavor >= PO2_NUM_FLAVORS) return PO2_E_FLAVOR;
-  if (flavor == PO2_FLAVOR_TORCH_CUDA && !PO2_HAVE_TORCH_CUDA_TABLE) return PO2_E_FLAVOR;
-  if ((int64_t)K * RS > LIN_MAX_ELEMS) return PO2_E_UNSUPPORTED;
-  const size_t smem = (size_t)K * RS * sizeof(float);
-  lin_quantize_kernel<<<C, LIN_THREADS, smem, (cudaStream_t)stream>>>((const float*)w, (float*)y, K, C, RS, bits,
-                                                                     num_iters, plus, flavor);
+  if (int e = lin_check_args(K, C, RS, bits, num_iters, flavor)) return e;
+  return lin_launch((const float*)w, (float*)y, K, C, RS, bits, num_iters, plus, flavor, PackArgs{},
+                    (cudaStream_t)stream);
+}
+
+size_t po2_lin_multi_desc_bytes(void) { return sizeof(LinDesc); }
+
+int po2_lin_quantize_pack_multi(const void* device_table, int ntensors, int total_ctas, int max_channel_elems,
+                                void* stream) {
+  if (!device_table) return PO2_E_NULL;
+  if (ntensors < 0 || total_ctas < 0) return PO2_E_SIZE;
+  if (ntensors == 0 || total_ctas == 0) return 0;
+  if (max_channel_elems <= 0 || max_channel_elems > LIN_MAX_ELEMS) return PO2_E_UNSUPPORTED;
+  const size_t smem = (size_t)max_channel_elems * sizeof(float);
+  lin_multi_kernel<<<total_ctas, LIN_THREADS, smem, (cudaStream_t)stream>>>((const LinDesc*)device_table, ntensors);
   return (int)cudaGetLastError();
 }
 

@@ -504,28 +504,8 @@ __device__ __forceinline__ void pack_vec(const PackArgs& pk, const uint4& o, int
     const int rem = e - k * pk.C * pk.taps;
     const int c = fdiv(rem, pk.div_t);
     const int tap = rem - c * pk.taps;
-    const int nt = fdiv(k, pk.div_nt);
-    const int n = k - nt * pk.NT;
     const float yv = __uint_as_float(ob[j]);
-    const float r = (s == 1.0f) ? yv : __fdiv_rn(yv, s);
-    const int cg = pk.G == 8 ? (c >> 3) : (c >> 2), cj = c & (pk.G - 1);
-    const size_t idx = pk.tapminor
-        ? (((((size_t)nt * 3 + tap / 3) * pk.ncg + cg) * 3 + tap % 3) * pk.NT + n) * pk.G + cj
-        : ((((size_t)nt * pk.taps + tap) * pk.ncg + cg) * pk.NT + n) * pk.G + cj;
-    if (pk.G == 8) reinterpret_cast<__nv_bfloat16*>(pk.Bp)[idx] = __float2bfloat16_rn(r);
-    else reinterpret_cast<float*>(pk.Bp)[idx] = r;
-    if (pk.Bp2) {
-      // data-gradient operand: out channel = c, in channel = k, tap rotated (csrc/po2_conv.cu, transpose)
-      const int tap2 = pk.taps - 1 - tap;
-      const int nt2 = fdiv(c, pk.div_nt2);
-      const int n2 = c - nt2 * pk.NT2;
-      const int cg2 = pk.G == 8 ? (k >> 3) : (k >> 2), cj2 = k & (pk.G - 1);
-      const size_t idx2 = pk.tapminor2
-          ? (((((size_t)nt2 * 3 + tap2 / 3) * pk.ncg2 + cg2) * 3 + tap2 % 3) * pk.NT2 + n2) * pk.G + cj2
-          : ((((size_t)nt2 * pk.taps + tap2) * pk.ncg2 + cg2) * pk.NT2 + n2) * pk.G + cj2;
-      if (pk.G == 8) reinterpret_cast<__nv_bfloat16*>(pk.Bp2)[idx2] = __float2bfloat16_rn(r);
-      else reinterpret_cast<float*>(pk.Bp2)[idx2] = r;
-    }
+    pack_store(pk, k, c, tap, (s == 1.0f) ? yv : __fdiv_rn(yv, s));
   }
 }
 

@@ -691,6 +691,91 @@ qconv2d.register_autograd(_qconv2d_bwd, setup_context=_qconv2d_setup)
 
 
 # ------------------------------------------------------------------------------------------------
+# lin / lin+ QAT forward (utils/quantizers.py:59-136 + models/quantized_conv.py:34-36).  A lin weight is n * 2^k per
+# input channel (|n| <= 2^(bits-1) - 1), so it is its own exact tensor-core operand up to these bit widths; every
+# consumer of (packed, scale) then takes it with scale = 1.0.
+# ------------------------------------------------------------------------------------------------
+LIN_EXACT_BITS = {"tc": 9, "tf32": 12, "fp32": 16}
+LIN_ITERS = 10                     # utils/quantizers.py: num_iters default, what QuantizedConv2d and quantize_model use
+_ones = {}
+
+
+def lin_scale(device) -> torch.Tensor:
+    """the per-device fp32 1.0 that stands for the scale of a lin operand (created on first use, outside a capture)"""
+    one = _ones.get(device.index)
+    if one is None:
+        one = _ones[device.index] = torch.ones((), dtype=torch.float32, device=device)
+    return one
+
+
+@torch.library.custom_op("po2::lin_qconv2d", mutates_args=(), device_types="cuda")
+def lin_qconv2d(x: torch.Tensor, weight: torch.Tensor, bits: int, plus: bool, stride: int, pad: int, groups: int,
+                compute: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """(out, y) = (conv2d(x, y), y) with y = lin(weight) (lin+ with plus): the quantizer kernel also writes the conv's
+    packed operand where the shape has one, so the forward is two launches; elsewhere (depthwise, small pointwise,
+    compute 1) the CUDA-core kernels read y directly."""
+    global LAUNCHES
+    _require_cuda(x, "po2::lin_qconv2d")
+    if x.dtype != torch.float32 or weight.dtype != torch.float32:
+        raise TypeError("po2::lin_qconv2d: fp32 NCHW activations and fp32 weights only")
+    check_conv_shapes(x.shape, weight.shape, groups, pad)
+    x = x.contiguous()
+    w = weight.contiguous()
+    lib = _lib.load()
+    B, C, H, W_ = x.shape
+    K, Cg, R, S = w.shape
+    out = torch.empty(_conv_out_shape(x, w, stride, pad), dtype=torch.float32, device=x.device)
+    y = torch.empty_like(w)
+    with torch.cuda.device(x.device):
+        one = lin_scale(x.device)
+        st = _stream_ptr(x.device)
+        nbytes = int(lib.po2_conv2d_pack_bytes(B, C, H, W_, K, R, S, stride, pad, groups, compute))
+        if nbytes:
+            packed = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
+            LAUNCHES += 2 if (C % 16 == 0 and K % 16 == 0) else 3
+            _lib.check(lib.po2_lin_quantize_pack(w.data_ptr(), y.data_ptr(), packed.data_ptr(), nbytes, None, 0, B, C, H, W_,
+                                                 K, R, S, stride, pad, groups, int(bits), LIN_ITERS, int(plus), _flavor,
+                                                 compute, st), "po2_lin_quantize_pack")
+            _lib.check(lib.po2_conv2d_fwd_packed(x.data_ptr(), packed.data_ptr(), one.data_ptr(), out.data_ptr(), B, C, H,
+                                                 W_, K, R, S, stride, pad, groups, compute, st), "po2_conv2d_fwd_packed")
+        else:
+            LAUNCHES += 1
+            _lib.check(lib.po2_lin_quantize(w.data_ptr(), y.data_ptr(), K, Cg, R * S, int(bits), LIN_ITERS, int(plus),
+                                            _flavor, st), "po2_lin_quantize")
+            conv2d_out(x, y, one, out, stride, pad, groups, compute)
+    return out, y
+
+
+@lin_qconv2d.register_fake
+def _(x, weight, bits, plus, stride, pad, groups, compute):
+    return x.new_empty(_conv_out_shape(x, weight, stride, pad)), torch.empty_like(weight, memory_format=torch.contiguous_format)
+
+
+def _lin_qconv2d_setup(ctx, inputs, output):
+    x, weight, bits, plus, stride, pad, groups, compute = inputs
+    out, y = output
+    ctx.save_for_backward(x, y)
+    ctx.cfg = (stride, pad, groups, compute)
+    ctx.set_materialize_grads(False)
+
+
+def _lin_qconv2d_bwd(ctx, g, g_y):
+    x, y = ctx.saved_tensors
+    stride, pad, groups, compute = ctx.cfg
+    if g is None:                            # only the quantized weight was used: straight-through
+        return None, g_y, None, None, None, None, None, None
+    gx, gw = _conv_backward(g, x, y, lin_scale(x.device), stride, pad, groups, compute, ctx.needs_input_grad[0],
+                            ctx.needs_input_grad[1])
+    if g_y is not None:
+        gw = g_y if gw is None else gw + g_y
+    # straight-through estimator (utils/quantizers.py:94-96): d/d weight == d/d quantized weight
+    return gx, gw, None, None, None, None, None, None
+
+
+lin_qconv2d.register_autograd(_lin_qconv2d_bwd, setup_context=_lin_qconv2d_setup)
+
+
+# ------------------------------------------------------------------------------------------------
 # static weights: pack once, then one launch per forward
 # ------------------------------------------------------------------------------------------------
 def conv2d_pack(w: torch.Tensor, scale: Optional[torch.Tensor], xshape, stride: int, pad: int, groups: int,

@@ -21,6 +21,7 @@ from typing import Iterable
 import torch
 
 from . import _lib, ops
+from . import quantizers as _quantizers
 
 
 class _Slot:
@@ -33,7 +34,8 @@ class _Table:
 
 
 def _layer_key(m, xshape, mode):
-    return (m.weight._version, tuple(xshape), mode, int(m.bits), bool(getattr(m.quantize_fn, "_PLUS")), m.weight.device)
+    fam, plus = _quantizers.quantizer_family(m.quantize_fn)
+    return (m.weight._version, tuple(xshape), mode, int(m.bits), plus, m.weight.device, fam)
 
 
 def _static(key):
@@ -64,14 +66,25 @@ def prefetch_weights(modules: Iterable[torch.nn.Module]) -> int:
         return 0
     compute = ops.COMPUTE[mode]
     lib = _lib.load()
-    layers, stale = [], False
+    layers, stale = {"po2": [], "lin": []}, {"po2": False, "lin": False}
+    lin_on = os.environ.get("PO2_LIN", "cuda") == "cuda"
     for m in modules:
-        if not isinstance(m, QuantizedConv2d) or m.quantize_fn is None or getattr(m.quantize_fn, "_PLUS", None) is None:
+        if not isinstance(m, QuantizedConv2d) or m.quantize_fn is None:
+            continue
+        fam = _quantizers.quantizer_family(m.quantize_fn)
+        if fam is None:
             continue
         xshape = m.__dict__.get("_po2_xshape")
         w = m.weight
         if xshape is None or not w.is_cuda or w.dtype != torch.float32 or not w.is_contiguous():
             continue
+        if fam[0] == "lin":
+            # only weights that are their own exact operand and that the lin quantizer kernel takes (the inline path
+            # reports the others)
+            K, _, R, S = w.shape
+            if not lin_on or not 2 <= int(m.bits) <= ops.LIN_EXACT_BITS[mode] or \
+                    K * R * S > lib.po2_lin_max_channel_elems():
+                continue
         key = _layer_key(m, xshape, mode)
         slot = m.__dict__.get("_po2_prefetch")
         if slot is False:                                        # known not to run on the tensor-core kernel
@@ -88,9 +101,13 @@ def prefetch_weights(modules: Iterable[torch.nn.Module]) -> int:
                 continue
             slot = _Slot()
             slot.qw = torch.empty_like(w, memory_format=torch.contiguous_format)
-            slot.scale = torch.empty((), dtype=torch.float32, device=w.device)
             slot.packed = torch.empty(nbytes, dtype=torch.uint8, device=w.device)
-            slot.sse = torch.zeros((), dtype=torch.float64, device=w.device)   # sum((Q(w)-w)^2), refreshed by every launch
+            if fam[0] == "lin":
+                slot.scale = ops.lin_scale(w.device)                        # the lin operand is y itself
+                slot.sse = None
+            else:
+                slot.scale = torch.empty((), dtype=torch.float32, device=w.device)
+                slot.sse = torch.zeros((), dtype=torch.float64, device=w.device)   # sum((Q(w)-w)^2), refreshed by every launch
             # the data-gradient conv's operand (stride-1 dense layers), emitted by the same launch
             nd = 0
             if m.stride[0] == 1 and m.groups == 1 and ops._dgrad_mode == "tc":
@@ -99,10 +116,17 @@ def prefetch_weights(modules: Iterable[torch.nn.Module]) -> int:
             slot.key = None
             m.__dict__["_po2_prefetch"] = slot
         if slot.key != key:
-            stale = True
-        layers.append((m, slot, key))
-    if not layers or not stale:
-        return len(layers)
+            stale[fam[0]] = True
+        layers[fam[0]].append((m, slot, key))
+    # a model that mixes families gets one launch per family
+    if layers["po2"] and stale["po2"]:
+        _launch_po2(layers["po2"], lib, compute)
+    if layers["lin"] and stale["lin"]:
+        _launch_lin(layers["lin"], lib, compute)
+    return len(layers["po2"]) + len(layers["lin"])
+
+
+def _launch_po2(layers, lib, compute) -> None:
     dev = layers[0][0].weight.device
     with torch.cuda.device(dev):
         stream = ops._stream_ptr(dev)
@@ -176,7 +200,59 @@ def prefetch_weights(modules: Iterable[torch.nn.Module]) -> int:
                                                  m.stride[0], m.padding[0], m.groups, int(m.bits), 1, int(key[4]),
                                                  ops._flavor, compute, qws, stream), "po2_quantize_pack")
             slot.key = key
-    return len(layers)
+
+
+def _launch_lin(layers, lib, compute) -> None:
+    """lin / lin+ layers: y, the forward operand and the stride-1 data-gradient operand of every layer in ONE launch of
+    the multi-tensor lin kernel (one CTA per input channel); layers whose operand needs channel padding one by one"""
+    dev = layers[0][0].weight.device
+    with torch.cuda.device(dev):
+        stream = ops._stream_ptr(dev)
+        ident = tuple((id(m), slot.qw.data_ptr(), m.weight.data_ptr(), _static(key)) for m, slot, key in layers)
+        tkey = (id(layers[0][0]), "lin")
+        tab = _tables.get(tkey)
+        if tab is None or tab.ident != ident:
+            dbytes = int(lib.po2_lin_multi_desc_bytes())
+            host = torch.zeros(len(layers) * dbytes, dtype=torch.uint8)
+            n, ctas, max_elems, single = 0, 0, 1, set()
+            for m, slot, key in layers:
+                B, C, H, W_ = key[1]
+                K, _, R, S = m.weight.shape
+                pd = slot.packed_d
+                rc = lib.po2_lin_multi_desc_fill(host.data_ptr(), n, m.weight.data_ptr(), slot.qw.data_ptr(),
+                                                 slot.packed.data_ptr(), slot.packed.numel(),
+                                                 pd.data_ptr() if pd is not None else None, pd.numel() if pd is not None else 0,
+                                                 B, C, H, W_, K, R, S, m.stride[0], m.padding[0], m.groups, int(m.bits),
+                                                 ops.LIN_ITERS, int(key[4]), ops._flavor, compute)
+                if rc == -10:
+                    single.add(id(m))
+                    slot.packed_d = None
+                    continue
+                if rc <= 0:
+                    _lib.check(rc if rc < 0 else -6, "po2_lin_multi_desc_fill")
+                n += 1
+                ctas += rc
+                max_elems = max(max_elems, K * R * S)
+            tab = _Table()
+            tab.ident, tab.n, tab.csize = ident, n, (ctas, max_elems)
+            tab.dev = host[:max(n, 1) * dbytes].to(dev)
+            _tables[tkey] = tab
+            for m, slot, key in layers:
+                m.__dict__["_po2_prefetch_single"] = id(m) in single
+        if tab.n:
+            ops.LAUNCHES += 1
+            _lib.check(lib.po2_lin_quantize_pack_multi(tab.dev.data_ptr(), tab.n, tab.csize[0], tab.csize[1], stream),
+                       "po2_lin_quantize_pack_multi")
+        for m, slot, key in layers:
+            if m.__dict__.get("_po2_prefetch_single"):
+                B, C, H, W_ = key[1]
+                K, _, R, S = m.weight.shape
+                ops.LAUNCHES += 2
+                _lib.check(lib.po2_lin_quantize_pack(m.weight.data_ptr(), slot.qw.data_ptr(), slot.packed.data_ptr(),
+                                                     slot.packed.numel(), None, 0, B, C, H, W_, K, R, S, m.stride[0],
+                                                     m.padding[0], m.groups, int(m.bits), ops.LIN_ITERS, int(key[4]),
+                                                     ops._flavor, compute, stream), "po2_lin_quantize_pack")
+            slot.key = key
 
 
 class _QConvPrefetched(torch.autograd.Function):

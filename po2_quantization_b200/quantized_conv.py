@@ -5,6 +5,7 @@ attributes (``quantize_fn``, ``bits``), ``state_dict`` (``{weight}``) and method
 reference's model files build on it unchanged (SURVEY.md section 8b).
 """
 import copy
+import os
 
 import torch
 import torch.nn as nn
@@ -28,9 +29,10 @@ class QuantizedConv2d(nn.Conv2d):
         memo[id(self)] = new
         new.__dict__ = {k: copy.deepcopy(v, memo) for k, v in self.__dict__.items()
                         if k not in ("_po2_pack_cache", "_po2_prefetch", "_po2_prefetch_single", "_po2_prefetch_static")}
-        tag = self.__dict__.get("_po2_ptq")
-        if tag is not None and tag[0] == self.weight._version:
-            new.__dict__["_po2_ptq"] = (new.weight._version,) + tuple(new.__dict__["_po2_ptq"][1:])
+        for name in ("_po2_ptq", "_po2_lin_ptq"):
+            tag = self.__dict__.get(name)
+            if tag is not None and tag[0] == self.weight._version:
+                new.__dict__[name] = (new.weight._version,) + tuple(new.__dict__[name][1:])
         return new
 
     # ---- which inputs the sm_100a conv kernels take.  Anything else goes to nn.Conv2d's own path
@@ -59,6 +61,73 @@ class QuantizedConv2d(nn.Conv2d):
     def _po2_conv_ok(self, input) -> bool:
         return self._why_not(input) == ""
 
+    def _lin_why_not(self, input, bits, quantizes=True):
+        """_why_not for a lin / lin+ weight, which is its own exact operand only up to ops.LIN_EXACT_BITS of the mode
+        (quantizes: the lin quantizer kernel runs in this forward and must take the channel size)"""
+        why = self._why_not(input)
+        if why != "":
+            return why
+        mode = ops.get_conv_mode()
+        if not 2 <= bits <= ops.LIN_EXACT_BITS[mode]:
+            return f"lin weights of {bits} bits are not exact as {mode} operands (at most {ops.LIN_EXACT_BITS[mode]} bits)"
+        if quantizes:
+            from . import _lib
+            K, _, R, S = self.weight.shape
+            if K * R * S > _lib.load().po2_lin_max_channel_elems():
+                return f"lin quantizer channel of {K * R * S} weights exceeds the kernel's shared-memory capacity"
+        return ""
+
+    def _lin_forward(self, input, plus):
+        """QAT forward of a lin / lin+ layer, or None where it keeps nn.Conv2d's own convolution (reported on CUDA)"""
+        bits = int(self.bits)
+        if os.environ.get("PO2_LIN", "cuda") != "cuda":
+            return None                                       # the op-by-op quantizer reports itself
+        why = self._lin_why_not(input, bits)
+        if why is None or not input.is_cuda:
+            return None                                       # cudnn mode / CPU: the stock path, as requested
+        if why:
+            ops.note_library_path("qconv:" + why, f"QuantizedConv2d runs nn.Conv2d's own convolution (cuDNN) for this "
+                                  f"layer: {why}")
+            return None
+        mode = ops.get_conv_mode()
+        if mode in ("tc", "tf32"):
+            from . import prefetch
+            out = prefetch.try_prefetched_forward(self, input, mode)
+            if out is not None:
+                return out
+            self.__dict__["_po2_xshape"] = tuple(input.shape)
+        out, _y = ops.lin_qconv2d(input, self.weight, bits, bool(plus), self.stride[0], self.padding[0], self.groups,
+                                  ops.COMPUTE[mode])
+        return out
+
+    def _lin_ptq_forward(self, input, tag):
+        """forward of a layer quantize_model() wrote lin / lin+ weights into: the weight is its own operand, scale 1.0"""
+        why = self._lin_why_not(input, tag[1], quantizes=False)
+        if why is None or (why and not input.is_cuda):
+            return self._conv_forward(input, self.weight, self.bias)
+        if why:
+            return self._library_conv(input, self.weight, why)
+        mode = ops.get_conv_mode()
+        one = ops.lin_scale(input.device)
+        if mode in ("tc", "tf32") and not (torch.is_grad_enabled() and (input.requires_grad or self.weight.requires_grad)):
+            packed = self._ptq_packed(input, tag[0], one, mode)
+            if packed is not None:
+                K, _, R, S = self.weight.shape
+                return ops.conv2d_packed(input, packed, one, K, R, S, self.stride[0], self.padding[0], self.groups,
+                                         ops.COMPUTE[mode])
+        return ops.conv2d(input, self.weight, one, self.stride[0], self.padding[0], self.groups, ops.COMPUTE[mode])
+
+    def _ptq_packed(self, input, version, scale, mode):
+        """the packed operand of the static weight, built once per (weight version, input shape); None: no such operand"""
+        key = (version, tuple(input.shape), input.device, mode)
+        cache = self.__dict__.get("_po2_pack_cache")
+        if cache is None or cache[0] != key:
+            packed = ops.conv2d_pack(self.weight.detach(), scale, tuple(input.shape), self.stride[0], self.padding[0],
+                                     self.groups, ops.COMPUTE[mode])
+            cache = (key, packed)
+            self.__dict__["_po2_pack_cache"] = cache
+        return cache[1]
+
     def _library_conv(self, input, weight, why):
         if why:
             ops.note_library_path("qconv:" + why, f"QuantizedConv2d runs nn.Conv2d's own convolution (cuDNN) for this "
@@ -74,7 +143,12 @@ class QuantizedConv2d(nn.Conv2d):
     def forward(self, input):
         # models/quantized_conv.py:32-38: quantize the weight on every forward (QAT), then conv
         if self.quantize_fn is not None:
-            plus = getattr(self.quantize_fn, "_PLUS", None)
+            fam = _quantizers.quantizer_family(self.quantize_fn)
+            if fam is not None and fam[0] == "lin":
+                out = self._lin_forward(input, fam[1])
+                if out is not None:
+                    return out
+            plus = fam[1] if fam is not None and fam[0] == "po2" else None
             if plus is not None and self._po2_conv_ok(input):
                 mode = ops.get_conv_mode()
                 if mode in ("tc", "tf32"):
@@ -90,8 +164,8 @@ class QuantizedConv2d(nn.Conv2d):
                 out, _qw, _scale = ops.qconv2d(input, self.weight, int(self.bits), 1, bool(plus), self.stride[0],
                                                self.padding[0], self.groups, ops.COMPUTE[ops.get_conv_mode()])
                 return out
-            # lin / lin+ (the conv of their result is nn.Conv2d's: those weights are not on a PO2 grid), or
-            # a PO2 layer whose configuration the kernels do not take
+            # a lin / lin+ layer the kernels do not take (reported by _lin_forward on CUDA), or a PO2 layer whose
+            # configuration the kernels do not take
             quantized_weight = self.quantize_fn.apply(self.weight, self.bits)
             return self._library_conv(input, quantized_weight, self._why_not(input) if plus is not None else None)
         tag = getattr(self, "_po2_ptq", None)
@@ -118,6 +192,9 @@ class QuantizedConv2d(nn.Conv2d):
             if why is None:
                 return self._conv_forward(input, self.weight, self.bias)
             return self._po2_conv(input, self.weight, tag[1])
+        tag = self.__dict__.get("_po2_lin_ptq")
+        if tag is not None and tag[0] == self.weight._version:
+            return self._lin_ptq_forward(input, tag)
         # no quantizer and no PTQ tag: a full-precision layer, i.e. plain nn.Conv2d (models/quantized_conv.py:38)
         return self._conv_forward(input, self.weight, self.bias)
 
@@ -126,7 +203,7 @@ class QuantizedConv2d(nn.Conv2d):
         accumulates the batch statistics of the norm behind it (stats["sums"], fp64 [sum | sum of squares | ticket])
         in the conv's epilogue; stats["ok"] reports whether it did."""
         stats["ok"] = False
-        if self.quantize_fn is not None and getattr(self.quantize_fn, "_PLUS", None) is not None and self._po2_conv_ok(input):
+        if self.quantize_fn is not None and _quantizers.quantizer_family(self.quantize_fn) is not None and self._po2_conv_ok(input):
             mode = ops.get_conv_mode()
             if mode == "tf32":
                 from . import prefetch
@@ -148,8 +225,7 @@ class QuantizedConv2d(nn.Conv2d):
         compute = ops.COMPUTE[mode]
         K, _, R, S = self.weight.shape
         if self.quantize_fn is not None:
-            plus = getattr(self.quantize_fn, "_PLUS", None)
-            if plus is None or mode not in ("tc", "tf32"):
+            if _quantizers.quantizer_family(self.quantize_fn) is None or mode not in ("tc", "tf32"):
                 return None
             from . import prefetch
             slot = self.__dict__.get("_po2_prefetch")
@@ -161,7 +237,16 @@ class QuantizedConv2d(nn.Conv2d):
                                         compute, ep_a, ep_b, residual, int(act))
         tag = getattr(self, "_po2_ptq", None)
         if tag is None or tag[0] != self.weight._version:
-            return None                                          # a full-precision layer: plain nn.Conv2d
+            tag = self.__dict__.get("_po2_lin_ptq")
+            if tag is None or tag[0] != self.weight._version or self._lin_why_not(input, tag[1], quantizes=False) != "":
+                return None                                      # a full-precision layer: plain nn.Conv2d
+            one = ops.lin_scale(input.device)
+            packed = self._ptq_packed(input, tag[0], one, mode) if mode in ("tc", "tf32") else None
+            if packed is not None:
+                return ops.conv2d_packed_ep(input, packed, one, K, R, S, self.stride[0], self.padding[0], self.groups,
+                                            compute, ep_a, ep_b, residual, int(act))
+            return ops.conv2d_ep(input, self.weight.detach(), one, self.stride[0], self.padding[0], self.groups, compute,
+                                 ep_a, ep_b, residual, int(act))
         if mode in ("tc", "tf32"):
             key = (tag[0], tuple(input.shape), input.device, mode)
             cache = self.__dict__.get("_po2_pack_cache")
@@ -199,3 +284,7 @@ class QuantizedConv2d(nn.Conv2d):
             quantized_weight = self.quantize_fn.apply(self.weight, self.bits)
             return torch.sum((quantized_weight - self.weight) ** 2), self.weight.numel()
         return 0, self.weight.numel()
+
+
+# quantizers.py imports QuantizedConv2d (quantize_model walks the layers): bound last, read at call time
+from . import quantizers as _quantizers  # noqa: E402

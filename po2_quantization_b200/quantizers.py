@@ -111,6 +111,8 @@ def _lin_forward(w: torch.Tensor, bits: int, num_iters: int, plus: bool) -> torc
 
 class LinearPowerOfTwoQuantizer(torch.autograd.Function):
     """reference utils/quantizers.py:59-96"""
+    # (family, plus): NOT _PLUS, which the PO2 code paths (checkpoint codes, prefetch) read as "PO2 grid"
+    _FAMILY = ("lin", False)
 
     @staticmethod
     def forward(ctx, input: torch.Tensor, bits: int = 4, num_iters: int = 10):
@@ -123,6 +125,7 @@ class LinearPowerOfTwoQuantizer(torch.autograd.Function):
 
 class LinearPowerOfTwoPlusQuantizer(torch.autograd.Function):
     """reference utils/quantizers.py:99-136"""
+    _FAMILY = ("lin", True)
 
     @staticmethod
     def forward(ctx, input: torch.Tensor, bits: int = 4, num_iters: int = 10):
@@ -131,6 +134,16 @@ class LinearPowerOfTwoPlusQuantizer(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_output):
         return grad_output, None, None
+
+
+def quantizer_family(quantizer):
+    """("po2", plus) for PowerOfTwo[Plus]Quantizer, ("lin", plus) for LinearPowerOfTwo[Plus]Quantizer, None for
+    anything else (no quantizer, or one this library has no kernel path for)"""
+    fam = getattr(quantizer, "_FAMILY", None)
+    if fam is not None:
+        return fam
+    plus = getattr(quantizer, "_PLUS", None)
+    return None if plus is None else ("po2", bool(plus))
 
 
 def quantize_model(model: torch.nn.Module, quantizer: Optional[Callable[..., None]], bits: int) -> float:
@@ -160,6 +173,12 @@ def quantize_model(model: torch.nn.Module, quantizer: Optional[Callable[..., Non
                     # non-persistent tag (state_dict stays {weight}): the weight is now on the grid
                     # +-scale*2^q, which lets forward() feed the tensor-core conv an exact operand
                     module._po2_ptq = (param._version, scale, int(bits), bool(quantizer._PLUS))
+                fam = quantizer_family(quantizer)
+                if (fam is not None and fam[0] == "lin" and param is module.weight and param.is_cuda
+                        and os.environ.get("PO2_LIN", "cuda") == "cuda"):
+                    # lin / lin+: n * 2^k per input channel, its own exact operand (scale 1.0); a separate tag, since
+                    # _po2_ptq means PO2 codes to the checkpoint writer
+                    module._po2_lin_ptq = (param._version, int(bits), fam[1])
     if total is None:
         raise ZeroDivisionError("quantize_model: the model has no QuantizedConv2d parameters")
     return float((total / numel).item())
