@@ -140,20 +140,6 @@ int po2_conv2d_fwd_packed_ep(const void* x, const void* packed, const float* sca
                              int W, int K, int R, int S, int stride, int pad, int groups, int compute,
                              const float* ep_a, const float* ep_b, const void* residual, int act, void* stream);
 
-/* Training: the batch statistics of the BatchNorm behind a conv come out of the conv's own epilogue
- * (models/resnet.py:55-71 in train(): bn(conv(x))).  po2_conv2d_fwd_packed_stats = po2_conv2d_fwd_packed that also adds,
- * per out channel, the sum and the sum of squares of its output into `sums` (fp64 atomics; layout [sum (K) | sum of
- * squares (K) | 8-byte ticket slot], zero before the first call); po2_bn_apply_sums is the one-launch train-mode
- * forward of the norm for ONE rank that consumes them and zeroes them again.  PO2_E_UNSUPPORTED from the conv:
- * run it plainly and let the norm compute its statistics. */
-int po2_conv2d_fwd_packed_stats(const void* x, const void* packed, const float* scale, void* out, int B, int C, int H,
-                                int W, int K, int R, int S, int stride, int pad, int groups, int compute, void* sums,
-                                void* stream);
-int po2_bn_apply_sums(const void* x, const void* residual, void* y, void* sums, float* stats_dense, const float* gamma,
-                      const float* beta, float* running_mean, float* running_var, long long* num_batches_tracked,
-                      float momentum, float eps, int act, float* save_mean, float* save_invstd, int B, int C, int HW,
-                      void* stream);
-
 /* QuantizedConv2d.forward in QAT mode as one call -- models/quantized_conv.py:34-36: quantize the fp32
  * master weight w (K, C/groups, R, S) with PO2 (mode 0) / PO2+ (mode 1), then convolve.  qw_out receives
  * the quantized weight (what quantize_fn.apply returns), scale_out its scale.  Where the shape allows,
@@ -354,23 +340,6 @@ size_t po2_bn_mailbox_bytes(void);
 size_t po2_conv2d_stem_wgrad_workspace(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups);
 int po2_conv2d_stem_wgrad(const void* g, const void* x, void* gw, int B, int C, int H, int W, int K, int R, int S, int stride,
                           int pad, int groups, void* workspace, size_t workspace_bytes, void* stream);
-
-/* ---- conv + train-mode BatchNorm (+ residual add) (+ activation) in ONE launch --------------------------------
- * models/resnet.py:55-71 in train(): y = act(bn(conv2d(x, Q(w))) + residual) with batch statistics, from the packed
- * operand (po2_conv2d_pack / the multi-tensor quantizer).  The TMA-fed kernel keeps every tile's accumulator in TMEM,
- * sums the conv output per channel, meets at a grid barrier (cooperative launch), adds the per-CTA partial sums in CTA
- * order (deterministic) and normalises straight out of TMEM: the norm kernel's launch, its read of the conv output
- * and its statistics pass disappear.  conv_out: the conv result (po2_bn_bwd_* read it); save_mean / save_invstd /
- * stats_dense[2K+1] / running statistics as po2_bn_apply writes them (one rank).  workspace:
- * po2_conv2d_bn_workspace(...) bytes (0: shape not taken), zeroed ONCE by the caller and then reused call after call
- * on the same stream.  PO2_E_UNSUPPORTED: run the conv and the norm separately. */
-size_t po2_conv2d_bn_workspace(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups, int compute);
-int po2_conv2d_bn_fwd_packed(const void* x, const void* packed, const float* scale, void* conv_out, void* y,
-                             const void* residual, const float* gamma, const float* beta, float* running_mean,
-                             float* running_var, long long* num_batches_tracked, float momentum, float eps, int act,
-                             float* save_mean, float* save_invstd, float* stats_dense, int B, int C, int H, int W, int K,
-                             int R, int S, int stride, int pad, int groups, int compute, void* workspace,
-                             size_t workspace_bytes, void* stream);
 
 /* ---- the QAT step's parameter update (train.py:54-56 optim.SGD(lr, momentum, weight_decay), :92 optimizer.step()) ----
  * All parameters in one launch per po2_sgd_max_tensors_per_launch() tensors, torch.optim.SGD's arithmetic rounding by

@@ -35,8 +35,6 @@ SIGNATURES = {
     "po2_conv2d_fwd": (_i, [_vp, _vp, _vp, _vp] + [_i] * 14 + [_vp, _sz, _vp]),
     "po2_conv2d_fwd_ep": (_i, [_vp, _vp, _vp, _vp] + [_i] * 14 + [_vp, _sz, _vp, _vp, _vp, _i, _vp]),
     "po2_conv2d_fwd_packed_ep": (_i, [_vp] * 4 + [_i] * 11 + [_vp, _vp, _vp, _i, _vp]),
-    "po2_conv2d_fwd_packed_stats": (_i, [_vp] * 4 + [_i] * 11 + [_vp, _vp]),
-    "po2_bn_apply_sums": (_i, [_vp] * 10 + [_c.c_float, _c.c_float, _i, _vp, _vp, _i, _i, _i, _vp]),
     "po2_conv2d_pack_bytes": (_sz, [_i] * 11),
     "po2_conv2d_pack": (_i, [_vp, _vp, _vp, _sz] + [_i] * 14 + [_vp]),
     "po2_conv2d_fwd_packed": (_i, [_vp] * 4 + [_i] * 11 + [_vp]),
@@ -51,8 +49,6 @@ SIGNATURES = {
     "po2_conv2d_dgrad_workspace": (_sz, [_i] * 9),
     "po2_conv2d_dgrad": (_i, [_vp, _vp, _vp, _vp] + [_i] * 14 + [_vp, _sz, _vp]),
     "po2_dilate2": (_i, [_vp, _vp, _i, _i, _i, _vp]),
-    "po2_conv2d_bn_workspace": (_sz, [_i] * 11),
-    "po2_conv2d_bn_fwd_packed": (_i, [_vp] * 11 + [_c.c_float, _c.c_float, _i, _vp, _vp, _vp] + [_i] * 11 + [_vp, _sz, _vp]),
     "po2_conv2d_stem_wgrad_workspace": (_sz, [_i] * 10),
     "po2_conv2d_stem_wgrad": (_i, [_vp, _vp, _vp] + [_i] * 10 + [_vp, _sz, _vp]),
     "po2_sgd_step": (_i, [_vp, _vp, _vp, _vp, _i, _c.c_float, _c.c_float, _c.c_float, _i, _vp]),

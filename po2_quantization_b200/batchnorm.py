@@ -201,18 +201,6 @@ def bn_fwd_fused_out(x, residual, y, weight, bias, running_mean, running_var, nu
     return True
 
 
-def bn_apply_sums_out(x, residual, y, sums, stats_dense, weight, bias, running_mean, running_var, num_batches_tracked,
-                      momentum, eps, relu, save_mean, save_invstd) -> None:
-    """train-mode forward (one rank) from the per-channel sums the producing conv's epilogue accumulated: one launch"""
-    B, C = x.shape[0], x.shape[1]
-    HW = x.numel() // (B * C)
-    ops.LAUNCHES += 1
-    _lib.check(_lib.load().po2_bn_apply_sums(
-        x.data_ptr(), _ptr(residual), y.data_ptr(), sums.data_ptr(), stats_dense.data_ptr(), _ptr(weight), _ptr(bias),
-        _ptr(running_mean), _ptr(running_var), _ptr(num_batches_tracked), float(momentum), float(eps), int(relu),
-        _ptr(save_mean), _ptr(save_invstd), B, C, HW, ops._stream_ptr(x.device)), "po2_bn_apply_sums")
-
-
 def bn_bwd_fused_out(dy, x, y, save_mean, save_invstd, weight, dgamma, dbeta, dx, dres, relu, bias=None, dy2=None) -> bool:
     """sums + apply of the backward in one launch (one rank, tensors that fit the registers of their CTAs);
     False if the shape is not taken"""
@@ -262,7 +250,7 @@ def bn_bwd_apply_out(dy, x, y, save_mean, save_invstd, weight, sums, stats, dx, 
 class _BatchNormTrain(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, residual, weight, bias, running_mean, running_var, num_batches_tracked, momentum, eps,
-                relu, group, world, exch, sums=None):
+                relu, group, world, exch):
         x = x.contiguous()
         if residual is not None:
             residual = residual.contiguous()
@@ -273,13 +261,7 @@ class _BatchNormTrain(torch.autograd.Function):
             save_mean = torch.empty(C, dtype=torch.float32, device=x.device)
             save_invstd = torch.empty(C, dtype=torch.float32, device=x.device)
             fused = False
-            if sums is not None and world == 1:
-                # the producing conv's epilogue already accumulated the per-channel sums: normalise in one launch
-                stats = stat.view(1, -1)
-                bn_apply_sums_out(x, residual, y, sums, stat, weight, bias, running_mean, running_var, num_batches_tracked,
-                                  momentum, eps, relu, save_mean, save_invstd)
-                fused = True
-            elif world == 1 or (exch is not None and os.environ.get("PO2_BN_FUSED_MULTI", "0") == "1"):
+            if world == 1 or (exch is not None and os.environ.get("PO2_BN_FUSED_MULTI", "0") == "1"):
                 # small tensors: statistics + apply as ONE launch.  With several ranks the kernel can do the
                 # exchange inside too (verified by tools/check_sync_bn.py with PO2_BN_FUSED_MULTI=1), but its
                 # CTAs then sit on the SMs waiting for the peers with the NVLink latency fully exposed:
@@ -326,7 +308,7 @@ class _BatchNormTrain(torch.autograd.Function):
         dx, dres, dgamma, dbeta = bn_backward(dy, x, y, weight, bias, save_mean, save_invstd, stats, ctx.relu,
                                               ctx.has_res and need_res, ctx.world, ctx.exch, ctx.group, dy2=dy2)
         return (dx if need_x else None, dres, dgamma if need_w else None, dbeta if need_b else None,
-                None, None, None, None, None, None, None, None, None, None)
+                None, None, None, None, None, None, None, None, None)
 
 
 def bn_backward(dy, x, y, weight, bias, save_mean, save_invstd, stats, act, want_res, world=1, exch=None, group=None,
@@ -410,16 +392,7 @@ class FusedSyncBatchNorm(nn.SyncBatchNorm):
             raise ValueError(f"act must be one of {sorted(k for k in ACT if k)} or None")
         self.act = act
 
-    def conv_sums(self, device) -> torch.Tensor:
-        """The fp64 buffer [sum (C) | sum of squares (C) | ticket] a producing conv accumulates this norm's batch
-        statistics into (po2_conv2d_fwd_packed_stats); zero between forwards (po2_bn_apply_sums re-zeroes it)."""
-        t = self.__dict__.get("_po2_sums")
-        if t is None or t.device != device:
-            t = self.__dict__["_po2_sums"] = torch.zeros(2 * self.num_features + 1, dtype=torch.float64, device=device)
-        return t
-
-    def forward(self, input: torch.Tensor, residual: Optional[torch.Tensor] = None, relu: bool = False,
-                sums: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def forward(self, input: torch.Tensor, residual: Optional[torch.Tensor] = None, relu: bool = False) -> torch.Tensor:
         act = 1 if relu else ACT[getattr(self, "act", None)]
         use_batch_stats = self.training or (self.running_mean is None and self.running_var is None)
         fast = _kernel_ok(input) and (residual is None or (residual.shape == input.shape and _kernel_ok(residual)))
@@ -446,8 +419,7 @@ class FusedSyncBatchNorm(nn.SyncBatchNorm):
             out = _BatchNormTrain.apply(
                 input, residual, self.weight, self.bias, self.running_mean if track else None,
                 self.running_var if track else None, self.num_batches_tracked if track else None,
-                self.momentum if self.momentum is not None else 0.0, self.eps, kact, group, world, exch,
-                sums if world == 1 else None)
+                self.momentum if self.momentum is not None else 0.0, self.eps, kact, group, world, exch)
             if track:
                 # the kernels wrote the running statistics through raw pointers: bump their version counters, as
                 # torch's in-place update would (fold._affine caches the eval-mode scale / shift on them)

@@ -406,51 +406,13 @@ __global__ void __launch_bounds__(BN_THREADS, 4) bn_apply_kernel(const float* __
                                                               long long* num_batches_tracked, float momentum,
                                                               float eps, int act, int use_running,
                                                               float* __restrict__ save_mean,
-                                                              float* __restrict__ save_invstd, BnGeom g,
-                                                              double* sums, unsigned int* sums_ticket) {
+                                                              float* __restrict__ save_invstd, BnGeom g) {
   extern __shared__ float4 prm[];
   const int C = g.C;
   // x / residual were complete before the statistics kernel started; the statistics (and the mailbox
   // epoch) are that kernel's output
   asm volatile("griddepcontrol.wait;" ::: "memory");
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // the conv behind may set up under this kernel
-  if (sums) {
-    // one rank, statistics from the producing conv's epilogue: sums[c] = sum x, sums[C + c] = sum x^2 over the
-    // B*HW values of channel c (fp64).  Every CTA derives the same parameters; CTA 0 writes the per-channel
-    // outputs; the last CTA to have read the sums (ticket) zeroes them for the layer's next forward.
-    const double cnt = (double)g.B * (double)g.HW;
-    for (int c = threadIdx.x; c < C; c += BN_THREADS) {
-      const double s1 = __ldcg(sums + c), s2 = __ldcg(sums + C + c);
-      const double mean = s1 / cnt;
-      const double m2 = fmax(s2 - s1 * mean, 0.0);
-      const double var = m2 / cnt;
-      const float invstd = (float)(1.0 / sqrt(var + (double)eps));
-      const float ga = gamma ? gamma[c] : 1.0f, be = beta ? beta[c] : 0.0f;
-      prm[c] = make_float4((float)mean, ga * invstd, be, 0.f);
-      if (blockIdx.x == 0) {
-        if (stats_dense) { stats_dense[c] = (float)mean; stats_dense[C + c] = (float)m2; if (c == 0) stats_dense[2 * C] = (float)cnt; }
-        if (save_mean) save_mean[c] = (float)mean;
-        if (save_invstd) save_invstd[c] = invstd;
-        if (running_mean) {
-          const double unbiased = var * cnt / fmax(cnt - 1.0, 1.0);
-          running_mean[c] = (float)((1.0 - (double)momentum) * (double)running_mean[c] + (double)momentum * mean);
-          running_var[c] = (float)((1.0 - (double)momentum) * (double)running_var[c] + (double)momentum * unbiased);
-        }
-      }
-    }
-    if (blockIdx.x == 0 && threadIdx.x == 0 && num_batches_tracked) *num_batches_tracked += 1;
-    __syncthreads();
-    __shared__ int s_last;
-    if (threadIdx.x == 0) {
-      const unsigned int t = atomicAdd(sums_ticket, 1u);
-      s_last = (t == gridDim.x - 1);
-    }
-    __syncthreads();
-    if (s_last) {
-      for (int i = threadIdx.x; i < 2 * C; i += BN_THREADS) sums[i] = 0.0;
-      if (threadIdx.x == 0) *sums_ticket = 0u;
-    }
-  } else {
   const BnGather src = gather_from(stats, 2 * C + 1, use_running ? nullptr : mailbox);
   if (src.ll && blockIdx.x == 0 && stats_dense)          // dense copy of the gathered statistics for backward
     for (int i = threadIdx.x; i < 2 * C + 1; i += BN_THREADS) {
@@ -478,7 +440,6 @@ __global__ void __launch_bounds__(BN_THREADS, 4) bn_apply_kernel(const float* __
   }
   if (blockIdx.x == 0 && threadIdx.x == 0 && !use_running && num_batches_tracked) *num_batches_tracked += 1;
   __syncthreads();
-  }
   const int L = g.L;
   for (int i0 = blockIdx.x * (BN_UNROLL * BN_THREADS) + threadIdx.x; i0 < g.total;
        i0 += gridDim.x * (BN_UNROLL * BN_THREADS)) {
@@ -1159,42 +1120,9 @@ int po2_bn_apply(const void* x, const void* residual, void* y, const float* stat
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = use_running ? 0 : 1;                       // train mode: directly behind po2_bn_stats
-  double* no_sums = nullptr;
-  unsigned int* no_ticket = nullptr;
   return (int)cudaLaunchKernelEx(&cfg, kern, (const float*)x, (const float*)residual, (float*)y, stats, R,
                                  (BnMailbox*)mailbox, stats_dense, gamma, beta, running_mean, running_var,
-                                 num_batches_tracked, momentum, eps, act, use_running, save_mean, save_invstd, g, no_sums,
-                                 no_ticket);
-}
-
-// Train-mode forward for ONE rank whose batch statistics were accumulated by the producing conv's epilogue
-// (po2_conv2d_fwd_packed_stats): sums = [sum x (C) | sum x^2 (C)] in fp64 followed by one 32-bit ticket (8-byte slot),
-// i.e. (2C + 1) * 8 bytes that are zero before the first forward; this kernel zeroes them again.  One launch: no
-// statistics pass over x at all.  stats_dense (2C + 1 floats) receives [mean | M2 | count] for the backward.
-int po2_bn_apply_sums(const void* x, const void* residual, void* y, void* sums, float* stats_dense, const float* gamma,
-                      const float* beta, float* running_mean, float* running_var, long long* num_batches_tracked,
-                      float momentum, float eps, int act, float* save_mean, float* save_invstd, int B, int C, int HW,
-                      void* stream) {
-  if (!x || !y || !sums) return PO2_E_NULL;
-  if (act < 0 || act > 3) return PO2_E_MODE;
-  if (reinterpret_cast<uintptr_t>(sums) & 7) return PO2_E_ALIGN;
-  BnGeom g;
-  const int v = bn_geom(g, B, C, HW, aligned16(x) && aligned16(y) && aligned16(residual));
-  if (v < 0) return v;
-  const size_t smem = (size_t)C * sizeof(float4);
-  auto kern = v ? bn_apply_kernel<true> : bn_apply_kernel<false>;
-  if (smem > 48 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-  }
-  double* ds = reinterpret_cast<double*>(sums);
-  unsigned int* ticket = reinterpret_cast<unsigned int*>(ds + 2 * C);
-  const float* no_stats = nullptr;
-  BnMailbox* no_box = nullptr;
-  kern<<<elementwise_grid(g), BN_THREADS, smem, (cudaStream_t)stream>>>(
-      (const float*)x, (const float*)residual, (float*)y, no_stats, 1, no_box, stats_dense, gamma, beta, running_mean,
-      running_var, num_batches_tracked, momentum, eps, act, 0, save_mean, save_invstd, g, ds, ticket);
-  return (int)cudaGetLastError();
+                                 num_batches_tracked, momentum, eps, act, use_running, save_mean, save_invstd, g);
 }
 
 // One-launch kernels: the S CTAs of a channel as one thread-block cluster when 2 <= S <= 16 (hardware co-scheduling

@@ -182,10 +182,6 @@ struct ConvEpilogue {
   const float* b;
   const float* res;      // same shape as the output, or nullptr
   int act;
-  // training: per-out-channel sum and sum of squares of the conv output, added (fp64 atomics) into sums[0..K) and
-  // sums[K..2K) -- the batch statistics of the BatchNorm behind this conv come out of the conv's own epilogue
-  // (models/resnet.py:55-71 in train()); nullptr: off.  The consumer (po2_bn_apply_sums) zeroes them again.
-  double* sums;
 };
 __device__ __forceinline__ float conv_act(float v, int act) {
   if (act == 1) return fmaxf(v, 0.f);

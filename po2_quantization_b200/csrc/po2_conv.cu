@@ -909,8 +909,7 @@ static bool pdl_chain_enabled() {
 }
 static int launch_umma(const void* x, const void* w, const float* scale, void* out, ConvGeom& g, int w_format,
                        int bits, int fsr, int transpose, void* pack_buf, cudaStream_t st, bool pdl = true,
-                       const ConvEpilogue& ep = ConvEpilogue{nullptr, nullptr, nullptr, 0, nullptr}, bool chain = false) {
-  if (ep.sums && !g.tf32) return PO2_E_UNSUPPORTED;         // only the TMA-fed kernel accumulates statistics
+                       const ConvEpilogue& ep = ConvEpilogue{nullptr, nullptr, nullptr, 0}, bool chain = false) {
   {
     uint8_t* Bp = reinterpret_cast<uint8_t*>(pack_buf);
     cudaError_t e = cudaSuccess;
@@ -925,12 +924,11 @@ static int launch_umma(const void* x, const void* w, const float* scale, void* o
     }
     {                                                     // K3T where the shape allows: activations by tensor-map TMA
       TmaPlan tp;
-      if (g.tf32 && tma_enabled() && plan_tma(g, tp, ep.sums != nullptr)) {
+      if (g.tf32 && tma_enabled() && plan_tma(g, tp)) {
         // (the operand may already be packed in K3T's layout: an x that cannot be described by a tensor map --
         // misaligned -- is an error here, not a fallback)
         return launch_tma(x, Bp, scale, out, g, tp, st, (chain && transpose < 0 && pdl_chain_enabled()) ? 2 : (pdl ? 1 : 0), ep);
       }
-      if (ep.sums) return PO2_E_UNSUPPORTED;
     }
     static PerDeviceOnce attr_once;                       // the opt-in shared-memory size is a per-device attribute
     e = attr_once.run([]() -> cudaError_t {
@@ -1545,68 +1543,6 @@ int po2_conv2d_fwd_packed_ep(const void* x, const void* packed, const float* sca
                      /*pdl=*/false, ep, /*chain=*/true);
 }
 
-// Training forward from a pre-packed operand that also accumulates the batch statistics of the BatchNorm behind
-// the conv: sums[k] += sum of out[:, k], sums[K + k] += sum of out[:, k]^2 (fp64 atomics from the epilogue of the
-// TMA-fed kernel).  PO2_E_UNSUPPORTED: the geometry does not run on that kernel (or its N tile is wider than 32
-// channels) -- the caller then runs the conv plainly and the norm computes its own statistics.
-int po2_conv2d_fwd_packed_stats(const void* x, const void* packed, const float* scale, void* out, int B, int C, int H,
-                                int W, int K, int R, int S, int stride, int pad, int groups, int compute, void* sums,
-                                void* stream) {
-  if (!x || !packed || !out || !sums) return PO2_E_NULL;
-  if (reinterpret_cast<uintptr_t>(sums) & 7) return PO2_E_ALIGN;
-  ConvGeom g;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
-  if (compute != 2 || !umma_eligible(g) || !plan_umma(g, true)) return PO2_E_UNSUPPORTED;
-  TmaPlan tp;
-  if (!tma_enabled() || !plan_tma(g, tp) || g.NT > 32) return PO2_E_UNSUPPORTED;
-  if ((int64_t)B * C * H * W >= (1ll << 31) || (int64_t)B * K * g.P * g.Q >= (1ll << 31)) return PO2_E_SIZE;
-  const ConvEpilogue ep{nullptr, nullptr, nullptr, 0, reinterpret_cast<double*>(sums)};
-  return launch_umma(x, nullptr, scale, out, g, PO2_W_F32_PO2, 4, 1, -1, const_cast<void*>(packed), (cudaStream_t)stream,
-                     /*pdl=*/false, ep);
-}
-
-// conv2d(x, Q(w)) from the packed operand + the train-mode BatchNorm behind it (+ residual add, + activation) in ONE
-// cooperative launch of the TMA-fed kernel (models/resnet.py:55-71 in train(): out = relu(bn(conv(x)) + shortcut)).
-// conv_out receives the conv result (the norm's backward reads it), y the block output.  Workspace: zeroed once by
-// the caller, then reused (16 bytes of self-resetting barrier counters + the per-CTA partial sums).
-size_t po2_conv2d_bn_workspace(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups, int compute) {
-  ConvGeom g;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return 0;
-  if (compute != 2 || !umma_eligible(g) || !plan_umma(g, true)) return 0;
-  TmaPlan tp;
-  if (!tma_enabled() || !plan_tma(g, tp, true, true)) return 0;
-  return 16 + (size_t)tp.m_step * g.ntiles_n * 2 * g.NT * sizeof(double);
-}
-
-int po2_conv2d_bn_fwd_packed(const void* x, const void* packed, const float* scale, void* conv_out, void* y,
-                             const void* residual, const float* gamma, const float* beta, float* running_mean,
-                             float* running_var, long long* num_batches_tracked, float momentum, float eps, int act,
-                             float* save_mean, float* save_invstd, float* stats_dense, int B, int C, int H, int W, int K,
-                             int R, int S, int stride, int pad, int groups, int compute, void* workspace,
-                             size_t workspace_bytes, void* stream) {
-  if (!x || !packed || !conv_out || !y || !workspace) return PO2_E_NULL;
-  if (act < 0 || act > 3) return PO2_E_MODE;
-  if ((running_mean == nullptr) != (running_var == nullptr)) return PO2_E_NULL;
-  if (reinterpret_cast<uintptr_t>(workspace) & 15) return PO2_E_ALIGN;
-  ConvGeom g;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
-  if (compute != 2 || !umma_eligible(g) || !plan_umma(g, true)) return PO2_E_UNSUPPORTED;
-  TmaPlan tp;
-  if (!tma_enabled() || !plan_tma(g, tp, true, true)) return PO2_E_UNSUPPORTED;
-  if ((int64_t)B * C * H * W >= (1ll << 31) || (int64_t)B * K * g.P * g.Q >= (1ll << 31)) return PO2_E_SIZE;
-  if (workspace_bytes < 16 + (size_t)tp.m_step * g.ntiles_n * 2 * g.NT * sizeof(double)) return PO2_E_WORKSPACE;
-  ConvBnTrain bn{};
-  bn.gamma = gamma; bn.beta = beta; bn.y = (float*)y;
-  bn.running_mean = running_mean; bn.running_var = running_var; bn.num_batches_tracked = num_batches_tracked;
-  bn.momentum = momentum; bn.eps = eps;
-  bn.save_mean = save_mean; bn.save_invstd = save_invstd; bn.stats_dense = stats_dense;
-  bn.tickets = reinterpret_cast<unsigned int*>(workspace);
-  bn.partial = reinterpret_cast<double*>(reinterpret_cast<char*>(workspace) + 16);
-  bn.count = (double)B * (double)g.P * (double)g.Q;
-  const ConvEpilogue ep{nullptr, nullptr, (const float*)residual, act, nullptr};
-  return launch_tma(x, (const uint8_t*)packed, scale, conv_out, g, tp, (cudaStream_t)stream, /*pdl=*/false, ep, &bn);
-}
-
 // QuantizedConv2d.forward in QAT mode as ONE call (models/quantized_conv.py:34-36): quantize the fp32
 // master weight (utils/quantizers.py:21-32 / 41-52) and convolve.  When the shape runs on the
 // tensor-core kernel and needs no channel padding, the quantizer kernel itself emits the packed
@@ -1827,7 +1763,7 @@ int po2_conv2d_dgrad_packed(const void* g_out, const void* packed, const float* 
   ConvGeom g;
   if (!dgrad_geom(g, B, C, H, W, K, R, S, pad, compute)) return PO2_E_UNSUPPORTED;
   return launch_umma(g_out, nullptr, scale, gx, g, PO2_W_F32_PO2, 4, 1, -1, const_cast<void*>(packed), (cudaStream_t)stream,
-                     /*pdl=*/false, ConvEpilogue{nullptr, nullptr, nullptr, 0, nullptr}, /*chain=*/true);
+                     /*pdl=*/false, ConvEpilogue{nullptr, nullptr, nullptr, 0}, /*chain=*/true);
 }
 
 size_t po2_conv2d_dgrad_workspace(int B, int C, int H, int W, int K, int R, int S, int pad, int compute) {

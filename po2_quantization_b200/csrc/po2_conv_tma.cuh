@@ -69,29 +69,7 @@ struct TmaPlan {
   FastDiv div_ncol, div_nrb, div_tpi;
 };
 
-// STATS == 2: the train-mode BatchNorm (+ residual add, + activation) behind the conv in the SAME launch
-// (models/resnet.py:55-71 in train()).  Every tile of a CTA keeps its own TMEM accumulator; the epilogue runs twice
-// over them: pass 0 stores the conv output (the norm's backward needs it) and sums it per channel, the CTAs meet at
-// a grid barrier (cooperative launch), every CTA adds the per-CTA partial sums in CTA order (deterministic) and
-// pass 1 normalises straight out of TMEM.  The norm kernel's launch, its read of the conv output and its own
-// statistics pass disappear.
-struct ConvBnTrain {
-  const float* gamma;
-  const float* beta;
-  float* y;                          // act(bn(conv(x)) + ep.res), activation ep.act
-  float* running_mean;
-  float* running_var;
-  long long* num_batches_tracked;
-  float momentum, eps;
-  float* save_mean;
-  float* save_invstd;
-  float* stats_dense;                // [2K + 1]: mean, sum of squared deviations, count (po2_bn_bwd_apply's `stats`)
-  double* partial;                   // [grid][2][NT]
-  unsigned int* tickets;             // two zeroed counters (left zero)
-  double count;                      // B * P * Q
-};
-
-constexpr int KT_MAX_ACC = 8;         // TMEM accumulator stages (STATS == 2: tiles per CTA)
+constexpr int KT_MAX_ACC = 8;         // accumulator barrier slots in shared memory (nacc <= 2 used); sizes the stage count
 constexpr int KT_EPI_WARPS = 4;
 constexpr int KT_THREADS = 32 * (KT_EPI_WARPS + 2);
 constexpr uint32_t KT_SMEM_BUDGET = 222 * 1024;
@@ -122,14 +100,12 @@ __device__ __forceinline__ uint32_t make_idesc_tma(uint32_t m, uint32_t n) {
   return (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | ((n >> 3) << 17) | ((m >> 4) << 24);
 }
 
-// STATS: the epilogue also accumulates per-out-channel sum / sum of squares (64 more registers per thread: that
-// variant is built for one CTA per SM)
-template <int NTAPS, int STATS>
-__global__ void __launch_bounds__(KT_THREADS, STATS ? 1 : 2) conv_tma_kernel(const __grid_constant__ CUtensorMap tmx,
+template <int NTAPS>
+__global__ void __launch_bounds__(KT_THREADS, 2) conv_tma_kernel(const __grid_constant__ CUtensorMap tmx,
                                                                  const uint8_t* __restrict__ Bp,
                                                                  const float* __restrict__ scale,
                                                                  float* __restrict__ out, ConvGeom g, TmaPlan tp,
-                                                                 ConvEpilogue ep, ConvBnTrain bn) {
+                                                                 ConvEpilogue ep) {
   extern __shared__ __align__(128) uint8_t smem[];
   const uint32_t smem_base = smem_u32(smem);
   uint8_t* sB = smem;
@@ -342,7 +318,6 @@ __global__ void __launch_bounds__(KT_THREADS, STATS ? 1 : 2) conv_tma_kernel(con
     // folded BatchNorm: this CTA's NT scale / shift values are staged in shared memory once (the epilogue is on
     // the critical path: 2 x 16 broadcast global loads per thread and tile were measured to double the kernel)
     __shared__ float s_ep[2][256];                             // scale, shift
-    __shared__ float s_mean[64];                               // STATS == 2: the batch mean
     if (ep.a) {
       for (int i = tid; i < NT; i += 32 * KT_EPI_WARPS) {
         const bool ok = kbase + i < K;
@@ -351,32 +326,7 @@ __global__ void __launch_bounds__(KT_THREADS, STATS ? 1 : 2) conv_tma_kernel(con
       }
       asm volatile("bar.sync 2, %0;" ::"n"(32 * KT_EPI_WARPS) : "memory");
     }
-    // batch statistics for the norm behind this conv: every thread sums its pixels' values per out channel over
-    // all tiles of the CTA, reduced once at the end (16-column blocks in separately named arrays so that they stay
-    // in registers; STATS == 1: NT <= 32, STATS == 2: NT <= 64)
-    float st_s0[16], st_q0[16], st_s1[16], st_q1[16], st_s2[16], st_q2[16], st_s3[16], st_q3[16];
-#pragma unroll
-    for (int j = 0; j < 16; ++j) {
-      st_s0[j] = 0.f; st_q0[j] = 0.f; st_s1[j] = 0.f; st_q1[j] = 0.f;
-      st_s2[j] = 0.f; st_q2[j] = 0.f; st_s3[j] = 0.f; st_q3[j] = 0.f;
-    }
     const uint32_t accmask = (uint32_t)tp.nacc - 1u;
-    constexpr int NPASS = STATS == 2 ? 2 : 1;
-    // PO2_TMA_DEBUG bit 16 (STATS == 2): CTA 0 leaves globaltimer stamps 200 KB into the workspace
-    // (epilogue start, pass 0 done, partials written, barrier passed, statistics ready, pass 1 done)
-    unsigned long long* stamps = nullptr;
-    if (STATS == 2 && (tp.debug & 16) && blockIdx.x == 0 && tid == 0)
-      stamps = reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(bn.tickets) + 200 * 1024);
-    auto stamp = [&](int i) {
-      if (STATS == 2 && stamps) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); stamps[i] = t; }
-    };
-    stamp(0);
-#pragma unroll 1
-    for (int pass = 0; pass < NPASS; ++pass) {
-    // STATS == 2: pass 0 = conv output + sums, pass 1 = normalise from the same accumulators (their tfull barriers
-    // completed phase 0 for good: the second wait returns at once)
-    const bool affine = STATS == 2 ? pass == 1 : ep.a != nullptr;
-    float* __restrict__ dst = (STATS == 2 && pass == 1) ? bn.y : out;
     uint32_t acc = 0, aphase = 0;
     int tr_item = 0;
     (void)tr_item;
@@ -405,7 +355,7 @@ __global__ void __launch_bounds__(KT_THREADS, STATS ? 1 : 2) conv_tma_kernel(con
       // a kernel launched programmatically behind this conv may be scheduled once every CTA is at its last tile (not
       // earlier: a resident dependent that only waits takes registers and CTA slots from this grid's tail); it waits
       // for this grid's completion (griddepcontrol.wait) before it reads the output
-      if (m + m_step >= nitems && pass == NPASS - 1) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+      if (m + m_step >= nitems) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
       mbar_wait(tfull + acc, aphase);
       tc_fence_after();
       if (warp == 0 && lane == 0) K3_TRACE(1, 2 * tr_item);
@@ -432,25 +382,10 @@ __global__ void __launch_bounds__(KT_THREADS, STATS ? 1 : 2) conv_tma_kernel(con
 #pragma unroll
           for (int j = 0; j < 16; ++j) v[j] = __uint_as_float(r[j]) * sc;
         }
-        if (STATS != 0 && pass == 0 && valid) {
-          if (cb == 0) {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) { st_s0[j] += v[j]; st_q0[j] = fmaf(v[j], v[j], st_q0[j]); }
-          } else if (cb == 1) {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) { st_s1[j] += v[j]; st_q1[j] = fmaf(v[j], v[j], st_q1[j]); }
-          } else if (STATS == 2 && cb == 2) {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) { st_s2[j] += v[j]; st_q2[j] = fmaf(v[j], v[j], st_q2[j]); }
-          } else if (STATS == 2 && cb == 3) {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) { st_s3[j] += v[j]; st_q3[j] = fmaf(v[j], v[j], st_q3[j]); }
-          }
-        }
         if (valid) {
-          float* po = dst + obase + cb * 16 * HW;
+          float* po = out + obase + cb * 16 * HW;
           const int kleft = K - (kbase + cb * 16);
-          if (affine) {                                        // BatchNorm (+ residual) (+ activation)
+          if (ep.a) {                                          // BatchNorm (+ residual) (+ activation)
             float rs[16];
             if (ep.res) {
               const float* pr = ep.res + obase + cb * 16 * HW;
@@ -459,10 +394,7 @@ __global__ void __launch_bounds__(KT_THREADS, STATS ? 1 : 2) conv_tma_kernel(con
             }
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
-              // folded eval-mode norm: conv * a + b;  train mode: (conv - mean) * (gamma * invstd) + beta, the
-              // expression of bn_apply_kernel
-              float t = STATS == 2 ? fmaf(v[j] - s_mean[cb * 16 + j], s_ep[0][cb * 16 + j], s_ep[1][cb * 16 + j])
-                                   : fmaf(v[j], s_ep[0][cb * 16 + j], s_ep[1][cb * 16 + j]);
+              float t = fmaf(v[j], s_ep[0][cb * 16 + j], s_ep[1][cb * 16 + j]);   // folded eval-mode norm
               if (ep.res) t += rs[j];
               v[j] = conv_act(t, ep.act);
             }
@@ -479,181 +411,11 @@ __global__ void __launch_bounds__(KT_THREADS, STATS ? 1 : 2) conv_tma_kernel(con
       }
       tc_fence_before();
       __syncwarp();
-      if (STATS != 2 && lane == 0) mbar_arrive(tempty + acc);  // STATS == 2: every tile has its own accumulator
+      if (lane == 0) mbar_arrive(tempty + acc);
       if (warp == 0 && lane == 0) K3_TRACE(1, 2 * tr_item + 1);
       ++tr_item;
       acc = (acc + 1) & accmask;
       aphase ^= (acc == 0);
-    }
-    if (STATS == 2 && pass == 1) stamp(5);
-    if (STATS == 2 && pass == 0) {
-      stamp(1);
-      // ---- per-channel sums of this CTA: lanes (pixels) by a halving butterfly in fp32 -- 16 shuffles per 16
-      // channels, lane l ends with channel ((l>>4)&1)*8 + ((l>>3)&1)*4 + ((l>>2)&1)*2 + ((l>>1)&1) -- then the
-      // four warps and everything after in fp64
-      __shared__ float s_w[KT_EPI_WARPS][2][64];
-      __shared__ int s_ok2;
-      auto fold16 = [&](float (&a)[16]) -> float {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const bool hi = lane & 16;
-          const float send = hi ? a[i] : a[i + 8], keep = hi ? a[i + 8] : a[i];
-          a[i] = keep + __shfl_xor_sync(0xFFFFFFFFu, send, 16);
-        }
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const bool hi = lane & 8;
-          const float send = hi ? a[i] : a[i + 4], keep = hi ? a[i + 4] : a[i];
-          a[i] = keep + __shfl_xor_sync(0xFFFFFFFFu, send, 8);
-        }
-#pragma unroll
-        for (int i = 0; i < 2; ++i) {
-          const bool hi = lane & 4;
-          const float send = hi ? a[i] : a[i + 2], keep = hi ? a[i + 2] : a[i];
-          a[i] = keep + __shfl_xor_sync(0xFFFFFFFFu, send, 4);
-        }
-        {
-          const bool hi = lane & 2;
-          const float send = hi ? a[0] : a[1], keep = hi ? a[1] : a[0];
-          a[0] = keep + __shfl_xor_sync(0xFFFFFFFFu, send, 2);
-        }
-        return a[0] + __shfl_xor_sync(0xFFFFFFFFu, a[0], 1);
-      };
-      const int chl = ((lane >> 4) & 1) * 8 + ((lane >> 3) & 1) * 4 + ((lane >> 2) & 1) * 2 + ((lane >> 1) & 1);
-      {
-        float t;
-        t = fold16(st_s0); if (!(lane & 1)) s_w[warp][0][chl] = t;
-        t = fold16(st_q0); if (!(lane & 1)) s_w[warp][1][chl] = t;
-        if (NT > 16) {
-          t = fold16(st_s1); if (!(lane & 1)) s_w[warp][0][16 + chl] = t;
-          t = fold16(st_q1); if (!(lane & 1)) s_w[warp][1][16 + chl] = t;
-        }
-        if (NT > 32) {
-          t = fold16(st_s2); if (!(lane & 1)) s_w[warp][0][32 + chl] = t;
-          t = fold16(st_q2); if (!(lane & 1)) s_w[warp][1][32 + chl] = t;
-        }
-        if (NT > 48) {
-          t = fold16(st_s3); if (!(lane & 1)) s_w[warp][0][48 + chl] = t;
-          t = fold16(st_q3); if (!(lane & 1)) s_w[warp][1][48 + chl] = t;
-        }
-      }
-      asm volatile("bar.sync 2, %0;" ::"n"(32 * KT_EPI_WARPS) : "memory");
-      if (tid < 2 * NT) {
-        const int which = tid / NT, ch = tid - which * NT;
-        const double t = ((double)s_w[0][which][ch] + (double)s_w[1][which][ch]) +
-                         ((double)s_w[2][which][ch] + (double)s_w[3][which][ch]);
-        bn.partial[((size_t)blockIdx.x * 2 + which) * NT + ch] = t;
-      }
-      // ---- grid barrier (cooperative launch: every CTA is resident); self-resetting
-      __threadfence();
-      asm volatile("bar.sync 2, %0;" ::"n"(32 * KT_EPI_WARPS) : "memory");
-      stamp(2);
-      if (tid == 0) {
-        s_ok2 = 1;
-        __threadfence();
-        atomicAdd(bn.tickets, 1u);
-        unsigned long long t0;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-        while (*reinterpret_cast<volatile unsigned int*>(bn.tickets) < gridDim.x) {
-          unsigned long long t1;
-          asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-          if (t1 - t0 > 10000000000ull) { s_ok2 = 0; break; }   // never hang the GPU; the output is poisoned below
-          __nanosleep(20);
-        }
-        __threadfence();
-        const unsigned int d = atomicAdd(bn.tickets + 1, 1u);
-        if (d == gridDim.x - 1) { bn.tickets[0] = 0u; bn.tickets[1] = 0u; __threadfence(); }
-      }
-      asm volatile("bar.sync 2, %0;" ::"n"(32 * KT_EPI_WARPS) : "memory");
-      // ---- the batch statistics: every CTA adds the partials in a fixed order (same numbers everywhere).  The
-      // 128 threads split into (statistic, channel) pairs x `nparts` interleaved slices of the CTA list, eight
-      // loads in flight each (one thread per channel walking all CTAs pays one L2 latency per CTA: measured 12 us);
-      // the slices meet in shared memory (the pipeline stages are idle by now) and are added in slice order.
-      stamp(3);
-      double* s_red = reinterpret_cast<double*>(sA);          // [nparts][2 * NT]
-      {
-        const int npairs = 2 * NT;
-        const int nparts = (32 * KT_EPI_WARPS) / npairs > 0 ? (32 * KT_EPI_WARPS) / npairs : 1;
-        const int P = (int)gridDim.x / g.ntiles_n;            // the CTAs of this channel block: blockIdx.x = m * ntiles_n + nt
-        const size_t cta_stride = (size_t)g.ntiles_n * 2 * NT;
-        for (int item = tid; item < npairs * nparts; item += 32 * KT_EPI_WARPS) {
-          const int part = item / npairs, pair = item - part * npairs;
-          const double* pp = bn.partial + (size_t)nt * 2 * NT + pair;
-          double a = 0.0;
-          int c2 = part;
-          for (; c2 + 7 * nparts < P; c2 += 8 * nparts) {
-            double v8[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) v8[u] = __ldcg(pp + (size_t)(c2 + u * nparts) * cta_stride);
-#pragma unroll
-            for (int u = 0; u < 8; ++u) a += v8[u];
-          }
-          for (; c2 < P; c2 += nparts) a += __ldcg(pp + (size_t)c2 * cta_stride);
-          s_red[part * npairs + pair] = a;
-        }
-        asm volatile("bar.sync 2, %0;" ::"n"(32 * KT_EPI_WARPS) : "memory");
-      }
-      if (tid < NT) {
-        const int ch = tid;
-        const int npairs = 2 * NT;
-        const int nparts = (32 * KT_EPI_WARPS) / npairs > 0 ? (32 * KT_EPI_WARPS) / npairs : 1;
-        double S = 0.0, Q = 0.0;
-        for (int part = 0; part < nparts; ++part) { S += s_red[part * npairs + ch]; Q += s_red[part * npairs + NT + ch]; }
-        const double cnt = bn.count;
-        const double mean = S / cnt;
-        double m2 = Q - S * mean;                              // sum of squared deviations
-        if (m2 < 0.0) m2 = 0.0;
-        const double var = m2 / cnt;
-        float invstd = (float)(1.0 / sqrt(var + (double)bn.eps));
-        if (!s_ok2) invstd = __uint_as_float(0x7FC00000u);     // incomplete sums must not pass for a result
-        const int kch = kbase + ch;
-        const bool ok = kch < K;
-        const float ga = (ok && bn.gamma) ? __ldg(bn.gamma + kch) : 1.0f, be = (ok && bn.beta) ? __ldg(bn.beta + kch) : 0.0f;
-        s_ep[0][ch] = ga * invstd;
-        s_ep[1][ch] = be;
-        s_mean[ch] = (float)mean;
-        if (m_first == 0 && ok) {
-          if (bn.save_mean) bn.save_mean[kch] = (float)mean;
-          if (bn.save_invstd) bn.save_invstd[kch] = invstd;
-          if (bn.stats_dense) {
-            bn.stats_dense[kch] = (float)mean;
-            bn.stats_dense[K + kch] = (float)m2;
-            if (kch == 0) bn.stats_dense[2 * K] = (float)cnt;
-          }
-          if (bn.running_mean && s_ok2) {
-            const double unbiased = var * cnt / fmax(cnt - 1.0, 1.0), mo = (double)bn.momentum;
-            bn.running_mean[kch] = (float)((1.0 - mo) * (double)bn.running_mean[kch] + mo * mean);
-            bn.running_var[kch] = (float)((1.0 - mo) * (double)bn.running_var[kch] + mo * unbiased);
-          }
-          if (kch == 0 && bn.num_batches_tracked) *bn.num_batches_tracked += 1;
-        }
-      }
-      asm volatile("bar.sync 2, %0;" ::"n"(32 * KT_EPI_WARPS) : "memory");
-      stamp(4);
-    }
-    }  // pass
-    if (STATS == 1) {
-      // lanes -> warp (fp64 from here on) -> the four epilogue warps through shared memory -> one fp64 atomic per
-      // (channel, CTA) and statistic.  Rounding: fp32 only inside a thread's own <= a-dozen values.
-      __shared__ double s_st[KT_EPI_WARPS][2][32];
-#pragma unroll
-      for (int b = 0; b < 2; ++b)
-#pragma unroll
-        for (int j = 0; j < 16; ++j) {
-          double a = (double)(b == 0 ? st_s0[j] : st_s1[j]), q2 = (double)(b == 0 ? st_q0[j] : st_q1[j]);
-#pragma unroll
-          for (int o = 16; o > 0; o >>= 1) {
-            a += __shfl_xor_sync(0xFFFFFFFFu, a, o);
-            q2 += __shfl_xor_sync(0xFFFFFFFFu, q2, o);
-          }
-          if (lane == 0) { s_st[warp][0][b * 16 + j] = a; s_st[warp][1][b * 16 + j] = q2; }
-        }
-      asm volatile("bar.sync 2, %0;" ::"n"(32 * KT_EPI_WARPS) : "memory");
-      if (tid < 2 * NT && NT <= 32) {
-        const int which = tid / NT, ch = tid - which * NT;
-        const double t = s_st[0][which][ch] + s_st[1][which][ch] + s_st[2][which][ch] + s_st[3][which][ch];
-        if (kbase + ch < K) atomicAdd(ep.sums + which * K + kbase + ch, t);
-      }
     }
   }
   tc_fence_before();
@@ -691,8 +453,7 @@ static size_t tma_smem_bytes(const ConvGeom& g, const TmaPlan& tp) {
 
 // g: through plan_umma(g, tf32 = true) (supplies the weight-operand plan NT / ntiles_n / Cpad / slab bytes,
 // so that every existing pack path feeds this kernel unchanged).  False: shape stays on the register-fed kernel.
-// fused_bn: the STATS == 2 form -- one CTA per SM, every tile of a CTA in its own TMEM accumulator
-static bool plan_tma(const ConvGeom& g, TmaPlan& tp, bool one_cta_per_sm = false, bool fused_bn = false) {
+static bool plan_tma(const ConvGeom& g, TmaPlan& tp) {
   if (!g.tf32 || g.groups != 1 || g.stride != 1) return false;
   if (!((g.R == 3 && g.S == 3 && g.pad == 1) || (g.R == 1 && g.S == 1 && g.pad == 0))) return false;
   if (g.C % 8 || g.Cpad != g.C) return false;
@@ -724,8 +485,6 @@ static bool plan_tma(const ConvGeom& g, TmaPlan& tp, bool one_cta_per_sm = false
   // so that no pixel's horizontal neighbour lives in another warp)
   tp.MT = 128;
   if (count_items(128) * g.ntiles_n < sms && count_items(64) > count_items(128) && (tp.ntaps == 1 || tp.WB <= 16)) tp.MT = 64;
-  // (the fused conv + norm form runs one CTA per SM: 64-pixel tiles only when 128-pixel ones leave half the SMs idle)
-  if (fused_bn && tp.MT == 64 && count_items(128) * g.ntiles_n * 2 >= sms) tp.MT = 128;
   const int accw = (tp.ntaps == 9 ? 3 : 1) * g.NT;
   if (accw > 256) return false;                              // one MMA spans the accumulator row (N <= 256)
   tp.nacc = 2 * accw <= 512 ? 2 : 1;
@@ -769,7 +528,7 @@ static bool plan_tma(const ConvGeom& g, TmaPlan& tp, bool one_cta_per_sm = false
   while (ncols < (uint32_t)(tp.nacc * accw)) ncols <<= 1;
   size_t budget = KT_SMEM_BUDGET;
   tp.cps = 1;
-  if (!one_cta_per_sm && fixed + 3 * (size_t)tp.stage_bytes <= KT_SMEM_BUDGET_2 && 2 * ncols <= 512 && tp.nitems_m * g.ntiles_n > sms &&
+  if (fixed + 3 * (size_t)tp.stage_bytes <= KT_SMEM_BUDGET_2 && 2 * ncols <= 512 && tp.nitems_m * g.ntiles_n > sms &&
       !(getenv("PO2_TMA_CPS") && getenv("PO2_TMA_CPS")[0] == '1')) {
     tp.cps = 2;
     budget = KT_SMEM_BUDGET_2;
@@ -780,16 +539,6 @@ static bool plan_tma(const ConvGeom& g, TmaPlan& tp, bool one_cta_per_sm = false
   int per_n = tp.cps * sms / g.ntiles_n;
   if (per_n < 1) per_n = 1;
   tp.m_step = tp.nitems_m < per_n ? tp.nitems_m : per_n;
-  if (fused_bn) {
-    // all channels in one CTA column, every CTA resident, one accumulator per tile of a CTA
-    if (g.NT > 64 || tp.cps != 1 || g.ntiles_n > sms) return false;
-    if (tp.m_step * g.ntiles_n > sms) tp.m_step = sms / g.ntiles_n;
-    const int tiles = (tp.nitems_m + tp.m_step - 1) / tp.m_step;
-    int nacc = 1;
-    while (nacc < tiles) nacc <<= 1;
-    if (nacc > KT_MAX_ACC || nacc * accw > 512) return false;
-    tp.nacc = nacc;
-  }
   tp.div_ncol = make_fastdiv((uint32_t)(tp.ncol > 0 ? tp.ncol : 1));
   tp.div_nrb = make_fastdiv((uint32_t)(tp.nrb > 0 ? tp.nrb : 1));
   tp.div_tpi = make_fastdiv((uint32_t)(tp.tiles_per_img > 0 ? tp.tiles_per_img : 1));
@@ -834,7 +583,7 @@ static bool tma_takes(const ConvGeom& g) {
 
 // the conv launch behind the packed operand (same contract as the register-fed launch in launch_umma)
 static int launch_tma(const void* x, const uint8_t* Bp, const float* scale, void* out, const ConvGeom& g, const TmaPlan& tp_in,
-                      cudaStream_t st, int pdl, const ConvEpilogue& ep, const ConvBnTrain* bn = nullptr) {
+                      cudaStream_t st, int pdl, const ConvEpilogue& ep) {
   TmaPlan tp = tp_in;
   tp.pdl = pdl;
   CUtensorMap tm;
@@ -843,11 +592,9 @@ static int launch_tma(const void* x, const uint8_t* Bp, const float* scale, void
   cudaError_t e = attr_once.run([]() -> cudaError_t {
     const int smax = (int)KT_SMEM_BUDGET + 1024;
     cudaError_t a = cudaSuccess;
-    const void* kerns[6] = {(const void*)conv_tma_kernel<1, 0>, (const void*)conv_tma_kernel<9, 0>,
-                            (const void*)conv_tma_kernel<1, 1>, (const void*)conv_tma_kernel<9, 1>,
-                            (const void*)conv_tma_kernel<1, 2>, (const void*)conv_tma_kernel<9, 2>};
-    for (int i = 0; i < 6 && a == cudaSuccess; ++i) {
-      // dynamic + static shared memory <= 227 KB per CTA (the statistics variants carry more static arrays)
+    const void* kerns[2] = {(const void*)conv_tma_kernel<1>, (const void*)conv_tma_kernel<9>};
+    for (int i = 0; i < 2 && a == cudaSuccess; ++i) {
+      // dynamic + static shared memory <= 227 KB per CTA
       cudaFuncAttributes fa;
       a = cudaFuncGetAttributes(&fa, kerns[i]);
       if (a != cudaSuccess) break;
@@ -869,29 +616,8 @@ static int launch_tma(const void* x, const uint8_t* Bp, const float* scale, void
   cfg.attrs = attr;
   cfg.numAttrs = pdl ? 1 : 0;
   float* of = (float*)out;
-  if (bn) {                          // conv + train-mode BatchNorm in one cooperative launch (grid barrier inside)
-    if (pdl) return PO2_E_MODE;
-    const ConvBnTrain bnv = *bn;
-    ConvGeom gv = g;
-    ConvEpilogue epv = ep;
-    const uint8_t* bpv = Bp;
-    void* args[] = {&tm, &bpv, &scale, &of, &gv, &tp, &epv, const_cast<ConvBnTrain*>(&bnv)};
-    const void* kern = tp.ntaps == 1 ? (const void*)conv_tma_kernel<1, 2> : (const void*)conv_tma_kernel<9, 2>;
-    e = cudaLaunchCooperativeKernel(kern, cfg.gridDim, cfg.blockDim, args, cfg.dynamicSmemBytes, st);
-    if (e == cudaErrorCooperativeLaunchTooLarge) {
-      (void)cudaGetLastError();
-      return PO2_E_UNSUPPORTED;
-    }
-    return (int)e;
-  }
-  const ConvBnTrain nobn{};
-  if (ep.sums) {                     // the variant that also accumulates the following norm's batch statistics
-    if (tp.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_tma_kernel<1, 1>, tm, Bp, scale, of, g, tp, ep, nobn);
-    else e = cudaLaunchKernelEx(&cfg, conv_tma_kernel<9, 1>, tm, Bp, scale, of, g, tp, ep, nobn);
-  } else {
-    if (tp.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_tma_kernel<1, 0>, tm, Bp, scale, of, g, tp, ep, nobn);
-    else e = cudaLaunchKernelEx(&cfg, conv_tma_kernel<9, 0>, tm, Bp, scale, of, g, tp, ep, nobn);
-  }
+  if (tp.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_tma_kernel<1>, tm, Bp, scale, of, g, tp, ep);
+  else e = cudaLaunchKernelEx(&cfg, conv_tma_kernel<9>, tm, Bp, scale, of, g, tp, ep);
   return (int)e;
 }
 

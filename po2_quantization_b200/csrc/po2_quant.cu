@@ -895,7 +895,7 @@ using namespace po2;
 
 extern "C" {
 
-int po2_abi_version(void) { return 1; }
+int po2_abi_version(void) { return 2; }
 
 int po2_have_torch_cuda_table(void) { return PO2_HAVE_TORCH_CUDA_TABLE; }
 

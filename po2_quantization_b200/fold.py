@@ -55,22 +55,6 @@ def conv_bn_act(conv, bn, x: torch.Tensor, residual: Optional[torch.Tensor] = No
         out = conv.forward_folded(x, a, b, residual, act)
         if out is not None:
             return out
-    if bn.training and torch.is_grad_enabled():
-        # training on one rank: conv + batch statistics + normalise (+ add, + activation) as ONE launch
-        out = _try_conv_bn_train(conv, bn, x, residual, act)
-        if out is not None:
-            return out
-    if (isinstance(bn, FusedSyncBatchNorm) and isinstance(conv, QuantizedConv2d) and bn.training and x.is_cuda
-            and x.dtype == torch.float32 and bn.momentum is not None and os.environ.get("PO2_CONV_STATS", "0") == "1"
-            and not (torch.distributed.is_available() and torch.distributed.is_initialized()
-                     and torch.distributed.get_world_size() > 1)):
-        # training on one rank, opt-in (PO2_CONV_STATS=1): the conv's epilogue accumulates the norm's batch
-        # statistics (no statistics pass over the conv output).  Measured on the ResNet-56 step: 2.998 vs 3.013 ms --
-        # the one-launch norm kernel already reads x once, so little is left to save -- and the fp64 atomics make the
-        # summation order, hence the last bit of the statistics, run-dependent; off by default for reproducibility.
-        stats = {"sums": bn.conv_sums(x.device), "ok": False}
-        y = conv.forward_with_stats(x, stats)
-        return bn(y, residual, relu, stats["sums"] if stats["ok"] else None)
     y = conv(x)
     if getattr(bn, "fused_residual_relu", False):
         return bn(y, residual, relu)
@@ -78,119 +62,6 @@ def conv_bn_act(conv, bn, x: torch.Tensor, residual: Optional[torch.Tensor] = No
     if residual is not None:
         y = y + residual
     return F.relu(y) if relu else y
-
-
-_bn_workspaces = {}
-
-
-def _conv_bn_workspace(device, nbytes):
-    """zeroed once, reused by every fused conv + norm launch of a (device, stream): barrier counters + partial sums"""
-    key = (device.index, torch.cuda.current_stream(device).cuda_stream)
-    ws = _bn_workspaces.get(key)
-    if ws is None or ws.numel() < nbytes:
-        ws = _bn_workspaces[key] = torch.zeros(max(int(nbytes), 1 << 18), dtype=torch.uint8, device=device)
-    return ws
-
-
-class _ConvBNTrain(torch.autograd.Function):
-    """act(bn(conv2d(x, Q(weight))) + residual) with batch statistics from the layer's prefetched operand: ONE launch
-    (po2_conv2d_bn_fwd_packed).  Backward: the norm's backward kernels on the saved conv output, then the conv's
-    data / weight gradients (straight-through to ``weight``)."""
-
-    @staticmethod
-    def forward(ctx, x, weight, residual, gamma, beta, slot, conv_cfg, bn, act):
-        from . import _lib, ops
-        stride, pad, groups, compute = conv_cfg
-        x = x.contiguous()
-        if residual is not None:
-            residual = residual.contiguous()
-        B, C, H, W_ = x.shape
-        K, _, R, S = slot.qw.shape
-        dev = x.device
-        lib = _lib.load()
-        track = bn.training and bn.track_running_stats
-        with torch.cuda.device(dev):
-            conv_out = torch.empty((B, K, (H + 2 * pad - R) // stride + 1, (W_ + 2 * pad - S) // stride + 1),
-                                   dtype=torch.float32, device=dev)
-            y = torch.empty_like(conv_out)
-            save_mean = torch.empty(K, dtype=torch.float32, device=dev)
-            save_invstd = torch.empty(K, dtype=torch.float32, device=dev)
-            stats = torch.empty(1, 2 * K + 1, dtype=torch.float32, device=dev)
-            ws = _conv_bn_workspace(dev, slot.bn_ws)
-            ops.LAUNCHES += 1
-            _p = lambda t: t.data_ptr() if t is not None else None
-            _lib.check(lib.po2_conv2d_bn_fwd_packed(
-                x.data_ptr(), slot.packed.data_ptr(), slot.scale.data_ptr(), conv_out.data_ptr(), y.data_ptr(), _p(residual),
-                _p(gamma), _p(beta), _p(bn.running_mean if track else None), _p(bn.running_var if track else None),
-                _p(bn.num_batches_tracked if track else None), float(bn.momentum if bn.momentum is not None else 0.0),
-                float(bn.eps), int(act), save_mean.data_ptr(), save_invstd.data_ptr(), stats.data_ptr(), B, C, H, W_, K, R, S,
-                stride, pad, groups, compute, ws.data_ptr(), ws.numel(), ops._stream_ptr(dev)), "po2_conv2d_bn_fwd_packed")
-        if track:
-            torch.autograd.graph.increment_version([bn.running_mean, bn.running_var, bn.num_batches_tracked])
-        ctx.save_for_backward(x, slot.qw, slot.scale, conv_out, y if act in (1, 2) else None, gamma, save_mean, save_invstd,
-                              stats, beta if act == 3 else None)
-        ctx.cfg = (stride, pad, groups, compute, int(act), residual is not None)
-        ctx.packed_d = getattr(slot, "packed_d", None)
-        ctx.weight = weight
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        from . import ops
-        from .batchnorm import bn_backward
-        x, qw, scale, conv_out, y, gamma, save_mean, save_invstd, stats, beta = ctx.saved_tensors
-        stride, pad, groups, compute, act, has_res = ctx.cfg
-        need_x, need_w, need_res, need_g, need_b = ctx.needs_input_grad[:5]
-        dconv, dres, dgamma, dbeta = bn_backward(dy, conv_out, y, gamma, beta, save_mean, save_invstd, stats, act,
-                                                 has_res and need_res)
-        wp = ctx.weight
-        defer = (wp.is_leaf and wp.grad is None and not wp._backward_hooks
-                 and not getattr(wp, "_post_accumulate_grad_hooks", None))
-        gx, gw = ops._conv_backward(dconv, x, qw, scale, stride, pad, groups, compute, need_x, need_w,
-                                    packed_d=ctx.packed_d, defer_w=defer)
-        return gx, gw, dres, dgamma if need_g else None, dbeta if need_b else None, None, None, None, None
-
-
-def _try_conv_bn_train(conv, bn, x, residual, act):
-    """the one-launch train-mode forward, or None when this layer / call does not qualify"""
-    from . import _lib, ops, prefetch
-    # opt-in (PO2_CONV_BN=1): measured on the ResNet-56 step the one-launch form LOSES to the separate kernels --
-    # 23-27 / 20-22 / 15.5 us per layer class against 16.5 / 15 / 13.1 (2.98 vs 2.67 ms per step): its passes over
-    # the accumulators run on the four epilogue warps of ONE CTA per SM (instruction-issue bound, ~1 us per tile),
-    # and fence + grid barrier + reading every CTA's partial sums cost another ~7 us that the norm kernel's
-    # per-channel barrier does not pay.  Kept for the record and for other shapes; see DESIGN.md section 4.3b.
-    if os.environ.get("PO2_CONV_BN", "0") != "1" or ops.get_conv_mode() != "tf32":
-        return None
-    if not (isinstance(bn, FusedSyncBatchNorm) and isinstance(conv, QuantizedConv2d) and bn.training and x.is_cuda
-            and x.dtype == torch.float32 and x.dim() == 4 and (bn.momentum is not None or not bn.track_running_stats)):
-        return None
-    if torch.distributed.is_available() and torch.distributed.is_initialized() and \
-            torch.distributed.get_world_size(bn.process_group) > 1 and os.environ.get("PO2_BN_EXCHANGE") != "local":
-        return None                                          # SyncBatchNorm across ranks: the norm kernels do the exchange
-    if act == 3 and residual is not None:
-        return None
-    if residual is not None and (residual.dtype != torch.float32 or not residual.is_cuda):
-        return None
-    slot = conv.__dict__.get("_po2_prefetch")
-    if not slot or slot.key != prefetch._layer_key(conv, x.shape, "tf32"):
-        return None
-    nb = getattr(slot, "bn_ws", None)
-    if nb is None:
-        B, C, H, W_ = x.shape
-        K, _, R, S = conv.weight.shape
-        nb = slot.bn_ws = int(_lib.load().po2_conv2d_bn_workspace(B, C, H, W_, K, R, S, conv.stride[0], conv.padding[0],
-                                                                  conv.groups, ops.COMPUTE["tf32"]))
-    if nb == 0:
-        return None
-    K = conv.weight.shape[0]
-    if residual is not None and tuple(residual.shape) != (x.shape[0], K, (x.shape[2] + 2 * conv.padding[0] - conv.weight.shape[2]) // conv.stride[0] + 1,
-                                                          (x.shape[3] + 2 * conv.padding[0] - conv.weight.shape[3]) // conv.stride[0] + 1):
-        return None
-    if x.numel() // x.shape[1] <= 1:
-        return None
-    prefetch.wait_for_quantizer(x.device)
-    return _ConvBNTrain.apply(x, conv.weight, residual, bn.weight, bn.bias, slot, (conv.stride[0], conv.padding[0], conv.groups,
-                                                                                  ops.COMPUTE["tf32"]), bn, act)
 
 
 class FoldedConvBN(nn.Module):

@@ -826,21 +826,6 @@ def conv2d_packed(x: torch.Tensor, packed: torch.Tensor, scale: Optional[torch.T
     return out
 
 
-def conv2d_packed_stats_out(x, packed, scale, out, K, R, S, stride, pad, groups, compute, sums) -> bool:
-    """out = conv2d(x, W) from the packed operand AND sums += per-channel (sum, sum of squares) of out -- the batch
-    statistics of the BatchNorm behind the conv, from the conv's own epilogue.  False: shape not taken."""
-    global LAUNCHES
-    B, C, H, W_ = x.shape
-    rc = _lib.load().po2_conv2d_fwd_packed_stats(x.data_ptr(), packed.data_ptr(), scale.data_ptr() if scale is not None else None,
-                                                 out.data_ptr(), B, C, H, W_, K, R, S, stride, pad, groups, compute,
-                                                 sums.data_ptr(), _stream_ptr(x.device))
-    if rc == -10:
-        return False
-    _lib.check(rc, "po2_conv2d_fwd_packed_stats")
-    LAUNCHES += 1
-    return True
-
-
 @conv2d_packed.register_fake
 def _(x, packed, scale, K, R, S, stride, pad, groups, compute):
     B, C, H, W_ = x.shape

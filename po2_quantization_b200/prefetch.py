@@ -25,7 +25,7 @@ from . import quantizers as _quantizers
 
 
 class _Slot:
-    __slots__ = ("key", "qw", "scale", "packed", "sse", "packed_d", "bn_ws")
+    __slots__ = ("key", "qw", "scale", "packed", "sse", "packed_d")
 
 
 class _Table:
@@ -259,23 +259,9 @@ class _QConvPrefetched(torch.autograd.Function):
     """conv2d(x, Q(weight)) from a prefetched (qw, scale, packed) triple; straight-through gradient"""
 
     @staticmethod
-    def forward(ctx, x, weight, qw, scale, packed, stride, pad, groups, compute, packed_d, stats=None):
+    def forward(ctx, x, weight, qw, scale, packed, stride, pad, groups, compute, packed_d):
         K, _, R, S = qw.shape
-        out = None
-        if stats is not None:
-            # the BatchNorm behind this conv asked for its batch statistics: the conv's epilogue accumulates the
-            # per-channel sums into stats["sums"] (stats["ok"] tells the norm whether that happened)
-            xc = x.contiguous()
-            B, C, H, W_ = xc.shape
-            cand = torch.empty((B, K, (H + 2 * pad - R) // stride + 1, (W_ + 2 * pad - S) // stride + 1),
-                               dtype=torch.float32, device=x.device)
-            with torch.cuda.device(x.device):
-                stats["ok"] = ops.conv2d_packed_stats_out(xc, packed, scale, cand, K, R, S, stride, pad, groups, compute,
-                                                          stats["sums"])
-            if stats["ok"]:
-                out = cand
-        if out is None:
-            out = ops.conv2d_packed(x, packed, scale, K, R, S, stride, pad, groups, compute)
+        out = ops.conv2d_packed(x, packed, scale, K, R, S, stride, pad, groups, compute)
         ctx.save_for_backward(x, qw, scale)
         ctx.packed_d = packed_d          # valid until the next prefetch launch, i.e. through this step's backward
         ctx.weight = weight              # the parameter: backward defers the weight gradient only if it has no .grad
@@ -293,19 +279,18 @@ class _QConvPrefetched(torch.autograd.Function):
                  and not getattr(wp, "_post_accumulate_grad_hooks", None))
         gx, gw = ops._conv_backward(g, x, qw, scale, stride, pad, groups, compute, ctx.needs_input_grad[0],
                                     ctx.needs_input_grad[1], packed_d=ctx.packed_d, defer_w=defer)
-        return gx, gw, None, None, None, None, None, None, None, None, None
+        return gx, gw, None, None, None, None, None, None, None, None
 
 
-def try_prefetched_forward(m, x, mode, stats=None):
-    """The layer's forward from its prefetched operand, or None if there is no valid one.  stats: {"sums": fp64
-    tensor} of the norm behind the layer; on return stats["ok"] says whether the conv accumulated them."""
+def try_prefetched_forward(m, x, mode):
+    """The layer's forward from its prefetched operand, or None if there is no valid one."""
     slot = m.__dict__.get("_po2_prefetch")
     if not slot or slot.key != _layer_key(m, x.shape, mode):
         return None
     if _pending_quantize:
         wait_for_quantizer(x.device)
     return _QConvPrefetched.apply(x, m.weight, slot.qw, slot.scale, slot.packed, m.stride[0], m.padding[0], m.groups,
-                                  ops.COMPUTE[mode], getattr(slot, "packed_d", None), stats)
+                                  ops.COMPUTE[mode], getattr(slot, "packed_d", None))
 
 
 def enable_weight_prefetch(model: torch.nn.Module) -> torch.nn.Module:

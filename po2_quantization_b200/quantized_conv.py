@@ -198,20 +198,6 @@ class QuantizedConv2d(nn.Conv2d):
         # no quantizer and no PTQ tag: a full-precision layer, i.e. plain nn.Conv2d (models/quantized_conv.py:38)
         return self._conv_forward(input, self.weight, self.bias)
 
-    def forward_with_stats(self, input, stats):
-        """forward(input) that, where the layer runs from a prefetched operand on the TMA-fed kernel, also
-        accumulates the batch statistics of the norm behind it (stats["sums"], fp64 [sum | sum of squares | ticket])
-        in the conv's epilogue; stats["ok"] reports whether it did."""
-        stats["ok"] = False
-        if self.quantize_fn is not None and _quantizers.quantizer_family(self.quantize_fn) is not None and self._po2_conv_ok(input):
-            mode = ops.get_conv_mode()
-            if mode == "tf32":
-                from . import prefetch
-                out = prefetch.try_prefetched_forward(self, input, mode, stats)
-                if out is not None:
-                    return out
-        return self.forward(input)
-
     def forward_folded(self, input, ep_a, ep_b, residual=None, act=0):
         """Inference forward with a per-out-channel affine (an eval-mode BatchNorm folded in), the residual add
         and the activation in the conv kernel's epilogue: act(conv(input) * ep_a + ep_b + residual).  Returns

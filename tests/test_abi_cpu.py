@@ -15,7 +15,7 @@ def _declared_symbols():
     return sorted(set(re.findall(r"\b(po2_[a-z0-9_]+)\s*\(", src)))
 
 
-def test_header_symbols_all_exported():
+def test_header_symbols_all_exported_abi_v2():
     from po2_quantization_b200 import _lib
     lib = _lib.load()
     syms = _declared_symbols()
@@ -23,7 +23,7 @@ def test_header_symbols_all_exported():
     for s in syms:
         assert hasattr(lib, s), f"{s} declared in include/po2_b200.h but not exported"
     assert sorted(_lib.SIGNATURES) == syms, "ctypes signatures out of sync with the header"
-    assert lib.po2_abi_version() == 1
+    assert lib.po2_abi_version() == 2
     assert lib.po2_workspace_bytes() >= 16
 
 

@@ -347,111 +347,6 @@ def test_mobilenet_and_mobilevit_fused_norm_state_dict_and_forward():
         torch.backends.cudnn.allow_tf32 = old_tf32
 
 
-@pytest.mark.parametrize("shape", [(128, 16, 32, 32), (128, 32, 16, 16), (128, 64, 8, 8), (6, 24, 8, 8)], ids=lambda s: "x".join(map(str, s)))
-def test_batch_statistics_from_the_conv_epilogue(shape, monkeypatch):
-    """Training on one rank: QuantizedConv2d's TMA-fed kernel accumulates the per-channel sum / sum of squares of its
-    output (fp64 atomics) and FusedSyncBatchNorm normalises from them in one launch (conv_bn_act).  Against the same
-    layers with the norm computing its own statistics: output, running statistics and all gradients."""
-    import copy
-    import po2_quantization_b200 as P
-    from po2_quantization_b200 import ops
-    monkeypatch.setenv("PO2_CONV_STATS", "1")          # opt-in (fp64 atomics: summation order is run-dependent)
-    B, C, H, W = shape
-    torch.manual_seed(C)
-    conv = P.QuantizedConv2d(C, C, 3, quantize_fn=P.PowerOfTwoQuantizer, bits=4).cuda()
-    bn = P.FusedSyncBatchNorm(C).cuda().train()
-    with torch.no_grad():
-        bn.weight.uniform_(0.5, 1.5); bn.bias.normal_(0, 0.2)
-    conv2, bn2 = copy.deepcopy(conv), copy.deepcopy(bn)
-    P.enable_weight_prefetch(conv)                    # the statistics ride on the prefetched single-launch forward
-    P.enable_weight_prefetch(conv2)
-    x = torch.randn(B, C, H, W, device="cuda") * 1.3 + 0.4
-    res = torch.randn(B, C, H, W, device="cuda")
-    go = torch.randn(B, C, H, W, device="cuda")
-    outs = []
-    for cv, b, use in ((conv, bn, True), (conv2, bn2, False)):
-        for it in range(2):                            # first call records the input shape, second runs prefetched
-            xi = x.clone().requires_grad_(True)
-            cv(xi)
-        cv.weight.grad = None
-        xi = x.clone().requires_grad_(True)
-        n0 = ops.LAUNCHES
-        if use:
-            y = P.conv_bn_act(cv, b, xi, res, True)
-        else:
-            y = b(cv(xi), res, True)
-        launches = ops.LAUNCHES - n0
-        y.backward(go)
-        outs.append((y.detach(), xi.grad, cv.weight.grad, b.weight.grad, b.bias.grad, b.running_mean.clone(), b.running_var.clone(), launches))
-    a, r = outs
-    assert a[7] <= r[7], (a[7], r[7])
-    for u, v, name in zip(a[:7], r[:7], ("y", "dx", "dw", "dgamma", "dbeta", "running_mean", "running_var")):
-        err = ((u - v).abs().max() / v.abs().max().clamp_min(1e-12)).item()
-        assert err < 2e-4, (name, err)
-    assert float(bn.conv_sums(x.device).abs().sum()) == 0.0   # consumed and zeroed for the next forward
-
-
-@pytest.mark.parametrize("case", [
-    dict(B=128, C=16, K=16, HW=32, k=3, res=True, act="relu"),      # ResNet-56 layer classes
-    dict(B=128, C=32, K=32, HW=16, k=3, res=False, act="relu"),
-    dict(B=128, C=64, K=64, HW=8, k=3, res=True, act="relu"),
-    dict(B=16, C=16, K=32, HW=32, k=3, res=False, act=None),        # fewer tiles than SMs, K != C
-    dict(B=32, C=32, K=64, HW=16, k=1, res=False, act="relu6"),     # 1x1
-    dict(B=8, C=16, K=16, HW=16, k=3, res=False, act="silu"),
-], ids=lambda c: "_".join(f"{k}{v}" for k, v in c.items()))
-def test_conv_and_train_mode_norm_in_one_launch(case, monkeypatch):
-    """conv_bn_act in train(): conv + batch statistics + normalise (+ residual add, + activation) as ONE cooperative
-    launch of the TMA-fed kernel (po2_conv2d_bn_fwd_packed) against the separate conv and norm kernels: output,
-    every gradient, the running statistics -- and bit-identical results from one call to the next."""
-    import po2_quantization_b200 as P
-    from po2_quantization_b200 import ops
-    B, C, K, HW, k = case["B"], case["C"], case["K"], case["HW"], case["k"]
-    torch.manual_seed(B + C + K + HW)
-    conv = P.QuantizedConv2d(C, K, k, stride=1, padding=k // 2, bias=False, quantize_fn=P.PowerOfTwoQuantizer, bits=4).cuda()
-    bn = P.FusedSyncBatchNorm(K, act=case["act"] if case["act"] != "relu" else None).cuda().train()
-    relu = case["act"] == "relu"
-    with torch.no_grad():
-        bn.weight.copy_(torch.rand(K, device="cuda") + 0.5)
-        bn.bias.copy_(torch.randn(K, device="cuda") * 0.3)
-    x0 = torch.randn(B, C, HW, HW, device="cuda") + 0.2
-    r0 = torch.randn(B, K, HW, HW, device="cuda") if case["res"] else None
-    go = torch.randn(B, K, HW, HW, device="cuda")
-    ops.set_conv_mode("tf32")
-
-    def run(fused):
-        monkeypatch.setenv("PO2_CONV_BN", "1" if fused else "0")
-        bn.running_mean.zero_(); bn.running_var.fill_(1.0); bn.num_batches_tracked.zero_()
-        for m in (conv, bn):
-            m.zero_grad(set_to_none=True)
-        x = x0.clone().requires_grad_(True)
-        r = r0.clone().requires_grad_(True) if r0 is not None else None
-        P.prefetch_weights([conv])
-        before = ops.LAUNCHES
-        y = P.conv_bn_act(conv, bn, x, r, relu)
-        fwd = ops.LAUNCHES - before
-        y.backward(go)
-        torch.cuda.synchronize()
-        return dict(y=y.detach(), gx=x.grad, gr=r.grad if r is not None else None, gw=conv.weight.grad.clone(),
-                    gg=bn.weight.grad.clone(), gb=bn.bias.grad.clone(), rm=bn.running_mean.clone(), rv=bn.running_var.clone(),
-                    nbt=int(bn.num_batches_tracked)), fwd
-
-    try:
-        run(False)                                           # records the input shape for the prefetch
-        want, fwd_sep = run(False)
-        got, fwd_one = run(True)
-        again, _ = run(True)
-    finally:
-        ops.set_conv_mode(ops.DEFAULT_CONV_MODE)
-    assert fwd_one == 1 and fwd_sep >= 2, (fwd_one, fwd_sep)
-    assert got["nbt"] == want["nbt"] == 1
-    for key in ("y", "gx", "gr", "gw", "gg", "gb", "rm", "rv"):
-        if want[key] is None:
-            assert got[key] is None
-            continue
-        assert _rel(got[key], want[key]) < 2e-5, key
-        assert torch.equal(got[key], again[key]), key        # deterministic: fixed-order partial sums
-
-
 def test_skip_connection_gradient_is_added_inside_the_norm_kernels(monkeypatch):
     """A residual block's input receives two gradients: the conv branch's and the skip connection's.  With the
     FusedSyncBatchNorm modules of workloads/resnet_cifar.py the second one is left at the producing norm's autograd

@@ -13,11 +13,11 @@ import torch.nn.functional as F
 
 def conv_bn_act(conv, bn, x, residual=None, relu=False):
     """relu(bn(conv(x)) + residual).  With this repo's classes (po2_quantization_b200/fold.py): at inference the
-    norm, the add and the ReLU are folded into the conv kernel's epilogue (one launch); in training on one rank
-    the conv's epilogue accumulates the norm's batch statistics, so the norm is a single normalising pass."""
+    norm, the add and the ReLU are folded into the conv kernel's epilogue (one launch); in training the conv runs,
+    then the norm computes its batch statistics and normalises (+ add, + ReLU), in one launch where the tensor fits."""
     if getattr(bn, "fused_residual_relu", False):
-        from po2_quantization_b200 import conv_bn_act as fused                # inference: folded; training: the conv's
-        return fused(conv, bn, x, residual, relu)                             # epilogue supplies the batch statistics
+        from po2_quantization_b200 import conv_bn_act as fused                # inference: folded; training: conv,
+        return fused(conv, bn, x, residual, relu)                             # then the one-launch norm
     return bn_act(bn, conv(x), residual, relu)
 
 
