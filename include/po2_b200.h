@@ -216,7 +216,10 @@ int po2_conv2d_depthwise_wgrad(const void* g, const void* x, void* gw, int B, in
 size_t po2_conv2d_wgrad_workspace(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
                                   int compute);
 /* planning query: 0 = shape not taken (the caller keeps aten.convolution_backward), 1 = tcgen05 kernel with
- * bf16 operands, 2 = the TMA-fed tf32 kernel (compute == 2, dense stride-1 3x3 with W in {4,8,16,32} / 1x1) */
+ * bf16 operands, 2 = the TMA-fed tf32 kernel (compute == 2, dense stride-1 3x3 with W in {4,8,16,32} / 1x1),
+ * 3 = fp32 CUDA-core GEMM for the 1x1 stride-1 layers neither tensor-core kernel takes (K > 128 or C > 256) that
+ * are small: B*H*W <= 8192 and B*H*W*C*K <= 2^26, compute 0 or 2, exact fp32 FMA, per-CTA partials summed in a fixed order
+ * (deterministic); its workspace (never 0) holds the partials.  Answers without a device. */
 int po2_conv2d_wgrad_kernel_kind(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
                                  int compute);
 /* po2_conv2d_wgrad_z: the same as po2_conv2d_wgrad with `zeroed_tickets` = 8 bytes of device memory that are zero

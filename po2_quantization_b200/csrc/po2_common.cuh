@@ -203,6 +203,13 @@ int launch_wgrad_reduce(const float* partial, float* gw, int nparts, int K, int 
 bool pw_small_takes(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups);
 int launch_pw_small(const float* x, const float* w, float* out, int B, int C, int HW, int K, const ConvEpilogue& ep,
                     cudaStream_t st);
+// csrc/po2_conv_bwd.cu: the weight gradient of 1x1 stride-1 layers with B*H*W <= 8192 and B*H*W*C*K <= 2^26 -- fp32
+// split-reduction GEMM
+// + the fixed-order reduce kernel (two launches); the workspace holds the partials
+bool pw_wgrad_takes(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups, int compute);
+size_t pw_wgrad_partial_bytes(int B, int C, int H, int W, int K);
+int launch_pw_wgrad(const float* g, const float* x, float* gw, void* workspace, int B, int C, int HW, int K,
+                    cudaStream_t st);
 
 // ---- per-device one-time host state ---------------------------------------------------------------
 // Kernel attributes (cudaFuncSetAttribute) and the SM count belong to a DEVICE, not to the process:

@@ -1803,18 +1803,23 @@ size_t po2_conv2d_wgrad_workspace(int B, int C, int H, int W, int K, int R, int 
     return (wgrad_tma_partial_bytes(wp) + 255) / 256 * 256;
   ConvGeom g;
   WgGeom wg;
-  if (!wgrad_plan(g, wg, B, C, H, W, K, R, S, stride, pad, groups, compute == 2 ? 0 : compute)) return 0;
-  return (wgrad_partial_bytes(g, wg) + 255) / 256 * 256;
+  if (wgrad_plan(g, wg, B, C, H, W, K, R, S, stride, pad, groups, compute == 2 ? 0 : compute))
+    return (wgrad_partial_bytes(g, wg) + 255) / 256 * 256;
+  if (pw_wgrad_takes(B, C, H, W, K, R, S, stride, pad, groups, compute))
+    return (pw_wgrad_partial_bytes(B, C, H, W, K) + 255) / 256 * 256;
+  return 0;
 }
 
-// 0: not taken (aten), 1: bf16-operand tcgen05 kernel (K5), 2: TMA-fed tf32 kernel (K5T)
+// 0: not taken (aten), 1: bf16-operand tcgen05 kernel (K5), 2: TMA-fed tf32 kernel (K5T), 3: fp32 CUDA-core GEMM of
+// the small 1x1 layers that neither K5T nor K5 takes (csrc/po2_conv_bwd.cu, conv_wgrad_pw_kernel)
 int po2_conv2d_wgrad_kernel_kind(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
                                  int compute) {
   WgTmaPlan wp;
   if (wgrad_tma_plan(wp, B, C, H, W, K, R, S, stride, pad, groups, compute)) return 2;
   ConvGeom g;
   WgGeom wg;
-  return wgrad_plan(g, wg, B, C, H, W, K, R, S, stride, pad, groups, compute == 2 ? 0 : compute) ? 1 : 0;
+  if (wgrad_plan(g, wg, B, C, H, W, K, R, S, stride, pad, groups, compute == 2 ? 0 : compute)) return 1;
+  return pw_wgrad_takes(B, C, H, W, K, R, S, stride, pad, groups, compute) ? 3 : 0;
 }
 
 int po2_conv2d_wgrad(const void* g_out, const void* x, void* gw, int B, int C, int H, int W, int K, int R, int S,
@@ -1847,7 +1852,12 @@ int po2_conv2d_wgrad_z(const void* g_out, const void* x, void* gw, int B, int C,
   }
   ConvGeom g;
   WgGeom wg;
-  if (!wgrad_plan(g, wg, B, C, H, W, K, R, S, stride, pad, groups, compute == 2 ? 0 : compute)) return PO2_E_UNSUPPORTED;
+  if (!wgrad_plan(g, wg, B, C, H, W, K, R, S, stride, pad, groups, compute == 2 ? 0 : compute)) {
+    if (!pw_wgrad_takes(B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_UNSUPPORTED;
+    if (!workspace || workspace_bytes < pw_wgrad_partial_bytes(B, C, H, W, K)) return PO2_E_WORKSPACE;
+    return launch_pw_wgrad((const float*)g_out, (const float*)x, (float*)gw, workspace, B, C, H * W, K,
+                           (cudaStream_t)stream);
+  }
   const size_t need = wgrad_partial_bytes(g, wg);
   if (!workspace || workspace_bytes < need) return PO2_E_WORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;

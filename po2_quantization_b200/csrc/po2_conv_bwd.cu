@@ -470,4 +470,152 @@ int launch_pw_small(const float* x, const float* w, float* out, int B, int C, in
   return (int)cudaLaunchKernelEx(&cfg, conv_pw_small_kernel, x, w, out, g, ep);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Weight gradient of the same small pointwise layers, and of every 1x1 stride-1 layer with a short reduction that is
+// wider than the tcgen05 weight-gradient kernels take (K > 128 output or C > 256 input channels: MobileNetV2's
+// expansion / projection layers, MobileViT's 1x1 layers at 32x32):
+//   gw[k][c] = sum_{m = (image, pixel)} g[n][k][p] * x[n][c][p],   m < B*HW <= PWW_MAX_M
+// a GEMM with up to 960 x 960 outputs, a reduction of at most 8192 and at most 2^26 multiply-adds (MobileNetV2's
+// largest: 39 M).  Beyond that cuDNN's tensor-core kernels win (measured on a B200: 24->144 at B*H*W = 16384
+// 20.2 against 16.4 us, 160->960 at 8192 170 against 45 us).  fp32 CUDA cores, exact fmaf (no operand
+// rounding).  CTA (k tile, c tile, split) = 64 x 64 outputs, 256 threads with 4 x 4 accumulators each, summing
+// the contiguous range of 16-pixel chunks of its split; the reduction is split over blockIdx.z so that a small K x C
+// still fills the SMs.  Every CTA writes its partial tile [split][k][c]; conv_wgrad_reduce_kernel (ntaps = 1,
+// launched programmatically behind this grid) adds the splits in a fixed order: deterministic, no atomics.
+// ------------------------------------------------------------------------------------------------
+constexpr int PWW_TK = 64, PWW_TC = 64, PWW_TM = 16, PWW_THREADS = 256;
+constexpr int PWW_MAX_M = 8192;            // B*HW: MobileNetV2's largest reduction (24->144 @8x8, batch 128)
+constexpr int64_t PWW_MAX_FMA = 1ll << 26;  // B*HW*C*K
+
+struct PwWgGeom {
+  int M, C, K, HW;
+  int chunks_per_split;                    // 16-pixel chunks summed by one CTA
+  int vec;                                 // HW % 4 == 0 and 16-byte aligned operands: 128-bit loads
+  int vst;                                 // C % 4 == 0 and a 16-byte aligned workspace: 128-bit partial stores
+  FastDiv div_hw;
+};
+
+__global__ void __launch_bounds__(PWW_THREADS) conv_wgrad_pw_kernel(const float* __restrict__ g,
+                                                                    const float* __restrict__ x,
+                                                                    float* __restrict__ partial, PwWgGeom q) {
+  __shared__ __align__(16) float Gs[PWW_TM][PWW_TK + 4];   // [m][k]
+  __shared__ __align__(16) float Xs[PWW_TM][PWW_TC + 4];   // [m][c]
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // the reduce kernel waits for this grid's completion
+  const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
+  const int k0 = blockIdx.x * PWW_TK, c0 = blockIdx.y * PWW_TC;
+  const int M = q.M, C = q.C, K = q.K, HW = q.HW;
+  const int m_begin = blockIdx.z * q.chunks_per_split * PWW_TM;
+  const int m_end = min(M, m_begin + q.chunks_per_split * PWW_TM);
+  float acc[4][4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+#pragma unroll
+    for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
+  // loader role: channel lane = tid % 64 of both tiles, pixels (tid / 64) * 4 .. +3 of the chunk.  Consecutive lanes
+  // read consecutive channels: one 128-byte line per warp when HW == 1, 128-bit vectors along the pixels otherwise.
+  const int lch = tid & 63, lm = (tid >> 6) * 4;
+  const int lk = k0 + lch, lc = c0 + lch;
+  float gv[4], xv[4];
+  auto load_chunk = [&](int m0) {
+    const int m = m0 + lm;
+    if (q.vec) {                            // the quad m .. m + 3 lies in one image (HW % 4 == 0, m % 4 == 0)
+      float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
+      if (m < m_end) {
+        const int n = fdiv(m, q.div_hw), p = m - n * HW;
+        if (lk < K) a = __ldg(reinterpret_cast<const float4*>(g + ((size_t)n * K + lk) * HW + p));
+        if (lc < C) b = __ldg(reinterpret_cast<const float4*>(x + ((size_t)n * C + lc) * HW + p));
+      }
+      gv[0] = a.x; gv[1] = a.y; gv[2] = a.z; gv[3] = a.w;
+      xv[0] = b.x; xv[1] = b.y; xv[2] = b.z; xv[3] = b.w;
+    } else {
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        float a = 0.f, b = 0.f;
+        if (m + e < m_end) {
+          const int n = fdiv(m + e, q.div_hw), p = m + e - n * HW;
+          if (lk < K) a = __ldg(g + ((size_t)n * K + lk) * HW + p);
+          if (lc < C) b = __ldg(x + ((size_t)n * C + lc) * HW + p);
+        }
+        gv[e] = a; xv[e] = b;
+      }
+    }
+  };
+  int m0 = m_begin;
+  if (m0 < m_end) load_chunk(m0);
+  for (; m0 < m_end; m0 += PWW_TM) {
+    __syncthreads();                                        // the previous chunk has been consumed
+#pragma unroll
+    for (int e = 0; e < 4; ++e) { Gs[lm + e][lch] = gv[e]; Xs[lm + e][lch] = xv[e]; }
+    __syncthreads();
+    if (m0 + PWW_TM < m_end) load_chunk(m0 + PWW_TM);       // the next chunk's loads fly during this chunk's FMAs
+#pragma unroll
+    for (int mm = 0; mm < PWW_TM; ++mm) {
+      const float4 a4 = *reinterpret_cast<const float4*>(&Gs[mm][ty * 4]);
+      const float4 b4 = *reinterpret_cast<const float4*>(&Xs[mm][tx * 4]);
+      const float a[4] = {a4.x, a4.y, a4.z, a4.w}, b[4] = {b4.x, b4.y, b4.z, b4.w};
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
+    }
+  }
+  const int c = c0 + tx * 4;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int k = k0 + ty * 4 + i;
+    if (k >= K || c >= C) continue;
+    float* dst = partial + ((size_t)blockIdx.z * K + k) * C + c;
+    if (q.vst) {
+      *reinterpret_cast<float4*>(dst) = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
+    } else {
+#pragma unroll
+      for (int j = 0; j < 4; ++j)
+        if (c + j < C) dst[j] = acc[i][j];
+    }
+  }
+}
+
+// 1x1 stride-1 dense layers small enough for one CUDA-core GEMM (compute 0 / 2: the fp32 mode's backward is
+// aten.convolution_backward by design)
+bool pw_wgrad_takes(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups, int compute) {
+  if (R != 1 || S != 1 || stride != 1 || pad != 0 || groups != 1 || !(compute == 0 || compute == 2)) return false;
+  if (B < 1 || C < 1 || H < 1 || W < 1 || K < 1) return false;
+  const int64_t M = (int64_t)B * H * W;
+  return M <= PWW_MAX_M && M * C * K <= PWW_MAX_FMA;
+}
+
+// splits of the reduction: about two CTAs per SM, every CTA at least four 16-pixel chunks, and every split non-empty
+// (a pure function of the shape and the SM count, so the summation order -- the bits -- is too)
+static void pw_wgrad_split(int M, int C, int K, int& splits, int& chunks_per_split) {
+  const int tiles = ((K + PWW_TK - 1) / PWW_TK) * ((C + PWW_TC - 1) / PWW_TC);
+  const int chunks = (M + PWW_TM - 1) / PWW_TM;
+  int want = (2 * device_sm_count() + tiles - 1) / tiles;
+  if (want > chunks / 4) want = chunks / 4;
+  if (want < 1) want = 1;
+  chunks_per_split = (chunks + want - 1) / want;
+  splits = (chunks + chunks_per_split - 1) / chunks_per_split;
+}
+
+size_t pw_wgrad_partial_bytes(int B, int C, int H, int W, int K) {
+  int splits, cps;
+  pw_wgrad_split(B * H * W, C, K, splits, cps);
+  return (size_t)splits * K * C * sizeof(float);
+}
+
+int launch_pw_wgrad(const float* g, const float* x, float* gw, void* workspace, int B, int C, int HW, int K,
+                    cudaStream_t st) {
+  PwWgGeom q;
+  q.M = B * HW; q.C = C; q.K = K; q.HW = HW;
+  q.div_hw = make_fastdiv((uint32_t)HW);
+  q.vec = HW % 4 == 0 && (reinterpret_cast<uintptr_t>(g) & 15) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0;
+  q.vst = C % 4 == 0 && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0;
+  int splits;
+  pw_wgrad_split(q.M, C, K, splits, q.chunks_per_split);
+  const dim3 grid((unsigned)((K + PWW_TK - 1) / PWW_TK), (unsigned)((C + PWW_TC - 1) / PWW_TC), (unsigned)splits);
+  conv_wgrad_pw_kernel<<<grid, PWW_THREADS, 0, st>>>(g, x, (float*)workspace, q);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return (int)e;
+  return launch_wgrad_reduce((const float*)workspace, gw, splits, K, C, 1, st);
+}
+
 }  // namespace po2

@@ -355,7 +355,8 @@ def conv2d_dgrad_out(g, w, scale, gx, pad, compute: int = 0) -> bool:
 
 
 # "tc": weight gradient of stride-1 dense convs (K <= 128) on the tensor-core kernel (x and grad rounded
-# to bf16, fp32 accumulation, deterministic); "aten": aten.convolution_backward (cuDNN)
+# to bf16, fp32 accumulation, deterministic), and of small wider 1x1 layers (B*H*W <= 8192, B*H*W*C*K <= 2^26) on
+# the exact-fp32 CUDA-core GEMM (deterministic); "aten": aten.convolution_backward (cuDNN)
 _wgrad_mode = os.environ.get("PO2_CONV_WGRAD", "tc")
 
 
@@ -367,7 +368,10 @@ def set_wgrad_mode(mode: str) -> None:
 
 
 def conv2d_wgrad_out(g, x, gw, pad, compute: int = 0) -> bool:
-    """gw = dL/dW of conv2d(x, W) (stride 1, dense) from g = dL/dout.  False if the shape is not taken."""
+    """gw = dL/dW of conv2d(x, W) (stride 1, dense) from g = dL/dout.  False if the shape is not taken.
+    The library picks the kernel (po2_conv2d_wgrad_kernel_kind): 2 = K5T (tf32 operands, compute 2), 1 = K5 (bf16
+    operands), 3 = the fp32 CUDA-core GEMM of 1x1 layers wider than K5T / K5 take, with B*H*W <= 8192 and
+    B*H*W*C*K <= 2^26.  Each is the main kernel + the fixed-order reduce kernel (two launches)."""
     global LAUNCHES
     lib = _lib.load()
     check_conv_shapes(x.shape, gw.shape, 1, pad)
@@ -419,10 +423,10 @@ _wgrad_tickets = {}
 
 # ---- weight gradients on a second stream --------------------------------------------------------------------
 # The weight gradient of a layer is a leaf of the backward pass: nothing before the optimizer reads it.  With the
-# overlap on, K5T / K5 (+ their reduce kernel) are launched on a per-device side stream that forks from the
-# backward stream where the layer's output gradient exists, and the backward stream goes on to the data gradient
-# and the norm kernels of the layers below; one join is queued on the autograd engine for the end of the backward
-# pass.  Inside a CUDA-graph capture the side stream is a parallel branch of the graph.
+# overlap on, K5T / K5 / the pointwise GEMM (+ their reduce kernel) are launched on a per-device side stream that
+# forks from the backward stream where the layer's output gradient exists, and the backward stream goes on to the
+# data gradient and the norm kernels of the layers below; one join is queued on the autograd engine for the end of
+# the backward pass.  Inside a CUDA-graph capture the side stream is a parallel branch of the graph.
 _wgrad_overlap = os.environ.get("PO2_WGRAD_STREAM", "0") == "1"
 _side_streams = {}
 _side_pending = {}
@@ -516,9 +520,9 @@ def _depthwise_backward(g_full, x, w, need_x, need_w):
 
 def _conv_backward(g, x, w, scale, stride, pad, groups, compute, need_x, need_w, packed_d=None, defer_w=False):
     """(gx, gw) of conv2d(x, w) on our kernels: dense layers on the tcgen05 kernels (data gradient: the forward
-    kernel with transposed weights; weight gradient: K5T / K5) -- stride-2 layers through the zero-inserted
-    output gradient, which turns both into stride-1 problems -- and depthwise 3x3 layers on the CUDA-core
-    kernels of csrc/po2_conv_bwd.cu.  Whatever is left goes through aten.convolution_backward, loudly."""
+    kernel with transposed weights; weight gradient: K5T / K5, or the fp32 GEMM for small wide 1x1 layers) --
+    stride-2 layers through the zero-inserted output gradient, which turns both into stride-1 problems -- and
+    depthwise 3x3 layers on the CUDA-core kernels of csrc/po2_conv_bwd.cu.  Whatever is left goes through aten.convolution_backward, loudly."""
     g = g.contiguous()
     gx = gw = None
     B, C, H, W_ = x.shape
