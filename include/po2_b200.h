@@ -14,6 +14,15 @@
  *     synchronised, and is CUDA-graph capturable;
  *   - return value: 0 = success, > 0 = a cudaError_t from the launch, < 0 = PO2_E_* argument
  *     error.  Nothing throws or exits;
+ *   - alignment: any 4-byte-aligned fp32 tensor is accepted, except where the kernel a conv entry point
+ *     picks reads it with 128-bit loads or a tensor map.  Then po2_conv2d_fwd(_ep), po2_conv2d_fwd_packed(_ep),
+ *     po2_qconv2d_fwd, po2_conv2d_dgrad(_packed) and po2_conv2d_wgrad(_z) return PO2_E_ALIGN, before any
+ *     launch, unless x (the output gradient for the data gradient; both x and the output gradient for the
+ *     weight gradient) starts on a 16-byte boundary.  That is the tcgen05 forward / data gradient at
+ *     stride 1 with W % 4 == 0 (W = H*W for 1x1), or on a 1x1 feature map with C % 4 == 0, and the
+ *     tcgen05 weight gradients (po2_conv2d_wgrad_kernel_kind 1 or 2) at W % 4 == 0.  The direct,
+ *     depthwise and small-pointwise kernels take x at any alignment; the small-pointwise one
+ *     (po2_conv2d_kernel_kind 4) needs a 16-byte-aligned fp32 weight when C % 4 == 0;
  *   - re-entrant; the only process-global state is lazily cached device attributes;
  *   - element counts are 64-bit (the quantizer sweep reaches 2^32 elements).
  */

@@ -907,9 +907,20 @@ static bool pdl_chain_enabled() {
   static const bool on = []() { const char* e = getenv("PO2_CONV_PDL_CHAIN"); return !(e && e[0] == '0'); }();
   return on;
 }
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+// K3's activation producers read x with 128-bit loads on the vec4 path (stride 1, W % 4 == 0) and on the hw1 path
+// (1x1 feature map, C % 4 == 0); K3T's tensor map needs a 16-byte-aligned base too, and every geometry plan_tma
+// takes is stride 1 with W % 4 == 0, i.e. has vec4 set.  PO2_E_ALIGN before any launch when x does not allow that.
+static int umma_check_x(const void* x, const ConvGeom& g) {
+  const bool wide_loads = g.vec4 || (g.H * g.W == 1 && g.C % 4 == 0);
+  return (wide_loads && !aligned16(x)) ? PO2_E_ALIGN : 0;
+}
+
 static int launch_umma(const void* x, const void* w, const float* scale, void* out, ConvGeom& g, int w_format,
                        int bits, int fsr, int transpose, void* pack_buf, cudaStream_t st, bool pdl = true,
                        const ConvEpilogue& ep = ConvEpilogue{nullptr, nullptr, nullptr, 0}, bool chain = false) {
+  if (int a = umma_check_x(x, g)) return a;
   {
     uint8_t* Bp = reinterpret_cast<uint8_t*>(pack_buf);
     cudaError_t e = cudaSuccess;
@@ -925,8 +936,8 @@ static int launch_umma(const void* x, const void* w, const float* scale, void* o
     {                                                     // K3T where the shape allows: activations by tensor-map TMA
       TmaPlan tp;
       if (g.tf32 && tma_enabled() && plan_tma(g, tp)) {
-        // (the operand may already be packed in K3T's layout: an x that cannot be described by a tensor map --
-        // misaligned -- is an error here, not a fallback)
+        // (the operand may already be packed in K3T's layout: an x that cannot be described by a tensor map is an
+        // error here, not a fallback; a misaligned one was refused above with PO2_E_ALIGN)
         return launch_tma(x, Bp, scale, out, g, tp, st, (chain && transpose < 0 && pdl_chain_enabled()) ? 2 : (pdl ? 1 : 0), ep);
       }
     }
@@ -1427,6 +1438,10 @@ int po2_conv2d_fwd_ep(const void* x, const void* w, const float* scale, void* ou
     if (!workspace || workspace_bytes < need) return PO2_E_WORKSPACE;
     return launch_umma(x, w, scale, out, g, w_format, bits, fsr, 0, reinterpret_cast<char*>(workspace) + wbytes, st, true, ep);
   }
+  // the small-pointwise GEMM reads rows of the fp32 weight with 128-bit loads when C % 4 == 0
+  if (pw_small_takes(B, C, H, W, K, R, S, stride, pad, groups) && C % 4 == 0 &&
+      !aligned16(w_format == PO2_W_CODES ? workspace : w))
+    return PO2_E_ALIGN;
   // CUDA-core paths work on fp32 weights
   const float* wf = (const float*)w;
   if (w_format == PO2_W_CODES) {
@@ -1558,7 +1573,10 @@ int po2_qconv2d_fwd(const void* x, const void* w_master, void* qw_out, float* sc
   if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t wn = (int64_t)K * (C / groups) * R * S;
-  if (compute != 1 && umma_eligible(g) && plan_umma(g, compute == 2) && g.Cpad == C && g.ntiles_n * g.NT == K) {
+  const bool umma = compute != 1 && umma_eligible(g) && plan_umma(g, compute == 2);
+  if (umma)
+    if (int a = umma_check_x(x, g)) return a;                 // before the quantizer runs
+  if (umma && g.Cpad == C && g.ntiles_n * g.NT == K) {
     const size_t need = po2_conv2d_workspace(B, C, H, W, K, R, S, stride, pad, groups, compute);
     const size_t wbytes = ((size_t)wn * sizeof(float) + 255) / 256 * 256;
     if (!workspace || workspace_bytes < need) return PO2_E_WORKSPACE;
@@ -1846,6 +1864,7 @@ int po2_conv2d_wgrad_z(const void* g_out, const void* x, void* gw, int B, int C,
       // than the 1152-CTA reduce kernel (the cooperative launch itself is free: the fused BatchNorm kernels run the
       // same with a plain launch).  Opt-in only (PO2_WGRAD_FUSED_REDUCE=1).
       static const bool fuse = [] { const char* e = getenv("PO2_WGRAD_FUSED_REDUCE"); return e && e[0] == '1'; }();
+      if (!aligned16(g_out) || !aligned16(x)) return PO2_E_ALIGN;          // the bases of both tensor maps
       return launch_wgrad_tma(g_out, x, gw, workspace, wp, (cudaStream_t)stream,
                               fuse ? (unsigned int*)zeroed_tickets : nullptr);
     }
@@ -1860,6 +1879,7 @@ int po2_conv2d_wgrad_z(const void* g_out, const void* x, void* gw, int B, int C,
   }
   const size_t need = wgrad_partial_bytes(g, wg);
   if (!workspace || workspace_bytes < need) return PO2_E_WORKSPACE;
+  if (g.vec4 && (!aligned16(g_out) || !aligned16(x))) return PO2_E_ALIGN;   // produce_planes_bf16: 128-bit loads
   cudaStream_t st = (cudaStream_t)stream;
   static PerDeviceOnce wgrad_once;
   if (cudaError_t e0 = wgrad_once.run([]() -> cudaError_t {

@@ -39,6 +39,13 @@ def _require_cuda(t: torch.Tensor, what: str) -> None:
         raise TypeError(f"{what}: unsupported dtype {t.dtype} (float32, bfloat16, float16)")
 
 
+def _aligned16(t: torch.Tensor) -> torch.Tensor:
+    """t, or a copy of it when its data does not start on a 16-byte boundary.  A contiguous view can start at any
+    element (``buf[1:].view(...)``); the tensor-core conv kernels read activations with 128-bit loads or tensor maps
+    and the library refuses such a pointer (PO2_E_ALIGN), so the ops accept every input nn.Conv2d accepts."""
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
 _workspaces = {}
 
 # ---- library paths taken instead of our kernels are never silent ------------------------------------
@@ -306,8 +313,8 @@ def conv2d(x: torch.Tensor, w: torch.Tensor, scale: Optional[torch.Tensor], stri
     if x.dtype != torch.float32 or w.dtype != torch.float32:
         raise TypeError("po2::conv2d: fp32 NCHW activations and fp32 weights only")
     check_conv_shapes(x.shape, w.shape, groups, pad)
-    x = x.contiguous()
-    w = w.contiguous()
+    x = _aligned16(x.contiguous())
+    w = _aligned16(w.contiguous())
     out = torch.empty(_conv_out_shape(x, w, stride, pad), dtype=torch.float32, device=x.device)
     with torch.cuda.device(x.device):
         conv2d_out(x, w, scale, out, stride, pad, groups, compute)
@@ -523,7 +530,8 @@ def _conv_backward(g, x, w, scale, stride, pad, groups, compute, need_x, need_w,
     kernel with transposed weights; weight gradient: K5T / K5, or the fp32 GEMM for small wide 1x1 layers) --
     stride-2 layers through the zero-inserted output gradient, which turns both into stride-1 problems -- and
     depthwise 3x3 layers on the CUDA-core kernels of csrc/po2_conv_bwd.cu.  Whatever is left goes through aten.convolution_backward, loudly."""
-    g = g.contiguous()
+    g = _aligned16(g.contiguous())
+    x = _aligned16(x.contiguous())
     gx = gw = None
     B, C, H, W_ = x.shape
     K, _, R, S = w.shape
@@ -541,7 +549,7 @@ def _conv_backward(g, x, w, scale, stride, pad, groups, compute, need_x, need_w,
         elif stride == 2:
             ours = depthwise = False
         if depthwise:
-            gx, gw = _depthwise_backward(g_s1, x.contiguous(), w.contiguous(), need_x, need_w)
+            gx, gw = _depthwise_backward(g_s1, x, w.contiguous(), need_x, need_w)
         else:
             defer_w = defer_w and _wgrad_overlap and need_w and ours and _wgrad_mode == "tc" and \
                 torch._C._current_graph_task_id() >= 0
@@ -562,11 +570,10 @@ def _conv_backward(g, x, w, scale, stride, pad, groups, compute, need_x, need_w,
                 # tf32 mode: the TMA-fed tf32 kernel where the shape allows; elsewhere the library takes the
                 # bf16-operand kernel (the weight gradient is a leaf of the backward pass: its rounding does not
                 # propagate into other layers' gradients, unlike the data gradient)
-                xc = x.contiguous()
                 if defer_w:
-                    if _wgrad_on_side_stream(g_s1, xc, cand, pad, compute, ready):
+                    if _wgrad_on_side_stream(g_s1, x, cand, pad, compute, ready):
                         gw = cand
-                elif conv2d_wgrad_out(g_s1, xc, cand, pad, compute):
+                elif conv2d_wgrad_out(g_s1, x, cand, pad, compute):
                     gw = cand
     if (need_x and gx is None) or (need_w and gw is None):
         if x.is_cuda and _conv_mode != "cudnn":
@@ -641,7 +648,7 @@ def qconv2d(x: torch.Tensor, weight: torch.Tensor, bits: int, fsr: int, plus: bo
     if x.dtype != torch.float32 or weight.dtype != torch.float32:
         raise TypeError("po2::qconv2d: fp32 NCHW activations and fp32 weights only")
     check_conv_shapes(x.shape, weight.shape, groups, pad)
-    x = x.contiguous()
+    x = _aligned16(x.contiguous())
     w = weight.contiguous()
     lib = _lib.load()
     B, C, H, W_ = x.shape
@@ -723,7 +730,7 @@ def lin_qconv2d(x: torch.Tensor, weight: torch.Tensor, bits: int, plus: bool, st
     if x.dtype != torch.float32 or weight.dtype != torch.float32:
         raise TypeError("po2::lin_qconv2d: fp32 NCHW activations and fp32 weights only")
     check_conv_shapes(x.shape, weight.shape, groups, pad)
-    x = x.contiguous()
+    x = _aligned16(x.contiguous())
     w = weight.contiguous()
     lib = _lib.load()
     B, C, H, W_ = x.shape
@@ -811,7 +818,7 @@ def conv2d_packed(x: torch.Tensor, packed: torch.Tensor, scale: Optional[torch.T
     _require_cuda(x, "po2::conv2d_packed")
     if x.dim() != 4:
         raise RuntimeError(f"Expected 4D (batched) input to conv2d, but got input of size: {list(x.shape)}")
-    x = x.contiguous()
+    x = _aligned16(x.contiguous())
     B, C, H, W_ = x.shape
     # the packed operand was laid out for ONE (input shape, weight shape): re-validate it against this input
     need = int(_lib.load().po2_conv2d_pack_bytes(B, C, H, W_, K, R, S, stride, pad, groups, compute))
@@ -853,7 +860,7 @@ def conv2d_packed_ep(x: torch.Tensor, packed: torch.Tensor, scale: Optional[torc
     """act(conv2d(x, W) * ep_a[k] + ep_b[k] + residual) from a pre-packed weight operand: one launch (inference)."""
     global LAUNCHES
     _require_cuda(x, "po2::conv2d_packed_ep")
-    x = x.contiguous()
+    x = _aligned16(x.contiguous())
     B, C, H, W_ = x.shape
     need = int(_lib.load().po2_conv2d_pack_bytes(B, C, H, W_, K, R, S, stride, pad, groups, compute))
     if need == 0 or packed.numel() != need:
@@ -891,8 +898,8 @@ def conv2d_ep(x: torch.Tensor, w: torch.Tensor, scale: Optional[torch.Tensor], s
     if x.dtype != torch.float32 or w.dtype != torch.float32:
         raise TypeError("po2::conv2d_ep: fp32 NCHW activations and fp32 weights only")
     check_conv_shapes(x.shape, w.shape, groups, pad)
-    x = x.contiguous()
-    w = w.contiguous()
+    x = _aligned16(x.contiguous())
+    w = _aligned16(w.contiguous())
     lib = _lib.load()
     B, C, H, W_ = x.shape
     K, _, R, S = w.shape
