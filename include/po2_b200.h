@@ -197,7 +197,8 @@ int po2_conv2d_dgrad_packed(const void* g, const void* packed, const float* scal
 /* Data gradient of the same conv (SURVEY.md section 8f "next" #2, first half): gx = dL/dx given g = dL/dout,
  * for the stride-1 dense shapes (3x3 pad 1, 1x1 pad 0), on the tensor-core kernel with the
  * channel-transposed, 180-degree-rotated PO2 weights (exact in bf16; g is rounded to bf16).
- * Returns PO2_E_UNSUPPORTED for other shapes (the caller keeps aten.convolution_backward). */
+ * po2_conv2d_dgrad returns PO2_E_UNSUPPORTED for other shapes (the caller keeps aten.convolution_backward), and
+ * po2_conv2d_dgrad_workspace returns 0 for exactly the shapes po2_conv2d_dgrad refuses. */
 size_t po2_conv2d_dgrad_workspace(int B, int C, int H, int W, int K, int R, int S, int pad, int compute);
 int po2_conv2d_dgrad(const void* g, const void* w, const float* scale, void* gx, int B, int C, int H,
                      int W, int K, int R, int S, int stride, int pad, int groups, int w_format,

@@ -783,23 +783,24 @@ static bool fill_geom(ConvGeom& g, int B, int C, int H, int W, int K, int R, int
   return g.P > 0 && g.Q > 0;
 }
 
-// K3 takes: dense, square 3x3 pad 1 or 1x1 pad 0, stride 1 or 2
-static bool umma_shape_ok(const ConvGeom& g) {
-  if (g.groups != 1 || (g.stride != 1 && g.stride != 2)) return false;
-  if (!((g.R == 3 && g.S == 3 && g.pad == 1) || (g.R == 1 && g.S == 1 && g.pad == 0))) return false;
-  return true;
+// the tensor-core kernels index activations with 32-bit offsets: x (B, Cin, HWin) and out (B, Cout, HWout) must each
+// stay below 2^31 elements
+static bool index_fits(int64_t B, int64_t Cin, int64_t HWin, int64_t Cout, int64_t HWout) {
+  return B * Cin * HWin < (1ll << 31) && B * Cout * HWout < (1ll << 31);
 }
-// the FORWARD runs on K3 / K3T: shapes they take, minus the pointwise layers on tiny feature maps, which go to
-// the fp32 cluster GEMM of csrc/po2_conv_bwd.cu (no packed operand)
-static bool umma_eligible(const ConvGeom& g) {
-  return umma_shape_ok(g) && !pw_small_takes(g.B, g.C, g.H, g.W, g.K, g.R, g.S, g.stride, g.pad, g.groups);
+static bool index_fits(const ConvGeom& g) { return index_fits(g.B, g.C, (int64_t)g.H * g.W, g.K, (int64_t)g.P * g.Q); }
+
+// the filter windows of the tensor-core kernels: square 3x3 pad 1 or 1x1 pad 0
+static bool tc_window(int R, int S, int pad) { return (R == 3 && S == 3 && pad == 1) || (R == 1 && S == 1 && pad == 0); }
+
+// K3 takes: dense, tc_window, stride 1 or 2
+static bool umma_shape_ok(const ConvGeom& g) {
+  return g.groups == 1 && (g.stride == 1 || g.stride == 2) && tc_window(g.R, g.S, g.pad);
 }
 
 static size_t umma_smem_bytes(const ConvGeom& g) {
   return (size_t)g.b_slab_bytes + (size_t)g.nst * g.a_stage_bytes + (3 * K3_MAX_STAGES + 8) * 8 + 64;
 }
-
-static bool tma_takes(const ConvGeom& g);    // po2_conv_tma.cuh: the TMA-fed kernel runs this (planned) geometry
 
 // returns false if the shape does not fit the kernel's shared-memory plan
 static bool plan_umma(ConvGeom& g, bool tf32) {
@@ -880,11 +881,8 @@ static bool plan_umma(ConvGeom& g, bool tf32) {
   g.vec4 = (g.stride == 1 && g.W % 4 == 0) ? 1 : 0;
   g.items_per_row = g.W / 4 + (g.pitch > g.W ? 1 : 0);
   g.div_ipr = make_fastdiv((uint32_t)(g.items_per_row > 0 ? g.items_per_row : 1));
-  g.tapminor = (g.ntaps == 9 && tma_takes(g)) ? 1 : 0;
   return true;
 }
-
-static size_t umma_pack_bytes(const ConvGeom& g) { return (size_t)g.ntiles_n * g.b_slab_bytes; }
 
 // PO2_CONV_TMA=0 keeps every shape on the register-fed kernel (A/B measurements)
 static bool tma_enabled() {
@@ -896,13 +894,77 @@ static bool tma_enabled() {
 #include "po2_conv_tma.cuh"   // K3T: the TMA-fed tf32 form (plan_tma / launch_tma)
 namespace po2 {
 
-// transpose: 0/1 = run pack_weights_kernel first (forward / data-gradient orientation); -1 = pack_buf
-// already holds the operand.  pdl: launch the conv with programmatic stream serialization -- ONLY
-// legal when the kernel directly in front of it in the stream is one of ours that was launched
-// with a full dependency (pack_weights_kernel, fused_kernel): the conv's producers read x without a
-// griddepcontrol.wait, which is safe only if x's producer finished before that kernel started.
-// chain: the operand is already packed and the kernel directly in front in the stream produced x (a norm kernel):
-// the TMA-fed kernel is launched programmatically with the waits of TmaPlan::pdl == 2 (PO2_CONV_PDL_CHAIN=0: off).
+// Which kernel runs a conv, and how.  The forward plans with plan_fwd and the data gradient with plan_dgrad; every
+// query and launch of a shape goes through one of them, so all of them make the same decision.
+struct ConvPlan {
+  int kind;              // po2_conv2d_kernel_kind: 0 direct fp32, 1 depthwise, 2 K3, 3 K3T, 4 small-pointwise GEMM
+  ConvGeom g;            // through fill_geom, and for kinds 2 / 3 through plan_umma
+  TmaPlan tp;            // kind 3
+  size_t pack_bytes;     // the packed weight operand of kinds 2 / 3; 0 for the other kinds
+  size_t workspace;      // what the launching entry point needs
+  bool unpadded;         // kinds 2 / 3: the operand has no channel padding, so the fused quantizers can emit it
+};
+
+static size_t round256(size_t n) { return (n + 255) / 256 * 256; }
+
+// K3, or K3T where the TMA-fed kernel takes the planned geometry (it reads the 3x3 operand tap-minor); false: the
+// shape does not fit K3's shared-memory plan
+static bool plan_tc(ConvPlan& p, bool tf32) {
+  if (!plan_umma(p.g, tf32)) return false;
+  p.kind = (tf32 && tma_enabled() && plan_tma(p.g, p.tp)) ? 3 : 2;
+  p.g.tapminor = (p.kind == 3 && p.g.ntaps == 9) ? 1 : 0;
+  p.pack_bytes = (size_t)p.g.ntiles_n * p.g.b_slab_bytes;
+  p.unpadded = p.g.Cpad == p.g.C && p.g.ntiles_n * p.g.NT == p.g.K;
+  return true;
+}
+
+// false: not a conv shape (PO2_E_SHAPE)
+static bool plan_fwd(ConvPlan& p, int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
+                     int compute) {
+  p = ConvPlan{};
+  if (!fill_geom(p.g, B, C, H, W, K, R, S, stride, pad, groups)) return false;
+  // the pointwise layers on tiny feature maps go to the fp32 cluster GEMM of csrc/po2_conv_bwd.cu, not to K3 / K3T
+  const bool pw_small = pw_small_takes(B, C, H, W, K, R, S, stride, pad, groups);
+  if (compute == 1 || !umma_shape_ok(p.g) || pw_small || !plan_tc(p, compute == 2))
+    p.kind = pw_small ? 4 : (groups == C && groups == K) ? 1 : 0;
+  // the decoded fp32 weights (codes input), then the packed operand
+  const size_t wbytes = (size_t)K * (C / groups) * R * S * sizeof(float);
+  p.workspace = round256(wbytes + (p.pack_bytes ? p.pack_bytes + 256 : 0));
+  return true;
+}
+
+// The data gradient of a stride-1 dense layer (x: B, C, H, W; w: K, C, R, S) is the forward conv of the output
+// gradient (K channels) into C channels with the channel-transposed, 180-degree-rotated weight, on K3 / K3T.
+// Returns 0, or the code po2_conv2d_dgrad refuses the shape with.
+static int plan_dgrad(ConvPlan& p, int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
+                      int compute) {
+  p = ConvPlan{};
+  if (compute == 1 || stride != 1 || groups != 1 || !tc_window(R, S, pad)) return PO2_E_UNSUPPORTED;
+  if (!fill_geom(p.g, B, K, H, W, C, R, S, 1, pad, 1)) return PO2_E_SHAPE;
+  if (!index_fits(p.g)) return PO2_E_SIZE;
+  if (!plan_tc(p, compute == 2)) return PO2_E_UNSUPPORTED;
+  p.workspace = round256(p.pack_bytes + 256);
+  return 0;
+}
+
+// the fused quantizers' description of the planned operand (layout: pack_weights_kernel / pack_store)
+static PackArgs pack_args(const ConvGeom& g, void* Bp) {
+  PackArgs pk = {};
+  pk.Bp = Bp;
+  pk.G = g.G; pk.C = g.C; pk.K = g.K; pk.taps = g.ntaps; pk.NT = g.NT; pk.ncg = g.C / g.G; pk.tapminor = g.tapminor;
+  pk.div_ct = make_fastdiv((uint32_t)(g.C * g.ntaps));
+  pk.div_t = make_fastdiv((uint32_t)g.ntaps);
+  pk.div_nt = make_fastdiv((uint32_t)g.NT);
+  return pk;
+}
+// ... and the data-gradient operand of the same weight; gd: the plan_dgrad geometry
+static void add_dgrad_operand(PackArgs& pk, const ConvGeom& gd, void* Bp2) {
+  pk.Bp2 = Bp2;
+  pk.NT2 = gd.NT; pk.ncg2 = gd.C / gd.G; pk.tapminor2 = gd.tapminor;
+  pk.div_nt2 = make_fastdiv((uint32_t)gd.NT);
+}
+
+// PO2_CONV_PDL_CHAIN=0: the entry points that take a packed operand launch the conv with a full dependency
 static bool pdl_chain_enabled() {
   static const bool on = []() { const char* e = getenv("PO2_CONV_PDL_CHAIN"); return !(e && e[0] == '0'); }();
   return on;
@@ -917,62 +979,61 @@ static int umma_check_x(const void* x, const ConvGeom& g) {
   return (wide_loads && !aligned16(x)) ? PO2_E_ALIGN : 0;
 }
 
-static int launch_umma(const void* x, const void* w, const float* scale, void* out, ConvGeom& g, int w_format,
-                       int bits, int fsr, int transpose, void* pack_buf, cudaStream_t st, bool pdl = true,
-                       const ConvEpilogue& ep = ConvEpilogue{nullptr, nullptr, nullptr, 0}, bool chain = false) {
-  if (int a = umma_check_x(x, g)) return a;
-  {
-    uint8_t* Bp = reinterpret_cast<uint8_t*>(pack_buf);
-    cudaError_t e = cudaSuccess;
-    if (transpose >= 0) {                                  // transpose < 0: the operand is already packed
-      const int64_t total = (int64_t)umma_pack_bytes(g) / (g.tf32 ? 4 : 2);
-      const int pblocks = (int)((total + 255) / 256 < 1184 ? (total + 255) / 256 : 1184);
-      pack_weights_kernel<<<pblocks, 256, 0, st>>>(
-          w_format == PO2_W_CODES ? nullptr : (const float*)w, w_format == PO2_W_CODES ? (const uint8_t*)w : nullptr,
-          w_format == PO2_W_CODES ? nullptr : scale, Bp, g, bits, fsr, transpose);
-      e = cudaGetLastError();
-      if (e != cudaSuccess) return (int)e;
-    }
-    {                                                     // K3T where the shape allows: activations by tensor-map TMA
-      TmaPlan tp;
-      if (g.tf32 && tma_enabled() && plan_tma(g, tp)) {
-        // (the operand may already be packed in K3T's layout: an x that cannot be described by a tensor map is an
-        // error here, not a fallback; a misaligned one was refused above with PO2_E_ALIGN)
-        return launch_tma(x, Bp, scale, out, g, tp, st, (chain && transpose < 0 && pdl_chain_enabled()) ? 2 : (pdl ? 1 : 0), ep);
-      }
-    }
-    static PerDeviceOnce attr_once;                       // the opt-in shared-memory size is a per-device attribute
-    e = attr_once.run([]() -> cudaError_t {
-      const int smax = (int)K3_SMEM_BUDGET + 1024;
-      cudaError_t a = cudaFuncSetAttribute(conv_umma_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
-      if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<9, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
-      if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
-      if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<9, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
-      return a;
-    });
-    if (e != cudaSuccess) return (int)e;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(g.ntiles_n * g.m_step));
-    cfg.blockDim = dim3(K3_THREADS);
-    cfg.dynamicSmemBytes = umma_smem_bytes(g);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;   // overlap our prologue with the pack kernel
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    const float* xf = (const float*)x;
-    const uint8_t* bpc = Bp;
-    float* of = (float*)out;
-    if (g.tf32) {
-      if (g.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<1, true>, xf, bpc, scale, of, g, ep);
-      else e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<9, true>, xf, bpc, scale, of, g, ep);
-    } else {
-      if (g.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<1, false>, xf, bpc, scale, of, g, ep);
-      else e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<9, false>, xf, bpc, scale, of, g, ep);
-    }
-    return (int)e;
+// w (fp32 PO2-grid weights, or codes) -> the planned operand at Bp.  transpose: the data-gradient conv's operand
+// from the forward weight
+static int launch_pack(const ConvPlan& p, const void* w, int w_format, const float* scale, int bits, int fsr,
+                       int transpose, void* Bp, cudaStream_t st) {
+  const int64_t total = (int64_t)p.pack_bytes / (p.g.tf32 ? 4 : 2);
+  const int pblocks = (int)((total + 255) / 256 < 1184 ? (total + 255) / 256 : 1184);
+  const bool codes = w_format == PO2_W_CODES;
+  pack_weights_kernel<<<pblocks, 256, 0, st>>>(codes ? nullptr : (const float*)w, codes ? (const uint8_t*)w : nullptr,
+                                               codes ? nullptr : scale, Bp, p.g, bits, fsr, transpose);
+  return (int)cudaGetLastError();
+}
+
+// The K3 / K3T conv on the packed operand Bp.  pdl 1: launched with programmatic stream serialization -- ONLY legal
+// when the kernel directly in front of it in the stream is one of ours that was launched with a full dependency
+// (pack_weights_kernel, fused_kernel): the conv's producers read x without a griddepcontrol.wait, which is safe only if
+// x's producer finished before that kernel started.  pdl 2 (chain): the operand was packed earlier and the kernel
+// directly in front produced x (a norm kernel): K3T is launched programmatically with the waits of TmaPlan::pdl == 2,
+// K3 with a full dependency.  pdl 0: a full dependency.
+static int launch_conv(const ConvPlan& p, const void* x, const void* Bp, const float* scale, void* out, int pdl,
+                       const ConvEpilogue& ep, cudaStream_t st) {
+  const ConvGeom& g = p.g;
+  // (the operand may already be packed in K3T's layout: an x that cannot be described by a tensor map is an error
+  // here, not a fallback; a misaligned one is refused with PO2_E_ALIGN before any launch)
+  if (p.kind == 3) return launch_tma(x, (const uint8_t*)Bp, scale, out, g, p.tp, st, pdl, ep);
+  static PerDeviceOnce attr_once;                       // the opt-in shared-memory size is a per-device attribute
+  cudaError_t e = attr_once.run([]() -> cudaError_t {
+    const int smax = (int)K3_SMEM_BUDGET + 1024;
+    cudaError_t a = cudaFuncSetAttribute(conv_umma_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+    if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<9, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+    if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+    if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<9, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+    return a;
+  });
+  if (e != cudaSuccess) return (int)e;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)(g.ntiles_n * g.m_step));
+  cfg.blockDim = dim3(K3_THREADS);
+  cfg.dynamicSmemBytes = umma_smem_bytes(g);
+  cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;   // overlap our prologue with the pack kernel
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = pdl == 1 ? 1 : 0;
+  const float* xf = (const float*)x;
+  const uint8_t* bpc = (const uint8_t*)Bp;
+  float* of = (float*)out;
+  if (g.tf32) {
+    if (g.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<1, true>, xf, bpc, scale, of, g, ep);
+    else e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<9, true>, xf, bpc, scale, of, g, ep);
+  } else {
+    if (g.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<1, false>, xf, bpc, scale, of, g, ep);
+    else e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<9, false>, xf, bpc, scale, of, g, ep);
   }
+  return (int)e;
 }
 
 
@@ -1378,11 +1439,8 @@ int po2_debug_set_trace(void* buf) {
 
 size_t po2_conv2d_workspace(int B, int C, int H, int W, int K, int R, int S, int stride, int pad,
                             int groups, int compute) {
-  ConvGeom g;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return 0;
-  size_t bytes = (size_t)K * (C / groups) * R * S * sizeof(float);       // decoded fp32 weights (codes input)
-  if (compute != 1 && umma_eligible(g) && plan_umma(g, compute == 2)) bytes += umma_pack_bytes(g) + 256;
-  return (bytes + 255) / 256 * 256;
+  ConvPlan p;
+  return plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute) ? p.workspace : 0;
 }
 
 // which kernel po2_conv2d_fwd runs for this geometry: 0 direct fp32, 1 depthwise, 2 tcgen05 with the
@@ -1390,14 +1448,8 @@ size_t po2_conv2d_workspace(int B, int C, int H, int W, int K, int R, int S, int
 // pointwise layers on <= 16-pixel feature maps; < 0: PO2_E_*
 int po2_conv2d_kernel_kind(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
                            int compute) {
-  ConvGeom g;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
-  if (compute != 1 && umma_eligible(g) && plan_umma(g, compute == 2)) {
-    TmaPlan tp;
-    return (g.tf32 && tma_enabled() && plan_tma(g, tp)) ? 3 : 2;
-  }
-  if (pw_small_takes(B, C, H, W, K, R, S, stride, pad, groups)) return 4;
-  return (groups == C && groups == K) ? 1 : 0;
+  ConvPlan p;
+  return plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute) ? p.kind : PO2_E_SHAPE;
 }
 
 static int check_epilogue(const float* ep_a, const float* ep_b, int act) {
@@ -1424,24 +1476,25 @@ int po2_conv2d_fwd_ep(const void* x, const void* w, const float* scale, void* ou
   if (int e = check_epilogue(ep_a, ep_b, act)) return e;
   if (!ep_a && (residual || act)) return PO2_E_NULL;
   const ConvEpilogue ep{ep_a, ep_b, (const float*)residual, act};
-  ConvGeom g;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
+  ConvPlan p;
+  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  const ConvGeom& g = p.g;
   if (w_format != PO2_W_F32_PO2 && w_format != PO2_W_CODES) return PO2_E_UNSUPPORTED;
   if (w_format == PO2_W_CODES && (!scale || bits < 2 || bits > 8)) return PO2_E_BITS;
-  if ((int64_t)B * C * H * W >= (1ll << 31) || (int64_t)B * K * g.P * g.Q >= (1ll << 31)) return PO2_E_SIZE;
+  if (!index_fits(g)) return PO2_E_SIZE;
   cudaStream_t st = (cudaStream_t)stream;
-  const size_t need = po2_conv2d_workspace(B, C, H, W, K, R, S, stride, pad, groups, compute);
   const int64_t wn = (int64_t)K * (C / groups) * R * S;
-  const size_t wbytes = ((size_t)wn * sizeof(float) + 255) / 256 * 256;
+  const size_t wbytes = round256((size_t)wn * sizeof(float));
 
-  if (compute != 1 && umma_eligible(g) && plan_umma(g, compute == 2)) {
-    if (!workspace || workspace_bytes < need) return PO2_E_WORKSPACE;
-    return launch_umma(x, w, scale, out, g, w_format, bits, fsr, 0, reinterpret_cast<char*>(workspace) + wbytes, st, true, ep);
+  if (p.pack_bytes) {
+    if (!workspace || workspace_bytes < p.workspace) return PO2_E_WORKSPACE;
+    if (int a = umma_check_x(x, g)) return a;
+    void* Bp = reinterpret_cast<char*>(workspace) + wbytes;
+    if (int e = launch_pack(p, w, w_format, scale, bits, fsr, 0, Bp, st)) return e;
+    return launch_conv(p, x, Bp, scale, out, 1, ep, st);
   }
   // the small-pointwise GEMM reads rows of the fp32 weight with 128-bit loads when C % 4 == 0
-  if (pw_small_takes(B, C, H, W, K, R, S, stride, pad, groups) && C % 4 == 0 &&
-      !aligned16(w_format == PO2_W_CODES ? workspace : w))
-    return PO2_E_ALIGN;
+  if (p.kind == 4 && C % 4 == 0 && !aligned16(w_format == PO2_W_CODES ? workspace : w)) return PO2_E_ALIGN;
   // CUDA-core paths work on fp32 weights
   const float* wf = (const float*)w;
   if (w_format == PO2_W_CODES) {
@@ -1452,9 +1505,8 @@ int po2_conv2d_fwd_ep(const void* x, const void* w, const float* scale, void* ou
     if (e != cudaSuccess) return (int)e;
     wf = (const float*)workspace;
   }
-  if (pw_small_takes(B, C, H, W, K, R, S, stride, pad, groups))
-    return launch_pw_small((const float*)x, wf, (float*)out, B, C, H * W, K, ep, st);
-  if (groups == C && groups == K) {
+  if (p.kind == 4) return launch_pw_small((const float*)x, wf, (float*)out, B, C, H * W, K, ep, st);
+  if (p.kind == 1) {
     const int64_t total = (int64_t)B * C * g.P * g.Q;
     // vector kernel: 3x3 pad 1, stride 1 or 2, rows and outputs in whole 16-byte groups
     if (R == 3 && S == 3 && pad == 1 && (stride == 1 || stride == 2) && W % 4 == 0 && g.Q % 4 == 0 &&
@@ -1496,27 +1548,22 @@ int po2_conv2d_dgrad(const void* g_out, const void* w, const float* scale, void*
                      int W, int K, int R, int S, int stride, int pad, int groups, int w_format, int bits,
                      int fsr, int compute, void* workspace, size_t workspace_bytes, void* stream) {
   if (!g_out || !w || !gx) return PO2_E_NULL;
-  if (compute == 1) return PO2_E_UNSUPPORTED;
-  if (stride != 1 || groups != 1) return PO2_E_UNSUPPORTED;
-  if (!((R == 3 && S == 3 && pad == 1) || (R == 1 && S == 1 && pad == 0))) return PO2_E_UNSUPPORTED;
   if (w_format != PO2_W_F32_PO2 && w_format != PO2_W_CODES) return PO2_E_UNSUPPORTED;
-  ConvGeom g;
-  if (!fill_geom(g, B, K, H, W, C, R, S, 1, pad, 1)) return PO2_E_SHAPE;      // in = K channels, out = C channels
-  if ((int64_t)B * C * H * W >= (1ll << 31) || (int64_t)B * K * H * W >= (1ll << 31)) return PO2_E_SIZE;
-  if (!plan_umma(g, compute == 2)) return PO2_E_UNSUPPORTED;
-  const size_t need = umma_pack_bytes(g) + 256;
-  if (!workspace || workspace_bytes < need) return PO2_E_WORKSPACE;
-  return launch_umma(g_out, w, scale, gx, g, w_format, bits, fsr, 1, workspace, (cudaStream_t)stream);
+  ConvPlan p;
+  if (int e = plan_dgrad(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return e;
+  if (!workspace || workspace_bytes < p.workspace) return PO2_E_WORKSPACE;
+  if (int a = umma_check_x(g_out, p.g)) return a;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int e = launch_pack(p, w, w_format, scale, bits, fsr, 1, workspace, st)) return e;
+  return launch_conv(p, g_out, workspace, scale, gx, 1, ConvEpilogue{}, st);
 }
 
 // Static weights (PTQ / eval): build the packed tensor-core operand once, reuse it every forward.
 // po2_conv2d_pack_bytes == 0 means the shape does not run on the tensor-core kernel.
 size_t po2_conv2d_pack_bytes(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
                              int compute) {
-  ConvGeom g;
-  if (compute == 1 || !fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups) || !umma_eligible(g) ||
-      !plan_umma(g, compute == 2)) return 0;
-  return (umma_pack_bytes(g) + 255) / 256 * 256;
+  ConvPlan p;
+  return plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute) ? round256(p.pack_bytes) : 0;
 }
 
 int po2_conv2d_pack(const void* w, const float* scale, void* packed, size_t packed_bytes, int B, int C, int H,
@@ -1525,16 +1572,11 @@ int po2_conv2d_pack(const void* w, const float* scale, void* packed, size_t pack
   if (!w || !packed) return PO2_E_NULL;
   if (w_format != PO2_W_F32_PO2 && w_format != PO2_W_CODES) return PO2_E_UNSUPPORTED;
   if (w_format == PO2_W_CODES && (!scale || bits < 2 || bits > 8)) return PO2_E_BITS;
-  ConvGeom g;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
-  if (compute == 1 || !umma_eligible(g) || !plan_umma(g, compute == 2)) return PO2_E_UNSUPPORTED;
-  if (packed_bytes < umma_pack_bytes(g)) return PO2_E_WORKSPACE;
-  const int64_t total = (int64_t)umma_pack_bytes(g) / (g.tf32 ? 4 : 2);
-  const int pblocks = (int)((total + 255) / 256 < 1184 ? (total + 255) / 256 : 1184);
-  pack_weights_kernel<<<pblocks, 256, 0, (cudaStream_t)stream>>>(
-      w_format == PO2_W_CODES ? nullptr : (const float*)w, w_format == PO2_W_CODES ? (const uint8_t*)w : nullptr,
-      w_format == PO2_W_CODES ? nullptr : scale, packed, g, bits, fsr, 0);
-  return (int)cudaGetLastError();
+  ConvPlan p;
+  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (!p.pack_bytes) return PO2_E_UNSUPPORTED;
+  if (packed_bytes < p.pack_bytes) return PO2_E_WORKSPACE;
+  return launch_pack(p, w, w_format, scale, bits, fsr, 0, packed, (cudaStream_t)stream);
 }
 
 int po2_conv2d_fwd_packed(const void* x, const void* packed, const float* scale, void* out, int B, int C, int H,
@@ -1550,12 +1592,12 @@ int po2_conv2d_fwd_packed_ep(const void* x, const void* packed, const float* sca
   if (int e = check_epilogue(ep_a, ep_b, act)) return e;
   if (!ep_a && (residual || act)) return PO2_E_NULL;
   const ConvEpilogue ep{ep_a, ep_b, (const float*)residual, act};
-  ConvGeom g;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
-  if (compute == 1 || !umma_eligible(g) || !plan_umma(g, compute == 2)) return PO2_E_UNSUPPORTED;
-  if ((int64_t)B * C * H * W >= (1ll << 31) || (int64_t)B * K * g.P * g.Q >= (1ll << 31)) return PO2_E_SIZE;
-  return launch_umma(x, nullptr, scale, out, g, PO2_W_F32_PO2, 4, 1, -1, const_cast<void*>(packed), (cudaStream_t)stream,
-                     /*pdl=*/false, ep, /*chain=*/true);
+  ConvPlan p;
+  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (!p.pack_bytes) return PO2_E_UNSUPPORTED;
+  if (!index_fits(p.g)) return PO2_E_SIZE;
+  if (int a = umma_check_x(x, p.g)) return a;
+  return launch_conv(p, x, packed, scale, out, pdl_chain_enabled() ? 2 : 0, ep, (cudaStream_t)stream);
 }
 
 // QuantizedConv2d.forward in QAT mode as ONE call (models/quantized_conv.py:34-36): quantize the fp32
@@ -1569,26 +1611,18 @@ int po2_qconv2d_fwd(const void* x, const void* w_master, void* qw_out, float* sc
                     void* quant_workspace, void* stream) {
   if (!x || !w_master || !qw_out || !scale_out || !out) return PO2_E_NULL;
   if (!quant_workspace) return PO2_E_WORKSPACE;
-  ConvGeom g;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
+  ConvPlan p;
+  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t wn = (int64_t)K * (C / groups) * R * S;
-  const bool umma = compute != 1 && umma_eligible(g) && plan_umma(g, compute == 2);
-  if (umma)
-    if (int a = umma_check_x(x, g)) return a;                 // before the quantizer runs
-  if (umma && g.Cpad == C && g.ntiles_n * g.NT == K) {
-    const size_t need = po2_conv2d_workspace(B, C, H, W, K, R, S, stride, pad, groups, compute);
-    const size_t wbytes = ((size_t)wn * sizeof(float) + 255) / 256 * 256;
-    if (!workspace || workspace_bytes < need) return PO2_E_WORKSPACE;
-    if ((int64_t)B * C * H * W >= (1ll << 31) || (int64_t)B * K * g.P * g.Q >= (1ll << 31)) return PO2_E_SIZE;
-    PackArgs pk = {};
-    pk.Bp = reinterpret_cast<char*>(workspace) + wbytes;
-    pk.G = g.G; pk.C = C; pk.K = K; pk.taps = g.ntaps; pk.NT = g.NT; pk.ncg = C / g.G; pk.tapminor = g.tapminor;
-    pk.div_ct = make_fastdiv((uint32_t)(C * g.ntaps));
-    pk.div_t = make_fastdiv((uint32_t)g.ntaps);
-    pk.div_nt = make_fastdiv((uint32_t)g.NT);
+  if (p.pack_bytes)
+    if (int a = umma_check_x(x, p.g)) return a;               // before the quantizer runs
+  if (p.unpadded) {
+    if (!workspace || workspace_bytes < p.workspace) return PO2_E_WORKSPACE;
+    if (!index_fits(p.g)) return PO2_E_SIZE;
+    const PackArgs pk = pack_args(p.g, reinterpret_cast<char*>(workspace) + round256((size_t)wn * sizeof(float)));
     const int rc = fused_quantize_pack(w_master, qw_out, scale_out, wn, bits, fsr, mode, flavor, quant_workspace, pk, st);
-    if (rc == 0) return launch_umma(x, qw_out, scale_out, out, g, PO2_W_F32_PO2, bits, fsr, -1, pk.Bp, st);
+    if (rc == 0) return launch_conv(p, x, pk.Bp, scale_out, out, 1, ConvEpilogue{}, st);
     if (rc != PO2_E_UNSUPPORTED) return rc;
   }
   if (int e = po2_quantize_fused(w_master, qw_out, nullptr, nullptr, nullptr, scale_out, wn, PO2_F32, bits, fsr,
@@ -1605,20 +1639,15 @@ int po2_quantize_pack(const void* w_master, void* qw_out, float* scale_out, void
                       int mode, int flavor, int compute, void* quant_workspace, void* stream) {
   if (!w_master || !qw_out || !scale_out || !packed) return PO2_E_NULL;
   if (!quant_workspace) return PO2_E_WORKSPACE;
-  ConvGeom g;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
-  if (compute == 1 || !umma_eligible(g) || !plan_umma(g, compute == 2)) return PO2_E_UNSUPPORTED;
-  if (packed_bytes < umma_pack_bytes(g)) return PO2_E_WORKSPACE;
+  ConvPlan p;
+  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (!p.pack_bytes) return PO2_E_UNSUPPORTED;
+  if (packed_bytes < p.pack_bytes) return PO2_E_WORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t wn = (int64_t)K * (C / groups) * R * S;
-  if (g.Cpad == C && g.ntiles_n * g.NT == K) {
-    PackArgs pk = {};
-    pk.Bp = packed;
-    pk.G = g.G; pk.C = C; pk.K = K; pk.taps = g.ntaps; pk.NT = g.NT; pk.ncg = C / g.G; pk.tapminor = g.tapminor;
-    pk.div_ct = make_fastdiv((uint32_t)(C * g.ntaps));
-    pk.div_t = make_fastdiv((uint32_t)g.ntaps);
-    pk.div_nt = make_fastdiv((uint32_t)g.NT);
-    const int rc = fused_quantize_pack(w_master, qw_out, scale_out, wn, bits, fsr, mode, flavor, quant_workspace, pk, st);
+  if (p.unpadded) {
+    const int rc = fused_quantize_pack(w_master, qw_out, scale_out, wn, bits, fsr, mode, flavor, quant_workspace,
+                                       pack_args(p.g, packed), st);
     if (rc != PO2_E_UNSUPPORTED) return rc;
   }
   if (int e = po2_quantize_fused(w_master, qw_out, nullptr, nullptr, nullptr, scale_out, wn, PO2_F32, bits, fsr, mode,
@@ -1635,11 +1664,10 @@ int po2_multi_desc_fill(void* host_table, int index, const void* w_master, void*
                         int groups, int bits, int fsr, int mode, int flavor, int compute, double* sse_out) {
   if (!host_table || index < 0 || !w_master || !qw_out || !scale_out || !packed) return PO2_E_NULL;
   if (int e = check_quant_args(bits, fsr, mode, flavor)) return e;
-  ConvGeom g;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
-  if (compute == 1 || !umma_eligible(g) || !plan_umma(g, compute == 2)) return PO2_E_UNSUPPORTED;
-  if (!(g.Cpad == C && g.ntiles_n * g.NT == K)) return PO2_E_UNSUPPORTED;        // the packed operand has no padding
-  if (packed_bytes < umma_pack_bytes(g)) return PO2_E_WORKSPACE;
+  ConvPlan p;
+  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (!p.unpadded) return PO2_E_UNSUPPORTED;             // no tensor-core operand, or one with channel padding
+  if (packed_bytes < p.pack_bytes) return PO2_E_WORKSPACE;
   const int64_t wn = (int64_t)K * (C / groups) * R * S;
   if (wn % 4 || (reinterpret_cast<uintptr_t>(w_master) & 15) || (reinterpret_cast<uintptr_t>(qw_out) & 15))
     return PO2_E_UNSUPPORTED;
@@ -1650,11 +1678,7 @@ int po2_multi_desc_fill(void* host_table, int index, const void* w_master, void*
   MultiDesc d = {};
   d.x = (const uint4*)w_master; d.y = (uint4*)qw_out; d.scale_out = scale_out; d.sse_out = sse_out; d.n = wn;
   d.bits = bits; d.fsr = fsr; d.mode = mode; d.flavor = flavor;
-  d.pk.Bp = packed;
-  d.pk.G = g.G; d.pk.C = C; d.pk.K = K; d.pk.taps = g.ntaps; d.pk.NT = g.NT; d.pk.ncg = C / g.G; d.pk.tapminor = g.tapminor;
-  d.pk.div_ct = make_fastdiv((uint32_t)(C * g.ntaps));
-  d.pk.div_t = make_fastdiv((uint32_t)g.ntaps);
-  d.pk.div_nt = make_fastdiv((uint32_t)g.NT);
+  d.pk = pack_args(p.g, packed);
   reinterpret_cast<MultiDesc*>(host_table)[index] = d;
   return csize;
 }
@@ -1664,36 +1688,22 @@ int po2_quantize_pack_multi(const void* device_table, int ntensors, int cluster_
 }
 
 // ---- the data-gradient operand packed ahead of time (by the multi-tensor quantizer of the forward pass) ----
-// geometry of the data-gradient conv of a stride-1 dense layer: in = K channels, out = C channels
-static bool dgrad_geom(ConvGeom& g, int B, int C, int H, int W, int K, int R, int S, int pad, int compute) {
-  if (compute == 1) return false;
-  if (!((R == 3 && S == 3 && pad == 1) || (R == 1 && S == 1 && pad == 0))) return false;
-  if (!fill_geom(g, B, K, H, W, C, R, S, 1, pad, 1)) return false;
-  if ((int64_t)B * C * H * W >= (1ll << 31) || (int64_t)B * K * H * W >= (1ll << 31)) return false;
-  return plan_umma(g, compute == 2);
-}
-
 size_t po2_conv2d_dgrad_pack_bytes(int B, int C, int H, int W, int K, int R, int S, int pad, int compute) {
-  ConvGeom g;
-  if (!dgrad_geom(g, B, C, H, W, K, R, S, pad, compute)) return 0;
-  if (!(g.Cpad == K && g.ntiles_n * g.NT == C)) return 0;                 // the fused emitter writes no padding
-  return (umma_pack_bytes(g) + 255) / 256 * 256;
+  ConvPlan p;
+  if (plan_dgrad(p, B, C, H, W, K, R, S, 1, pad, 1, compute) || !p.unpadded) return 0;   // the fused emitter writes no padding
+  return round256(p.pack_bytes);
 }
 
 // amend entry `index` of a MultiDesc table (after po2_multi_desc_fill): also emit the data-gradient operand
 int po2_multi_desc_fill_dgrad(void* host_table, int index, void* packed_dgrad, size_t packed_bytes, int B, int C, int H,
                               int W, int K, int R, int S, int stride, int pad, int groups, int compute) {
   if (!host_table || index < 0 || !packed_dgrad) return PO2_E_NULL;
-  if (stride != 1 || groups != 1) return PO2_E_UNSUPPORTED;
-  ConvGeom g;
-  if (!dgrad_geom(g, B, C, H, W, K, R, S, pad, compute)) return PO2_E_UNSUPPORTED;
-  if (!(g.Cpad == K && g.ntiles_n * g.NT == C)) return PO2_E_UNSUPPORTED;
-  if (packed_bytes < umma_pack_bytes(g)) return PO2_E_WORKSPACE;
+  ConvPlan p;
+  if (plan_dgrad(p, B, C, H, W, K, R, S, stride, pad, groups, compute) || !p.unpadded) return PO2_E_UNSUPPORTED;
+  if (packed_bytes < p.pack_bytes) return PO2_E_WORKSPACE;
   MultiDesc& d = reinterpret_cast<MultiDesc*>(host_table)[index];
-  if (d.pk.G != g.G || d.pk.taps != g.ntaps) return PO2_E_SHAPE;
-  d.pk.Bp2 = packed_dgrad;
-  d.pk.NT2 = g.NT; d.pk.ncg2 = K / g.G; d.pk.tapminor2 = g.tapminor;
-  d.pk.div_nt2 = make_fastdiv((uint32_t)g.NT);
+  if (d.pk.G != p.g.G || d.pk.taps != p.g.ntaps) return PO2_E_SHAPE;
+  add_dgrad_operand(d.pk, p.g, packed_dgrad);
   return 0;
 }
 
@@ -1703,27 +1713,20 @@ int po2_multi_desc_fill_dgrad(void* host_table, int index, void* packed_dgrad, s
 // quantizer kernel writes it (and the stride-1 data-gradient operand) from the CTA that owns the input channel.
 // Fills pk for conv2d(x of shape (B, C, H, W), w (K, C/groups, R, S)); PO2_E_UNSUPPORTED when the geometry has no
 // tensor-core operand, needs channel padding (the per-channel emitter writes no padding) or bits is not exact.
-static int lin_pack_args(PackArgs& pk, ConvGeom& g, void* packed, size_t packed_bytes, void* packed_dgrad,
+static int lin_pack_args(PackArgs& pk, ConvPlan& p, void* packed, size_t packed_bytes, void* packed_dgrad,
                          size_t dgrad_bytes, int B, int C, int H, int W, int K, int R, int S, int stride, int pad,
                          int groups, int bits, int num_iters, int compute) {
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
-  if (compute == 1 || !umma_eligible(g) || !plan_umma(g, compute == 2)) return PO2_E_UNSUPPORTED;
-  if (num_iters < 1 || bits > (g.tf32 ? 12 : 9)) return PO2_E_UNSUPPORTED;      // step not a power of two / not exact
-  if (packed_bytes < umma_pack_bytes(g)) return PO2_E_WORKSPACE;
-  pk = PackArgs{};
-  pk.Bp = packed;
-  pk.G = g.G; pk.C = C; pk.K = K; pk.taps = g.ntaps; pk.NT = g.NT; pk.ncg = C / g.G; pk.tapminor = g.tapminor;
-  pk.div_ct = make_fastdiv((uint32_t)(C * g.ntaps));
-  pk.div_t = make_fastdiv((uint32_t)g.ntaps);
-  pk.div_nt = make_fastdiv((uint32_t)g.NT);
+  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (!p.pack_bytes) return PO2_E_UNSUPPORTED;
+  if (num_iters < 1 || bits > (p.g.tf32 ? 12 : 9)) return PO2_E_UNSUPPORTED;    // step not a power of two / not exact
+  if (packed_bytes < p.pack_bytes) return PO2_E_WORKSPACE;
+  pk = pack_args(p.g, packed);
   if (packed_dgrad) {
-    ConvGeom gd;
-    if (stride != 1 || groups != 1 || !dgrad_geom(gd, B, C, H, W, K, R, S, pad, compute)) return PO2_E_UNSUPPORTED;
-    if (!(gd.Cpad == K && gd.ntiles_n * gd.NT == C) || gd.G != g.G || gd.ntaps != g.ntaps) return PO2_E_UNSUPPORTED;
-    if (dgrad_bytes < umma_pack_bytes(gd)) return PO2_E_WORKSPACE;
-    pk.Bp2 = packed_dgrad;
-    pk.NT2 = gd.NT; pk.ncg2 = K / gd.G; pk.tapminor2 = gd.tapminor;
-    pk.div_nt2 = make_fastdiv((uint32_t)gd.NT);
+    ConvPlan d;
+    if (plan_dgrad(d, B, C, H, W, K, R, S, stride, pad, groups, compute) || !d.unpadded || d.g.G != p.g.G ||
+        d.g.ntaps != p.g.ntaps) return PO2_E_UNSUPPORTED;
+    if (dgrad_bytes < d.pack_bytes) return PO2_E_WORKSPACE;
+    add_dgrad_operand(pk, d.g, packed_dgrad);
   }
   return 0;
 }
@@ -1737,12 +1740,11 @@ int po2_lin_quantize_pack(const void* w, void* y_out, void* packed, size_t packe
   const int Cg = groups > 0 ? C / groups : 0;
   if (int e = lin_check_args(K, Cg, R * S, bits, num_iters, flavor)) return e;
   PackArgs pk;
-  ConvGeom g;
-  if (int e = lin_pack_args(pk, g, packed, packed_bytes, packed_dgrad, packed_dgrad_bytes, B, C, H, W, K, R, S, stride,
+  ConvPlan p;
+  if (int e = lin_pack_args(pk, p, packed, packed_bytes, packed_dgrad, packed_dgrad_bytes, B, C, H, W, K, R, S, stride,
                             pad, groups, bits, num_iters, compute)) return e;
   cudaStream_t st = (cudaStream_t)stream;
-  if (g.Cpad == C && g.ntiles_n * g.NT == K)
-    return lin_launch((const float*)w, (float*)y_out, K, C, R * S, bits, num_iters, plus, flavor, pk, st);
+  if (p.unpadded) return lin_launch((const float*)w, (float*)y_out, K, C, R * S, bits, num_iters, plus, flavor, pk, st);
   if (packed_dgrad) return PO2_E_UNSUPPORTED;
   if (int e = lin_launch((const float*)w, (float*)y_out, K, Cg, R * S, bits, num_iters, plus, flavor, PackArgs{}, st))
     return e;
@@ -1760,10 +1762,10 @@ int po2_lin_multi_desc_fill(void* host_table, int index, const void* w, void* y_
   const int Cg = groups > 0 ? C / groups : 0;
   if (int e = lin_check_args(K, Cg, R * S, bits, num_iters, flavor)) return e;
   PackArgs pk;
-  ConvGeom g;
-  if (int e = lin_pack_args(pk, g, packed, packed_bytes, packed_dgrad, packed_dgrad_bytes, B, C, H, W, K, R, S, stride,
+  ConvPlan p;
+  if (int e = lin_pack_args(pk, p, packed, packed_bytes, packed_dgrad, packed_dgrad_bytes, B, C, H, W, K, R, S, stride,
                             pad, groups, bits, num_iters, compute)) return e;
-  if (!(g.Cpad == C && g.ntiles_n * g.NT == K)) return PO2_E_UNSUPPORTED;
+  if (!p.unpadded) return PO2_E_UNSUPPORTED;
   LinDesc* t = reinterpret_cast<LinDesc*>(host_table);
   LinDesc d = {};
   d.w = (const float*)w; d.y = (float*)y_out;
@@ -1778,66 +1780,65 @@ int po2_lin_multi_desc_fill(void* host_table, int index, const void* w, void* y_
 int po2_conv2d_dgrad_packed(const void* g_out, const void* packed, const float* scale, void* gx, int B, int C, int H,
                             int W, int K, int R, int S, int pad, int compute, void* stream) {
   if (!g_out || !packed || !gx) return PO2_E_NULL;
-  ConvGeom g;
-  if (!dgrad_geom(g, B, C, H, W, K, R, S, pad, compute)) return PO2_E_UNSUPPORTED;
-  return launch_umma(g_out, nullptr, scale, gx, g, PO2_W_F32_PO2, 4, 1, -1, const_cast<void*>(packed), (cudaStream_t)stream,
-                     /*pdl=*/false, ConvEpilogue{nullptr, nullptr, nullptr, 0}, /*chain=*/true);
+  ConvPlan p;
+  if (plan_dgrad(p, B, C, H, W, K, R, S, 1, pad, 1, compute)) return PO2_E_UNSUPPORTED;
+  if (int a = umma_check_x(g_out, p.g)) return a;
+  return launch_conv(p, g_out, packed, scale, gx, pdl_chain_enabled() ? 2 : 0, ConvEpilogue{}, (cudaStream_t)stream);
 }
 
 size_t po2_conv2d_dgrad_workspace(int B, int C, int H, int W, int K, int R, int S, int pad, int compute) {
-  ConvGeom g;
-  if (compute == 1 || !fill_geom(g, B, K, H, W, C, R, S, 1, pad, 1) || !plan_umma(g, compute == 2)) return 0;
-  return (umma_pack_bytes(g) + 256 + 255) / 256 * 256;
+  ConvPlan p;
+  return plan_dgrad(p, B, C, H, W, K, R, S, 1, pad, 1, compute) ? 0 : p.workspace;
 }
 
 
 // Weight gradient of the same conv (SURVEY.md section 8f "next" #2, second half): gw = dL/dW given
 // g = dL/dout and the forward input x -- through the straight-through estimator this is the gradient
-// of the fp32 master weight.  Dense stride-1 shapes (3x3 pad 1, 1x1 pad 0) with K <= 128, bf16
-// operands; returns PO2_E_UNSUPPORTED otherwise (the caller keeps aten.convolution_backward).
-static bool wgrad_plan(ConvGeom& g, WgGeom& wg, int B, int C, int H, int W, int K, int R, int S, int stride, int pad,
-                       int groups, int compute) {
-  if (compute != 0 || stride != 1 || groups != 1) return false;
-  if (!((R == 3 && S == 3 && pad == 1) || (R == 1 && S == 1 && pad == 0))) return false;
-  if (!fill_geom(g, B, C, H, W, K, R, S, stride, pad, groups)) return false;
-  if ((int64_t)B * C * H * W >= (1ll << 31) || (int64_t)B * K * g.P * g.Q >= (1ll << 31)) return false;
-  if (!umma_shape_ok(g) || !plan_umma(g, false)) return false;
-  return plan_wgrad(g, wg);
-}
+// of the fp32 master weight.  Which kernel runs a shape, and its plan:
+struct WgradPlan {
+  int kind;              // po2_conv2d_wgrad_kernel_kind: 0 not taken, 1 K5, 2 K5T, 3 pointwise GEMM
+  WgTmaPlan wp;          // kind 2
+  ConvGeom g;            // kind 1: the forward geometry through plan_umma(g, false)
+  WgGeom wg;             // kind 1
+  size_t partial_bytes;  // the workspace: per-CTA partial sums
+};
 
-// compute == 2 (tf32 operands): the TMA-fed kernel K5T where the shape allows, else the bf16-operand kernel
-// (the weight gradient is a leaf of the backward pass: its rounding does not propagate into other gradients)
-static bool wgrad_tma_plan(WgTmaPlan& wp, int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
-                           int compute) {
-  if (compute != 2 || stride != 1 || groups != 1 || !tma_enabled()) return false;
-  static const bool off = [] { const char* e = getenv("PO2_WGRAD_TMA"); return e && e[0] == '0'; }();
-  return !off && plan_wgrad_tma(wp, B, C, H, W, K, R, S, pad);
+// K5 / K5T take the dense stride-1 shapes (3x3 pad 1, 1x1 pad 0) with K <= 128.  compute == 2 (tf32 operands): K5T
+// where the shape allows, else the bf16-operand K5 (the weight gradient is a leaf of the backward pass: its rounding
+// does not propagate into other gradients).  The small 1x1 layers neither takes go to the pointwise GEMM.
+static void plan_wgrad_conv(WgradPlan& p, int B, int C, int H, int W, int K, int R, int S, int stride, int pad,
+                            int groups, int compute) {
+  static const bool k5t_off = [] { const char* e = getenv("PO2_WGRAD_TMA"); return e && e[0] == '0'; }();
+  p = WgradPlan{};
+  const bool dense1 = stride == 1 && groups == 1;
+  if (compute == 2 && dense1 && tma_enabled() && !k5t_off && plan_wgrad_tma(p.wp, B, C, H, W, K, R, S, pad)) {
+    p.kind = 2;
+    p.partial_bytes = wgrad_tma_partial_bytes(p.wp);
+  } else if ((compute == 0 || compute == 2) && dense1 && tc_window(R, S, pad) &&
+             fill_geom(p.g, B, C, H, W, K, R, S, 1, pad, 1) && index_fits(p.g) && plan_umma(p.g, false) &&
+             plan_wgrad(p.g, p.wg)) {
+    p.kind = 1;
+    p.partial_bytes = wgrad_partial_bytes(p.g, p.wg);
+  } else if (pw_wgrad_takes(B, C, H, W, K, R, S, stride, pad, groups, compute)) {
+    p.kind = 3;
+    p.partial_bytes = pw_wgrad_partial_bytes(B, C, H, W, K);
+  }
 }
 
 size_t po2_conv2d_wgrad_workspace(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
                                   int compute) {
-  WgTmaPlan wp;
-  if (wgrad_tma_plan(wp, B, C, H, W, K, R, S, stride, pad, groups, compute))
-    return (wgrad_tma_partial_bytes(wp) + 255) / 256 * 256;
-  ConvGeom g;
-  WgGeom wg;
-  if (wgrad_plan(g, wg, B, C, H, W, K, R, S, stride, pad, groups, compute == 2 ? 0 : compute))
-    return (wgrad_partial_bytes(g, wg) + 255) / 256 * 256;
-  if (pw_wgrad_takes(B, C, H, W, K, R, S, stride, pad, groups, compute))
-    return (pw_wgrad_partial_bytes(B, C, H, W, K) + 255) / 256 * 256;
-  return 0;
+  WgradPlan p;
+  plan_wgrad_conv(p, B, C, H, W, K, R, S, stride, pad, groups, compute);
+  return round256(p.partial_bytes);
 }
 
 // 0: not taken (aten), 1: bf16-operand tcgen05 kernel (K5), 2: TMA-fed tf32 kernel (K5T), 3: fp32 CUDA-core GEMM of
 // the small 1x1 layers that neither K5T nor K5 takes (csrc/po2_conv_bwd.cu, conv_wgrad_pw_kernel)
 int po2_conv2d_wgrad_kernel_kind(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
                                  int compute) {
-  WgTmaPlan wp;
-  if (wgrad_tma_plan(wp, B, C, H, W, K, R, S, stride, pad, groups, compute)) return 2;
-  ConvGeom g;
-  WgGeom wg;
-  if (wgrad_plan(g, wg, B, C, H, W, K, R, S, stride, pad, groups, compute == 2 ? 0 : compute)) return 1;
-  return pw_wgrad_takes(B, C, H, W, K, R, S, stride, pad, groups, compute) ? 3 : 0;
+  WgradPlan p;
+  plan_wgrad_conv(p, B, C, H, W, K, R, S, stride, pad, groups, compute);
+  return p.kind;
 }
 
 int po2_conv2d_wgrad(const void* g_out, const void* x, void* gw, int B, int C, int H, int W, int K, int R, int S,
@@ -1854,55 +1855,35 @@ int po2_conv2d_wgrad_z(const void* g_out, const void* x, void* gw, int B, int C,
                        int stride, int pad, int groups, int compute, void* workspace, size_t workspace_bytes,
                        void* zeroed_tickets, void* stream) {
   if (!g_out || !x || !gw) return PO2_E_NULL;
-  {
-    WgTmaPlan wp;
-    if (wgrad_tma_plan(wp, B, C, H, W, K, R, S, stride, pad, groups, compute)) {
-      if (!workspace || workspace_bytes < wgrad_tma_partial_bytes(wp)) return PO2_E_WORKSPACE;
-      // measured (profiles/README.md, r02): the in-kernel reduction is SLOWER than the second launch -- 21.5 / 22.3 /
-      // 22.5 us against 20.0 / 15.4 / 13.2 us per ResNet-56 layer class, 3.33 against 3.00 ms per step: the grid
-      // barrier costs more than the launch it saves, and 148 CTAs have far less load parallelism for the partials
-      // than the 1152-CTA reduce kernel (the cooperative launch itself is free: the fused BatchNorm kernels run the
-      // same with a plain launch).  Opt-in only (PO2_WGRAD_FUSED_REDUCE=1).
-      static const bool fuse = [] { const char* e = getenv("PO2_WGRAD_FUSED_REDUCE"); return e && e[0] == '1'; }();
-      if (!aligned16(g_out) || !aligned16(x)) return PO2_E_ALIGN;          // the bases of both tensor maps
-      return launch_wgrad_tma(g_out, x, gw, workspace, wp, (cudaStream_t)stream,
-                              fuse ? (unsigned int*)zeroed_tickets : nullptr);
-    }
-  }
-  ConvGeom g;
-  WgGeom wg;
-  if (!wgrad_plan(g, wg, B, C, H, W, K, R, S, stride, pad, groups, compute == 2 ? 0 : compute)) {
-    if (!pw_wgrad_takes(B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_UNSUPPORTED;
-    if (!workspace || workspace_bytes < pw_wgrad_partial_bytes(B, C, H, W, K)) return PO2_E_WORKSPACE;
-    return launch_pw_wgrad((const float*)g_out, (const float*)x, (float*)gw, workspace, B, C, H * W, K,
-                           (cudaStream_t)stream);
-  }
-  const size_t need = wgrad_partial_bytes(g, wg);
-  if (!workspace || workspace_bytes < need) return PO2_E_WORKSPACE;
-  if (g.vec4 && (!aligned16(g_out) || !aligned16(x))) return PO2_E_ALIGN;   // produce_planes_bf16: 128-bit loads
+  WgradPlan p;
+  plan_wgrad_conv(p, B, C, H, W, K, R, S, stride, pad, groups, compute);
+  if (p.kind == 0) return PO2_E_UNSUPPORTED;
+  if (!workspace || workspace_bytes < p.partial_bytes) return PO2_E_WORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
+  if (p.kind == 2) {
+    // measured (profiles/README.md, r02): the in-kernel reduction is SLOWER than the second launch -- 21.5 / 22.3 /
+    // 22.5 us against 20.0 / 15.4 / 13.2 us per ResNet-56 layer class, 3.33 against 3.00 ms per step: the grid
+    // barrier costs more than the launch it saves, and 148 CTAs have far less load parallelism for the partials
+    // than the 1152-CTA reduce kernel (the cooperative launch itself is free: the fused BatchNorm kernels run the
+    // same with a plain launch).  Opt-in only (PO2_WGRAD_FUSED_REDUCE=1).
+    static const bool fuse = [] { const char* e = getenv("PO2_WGRAD_FUSED_REDUCE"); return e && e[0] == '1'; }();
+    if (!aligned16(g_out) || !aligned16(x)) return PO2_E_ALIGN;          // the bases of both tensor maps
+    return launch_wgrad_tma(g_out, x, gw, workspace, p.wp, st, fuse ? (unsigned int*)zeroed_tickets : nullptr);
+  }
+  if (p.kind == 3)
+    return launch_pw_wgrad((const float*)g_out, (const float*)x, (float*)gw, workspace, B, C, H * W, K, st);
+  if (p.g.vec4 && (!aligned16(g_out) || !aligned16(x))) return PO2_E_ALIGN;   // produce_planes_bf16: 128-bit loads
   static PerDeviceOnce wgrad_once;
   if (cudaError_t e0 = wgrad_once.run([]() -> cudaError_t {
         return cudaFuncSetAttribute(conv_wgrad_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     (int)K3_SMEM_BUDGET + 1024);
       })) return (int)e0;
-  const size_t smem = (size_t)wg.nst * wg.stage_bytes + WG_A_SPAN + 512;
-  conv_wgrad_umma_kernel<<<dim3(wg.m_ctas, wg.tap_splits), K3_THREADS, smem, st>>>((const float*)x, (const float*)g_out,
-                                                                                   (float*)workspace, g, wg);
+  const size_t smem = (size_t)p.wg.nst * p.wg.stage_bytes + WG_A_SPAN + 512;
+  conv_wgrad_umma_kernel<<<dim3(p.wg.m_ctas, p.wg.tap_splits), K3_THREADS, smem, st>>>((const float*)x, (const float*)g_out,
+                                                                                       (float*)workspace, p.g, p.wg);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return (int)e;
-  const int n = wg.ntaps * C * K;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)((n + 31) / 32));
-  cfg.blockDim = dim3(256);
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return (int)cudaLaunchKernelEx(&cfg, conv_wgrad_reduce_kernel, (const float*)workspace, (float*)gw, wg.m_ctas, K, C,
-                                 wg.ntaps);
+  return launch_wgrad_reduce((const float*)workspace, (float*)gw, p.wg.m_ctas, K, C, p.wg.ntaps, st);
 }
 
 }  // extern "C"

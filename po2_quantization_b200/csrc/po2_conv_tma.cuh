@@ -181,7 +181,7 @@ __global__ void __launch_bounds__(KT_THREADS, 2) conv_tma_kernel(const __grid_co
   if (tid == 0) K3_TRACE(6, 1);
   if (warp == KT_EPI_WARPS + 1) {
     // =========================== TMA producer (one lane) ===========================
-    // x was complete before the kernel in front of this one started (see launch_umma: programmatic
+    // x was complete before the kernel in front of this one started (see launch_conv: programmatic
     // launch only behind our own pack / quantize kernels), so no griddepcontrol.wait here.
     // (mode 4 issues 3 * APT boxes per stage: they are spread over the lanes of the warp -- a TMA issue costs a
     // thread ~150 cycles -- lane i owns box i; the other modes have one box per stage, issued by lane 0)
@@ -454,8 +454,7 @@ static size_t tma_smem_bytes(const ConvGeom& g, const TmaPlan& tp) {
 // g: through plan_umma(g, tf32 = true) (supplies the weight-operand plan NT / ntiles_n / Cpad / slab bytes,
 // so that every existing pack path feeds this kernel unchanged).  False: shape stays on the register-fed kernel.
 static bool plan_tma(const ConvGeom& g, TmaPlan& tp) {
-  if (!g.tf32 || g.groups != 1 || g.stride != 1) return false;
-  if (!((g.R == 3 && g.S == 3 && g.pad == 1) || (g.R == 1 && g.S == 1 && g.pad == 0))) return false;
+  if (!g.tf32 || g.groups != 1 || g.stride != 1 || !tc_window(g.R, g.S, g.pad)) return false;
   if (g.C % 8 || g.Cpad != g.C) return false;
   tp = TmaPlan{};
   tp.ntaps = g.R * g.S;
@@ -576,12 +575,7 @@ static bool encode_x_map(CUtensorMap* tm, const void* x, const ConvGeom& g, cons
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-static bool tma_takes(const ConvGeom& g) {
-  TmaPlan tp;
-  return g.tf32 && tma_enabled() && plan_tma(g, tp);
-}
-
-// the conv launch behind the packed operand (same contract as the register-fed launch in launch_umma)
+// the conv launch behind the packed operand (same contract as the register-fed launch in launch_conv)
 static int launch_tma(const void* x, const uint8_t* Bp, const float* scale, void* out, const ConvGeom& g, const TmaPlan& tp_in,
                       cudaStream_t st, int pdl, const ConvEpilogue& ep) {
   TmaPlan tp = tp_in;

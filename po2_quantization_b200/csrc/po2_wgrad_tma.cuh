@@ -397,7 +397,7 @@ __global__ void __launch_bounds__(WT_THREADS, 1) conv_wgrad_tma_kernel(const __g
 // host side
 // ------------------------------------------------------------------------------------------------
 static bool plan_wgrad_tma(WgTmaPlan& wp, int B, int C, int H, int W, int K, int R, int S, int pad) {
-  if (!((R == 3 && S == 3 && pad == 1) || (R == 1 && S == 1 && pad == 0))) return false;
+  if (!tc_window(R, S, pad)) return false;
   if (C % 8 || K % 8 || K > 128 || C > 256) return false;
   wp = WgTmaPlan{};
   wp.ntaps = R * S;
@@ -407,7 +407,7 @@ static bool plan_wgrad_tma(WgTmaPlan& wp, int B, int C, int H, int W, int K, int
   if (wp.ntaps == 9 && !(W == 32 || W == 16 || W == 8 || W == 4)) return false;   // a run holds whole image rows
   if (wp.ntaps == 1) wp.W = 32;
   wp.RPI = (wp.HW + 31) / 32;
-  if ((int64_t)B * C * wp.HW >= (1ll << 31) || (int64_t)B * K * wp.HW >= (1ll << 31)) return false;
+  if (!index_fits(B, C, wp.HW, K, wp.HW)) return false;
   const int sms = sm_count();
   // accumulator columns: all nine taps in one CTA, else the filter rows over blockIdx.y
   const int taps_w = wp.ntaps == 9 ? 3 : 1;
@@ -523,18 +523,7 @@ static int launch_wgrad_tma(const void* g_out, const void* x, void* gw, void* wo
   conv_wgrad_tma_kernel<<<dim3(wp.m_ctas, wp.rsplit), WT_THREADS, smem, st>>>(tmg, tmx, partial, wp, nogw, notk);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return (int)e;
-  const int n = wp.ntaps * wp.C * wp.K;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)((n + 31) / 32));
-  cfg.blockDim = dim3(256);
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return (int)cudaLaunchKernelEx(&cfg, conv_wgrad_reduce_kernel, (const float*)workspace, (float*)gw, wp.m_ctas, wp.K, wp.C,
-                                 wp.ntaps);
+  return launch_wgrad_reduce(partial, gwf, wp.m_ctas, wp.K, wp.C, wp.ntaps, st);
 }
 
 }  // namespace po2

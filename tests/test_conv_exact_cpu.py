@@ -10,6 +10,7 @@ import pytest
 from po2_quantization_b200 import _lib
 
 PO2_E_ALIGN = -5
+PO2_E_UNSUPPORTED = -10
 SMS = 148                        # B200; the library assumes 148 where it cannot ask a device
 
 # ---- forward cases -------------------------------------------------------------------------------------------------
@@ -225,6 +226,16 @@ def test_dgrad_case_runs_on_the_tensor_core_kernel(lib, case):
     assert lib.po2_conv2d_kernel_kind(B, K, H, W, C, k, k, 1, k // 2, 1, compute) in (2, 3), name
     assert lib.po2_conv2d_dgrad_workspace(B, C, H, W, K, k, k, k // 2, compute) > 0, name
     assert (lib.po2_conv2d_dgrad_pack_bytes(B, C, H, W, K, k, k, k // 2, compute) > 0) == packed, name
+
+
+def test_dgrad_workspace_is_zero_where_dgrad_refuses_the_shape(lib):
+    """5x5 pad 2 and 3x3 pad 0 have no tensor-core data gradient: the workspace query agrees with po2_conv2d_dgrad."""
+    ok, big = ctypes.c_void_p(0x1000), 1 << 30
+    for B, C, H, W, K, k, pad in ((2, 8, 8, 8, 8, 5, 2), (2, 8, 8, 8, 8, 3, 0)):
+        for compute in (0, 2):
+            assert lib.po2_conv2d_dgrad_workspace(B, C, H, W, K, k, k, pad, compute) == 0
+            assert lib.po2_conv2d_dgrad(ok, ok, ok, ok, B, C, H, W, K, k, k, 1, pad, 1, 0, 4, 1, compute, ok, big,
+                                        None) == PO2_E_UNSUPPORTED
 
 
 @pytest.mark.parametrize("case", WGRAD, ids=lambda c: c[0])
