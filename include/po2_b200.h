@@ -22,7 +22,9 @@
  *     stride 1 with W % 4 == 0 (W = H*W for 1x1), or on a 1x1 feature map with C % 4 == 0, and the
  *     tcgen05 weight gradients (po2_conv2d_wgrad_kernel_kind 1 or 2) at W % 4 == 0.  The direct,
  *     depthwise and small-pointwise kernels take x at any alignment; the small-pointwise one
- *     (po2_conv2d_kernel_kind 4) needs a 16-byte-aligned fp32 weight when C % 4 == 0;
+ *     (po2_conv2d_kernel_kind 4) needs a 16-byte-aligned fp32 weight when C % 4 == 0.  A bf16 x (the _dt forward
+ *     entry points) carries 8 pixels per 16 bytes, so the same rule reads W % 8 == 0 (W = H*W for 1x1) and, on a
+ *     1x1 feature map, C % 8 == 0; any 2-byte-aligned bf16 x is accepted otherwise;
  *   - re-entrant; the only process-global state is lazily cached device attributes;
  *   - element counts are 64-bit (the quantizer sweep reaches 2^32 elements).
  */
@@ -148,6 +150,35 @@ int po2_conv2d_fwd_ep(const void* x, const void* w, const float* scale, void* ou
 int po2_conv2d_fwd_packed_ep(const void* x, const void* packed, const float* scale, void* out, int B, int C, int H,
                              int W, int K, int R, int S, int stride, int pad, int groups, int compute,
                              const float* ep_a, const float* ep_b, const void* residual, int act, void* stream);
+
+/* The forward of a bf16 model at inference: the same entry points with the storage type of x, out and the residual as
+ * `dtype` (PO2_F32: exactly the forms above; PO2_BF16).  Weights, scale, ep_a / ep_b and the packed operand keep their
+ * formats: a bf16 weight is handed in as its exact fp32 widening.  A bf16 value is exact as a bf16 tensor-core operand,
+ * so a bf16 x runs on the register-fed tcgen05 kernel (kind 2) with bf16 operands in compute 0 and 2 alike (same result;
+ * compute 2 never gives the TMA-fed kind 3 here), on the depthwise kernel (kind 1) or the small-pointwise GEMM (kind 4);
+ * accumulation and the epilogue are fp32, and out is rounded to bf16 (round to nearest even) once.  Training (the
+ * gradients) is fp32 only.  PO2_E_UNSUPPORTED for a bf16 x with compute 1 or a shape that only the direct kernel
+ * takes (kind 0); PO2_E_DTYPE for any other dtype.  NULL ep_a / ep_b / residual with act 0 give the plain forms.
+ * Alignment of a bf16 x: 16 bytes (8 pixels) where the tcgen05 kernel reads it with 128-bit loads -- stride 1 with
+ * W % 8 == 0 (W = H*W for 1x1), or a 1x1 feature map with C % 8 == 0 -- else PO2_E_ALIGN before any launch; the
+ * depthwise kernel takes x at any 2-byte alignment. */
+size_t po2_conv2d_workspace_dt(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
+                               int compute, int dtype);
+int po2_conv2d_kernel_kind_dt(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
+                              int compute, int dtype);
+size_t po2_conv2d_pack_bytes_dt(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
+                                int compute, int dtype);
+int po2_conv2d_pack_dt(const void* w, const float* scale, void* packed, size_t packed_bytes, int B, int C, int H,
+                       int W, int K, int R, int S, int stride, int pad, int groups, int w_format, int bits,
+                       int fsr, int compute, int dtype, void* stream);
+int po2_conv2d_fwd_ep_dt(const void* x, const void* w, const float* scale, void* out, int B, int C, int H, int W, int K,
+                         int R, int S, int stride, int pad, int groups, int w_format, int bits, int fsr, int compute,
+                         void* workspace, size_t workspace_bytes, const float* ep_a, const float* ep_b,
+                         const void* residual, int act, int dtype, void* stream);
+int po2_conv2d_fwd_packed_ep_dt(const void* x, const void* packed, const float* scale, void* out, int B, int C, int H,
+                                int W, int K, int R, int S, int stride, int pad, int groups, int compute,
+                                const float* ep_a, const float* ep_b, const void* residual, int act, int dtype,
+                                void* stream);
 
 /* QuantizedConv2d.forward in QAT mode as one call -- models/quantized_conv.py:34-36: quantize the fp32
  * master weight w (K, C/groups, R, S) with PO2 (mode 0) / PO2+ (mode 1), then convolve.  qw_out receives

@@ -38,6 +38,12 @@ SIGNATURES = {
     "po2_conv2d_pack_bytes": (_sz, [_i] * 11),
     "po2_conv2d_pack": (_i, [_vp, _vp, _vp, _sz] + [_i] * 14 + [_vp]),
     "po2_conv2d_fwd_packed": (_i, [_vp] * 4 + [_i] * 11 + [_vp]),
+    "po2_conv2d_workspace_dt": (_sz, [_i] * 12),
+    "po2_conv2d_kernel_kind_dt": (_i, [_i] * 12),
+    "po2_conv2d_pack_bytes_dt": (_sz, [_i] * 12),
+    "po2_conv2d_pack_dt": (_i, [_vp, _vp, _vp, _sz] + [_i] * 15 + [_vp]),
+    "po2_conv2d_fwd_ep_dt": (_i, [_vp, _vp, _vp, _vp] + [_i] * 14 + [_vp, _sz, _vp, _vp, _vp, _i, _i, _vp]),
+    "po2_conv2d_fwd_packed_ep_dt": (_i, [_vp] * 4 + [_i] * 11 + [_vp, _vp, _vp, _i, _i, _vp]),
     "po2_qconv2d_fwd": (_i, [_vp] * 5 + [_i] * 15 + [_vp, _sz, _vp, _vp]),
     "po2_quantize_pack": (_i, [_vp, _vp, _vp, _vp, _sz] + [_i] * 15 + [_vp, _vp]),
     "po2_multi_desc_bytes": (_sz, []),

@@ -180,7 +180,7 @@ int lin_launch(const float* w, float* y, int K, int C, int RS, int bits, int ite
 struct ConvEpilogue {
   const float* a;
   const float* b;
-  const float* res;      // same shape as the output, or nullptr
+  const float* res;      // same shape as the output, or nullptr; stored in the output's type (bf16 for a bf16 conv)
   int act;
 };
 __device__ __forceinline__ float conv_act(float v, int act) {
@@ -189,10 +189,19 @@ __device__ __forceinline__ float conv_act(float v, int act) {
   if (act == 3) return v / (1.f + __expf(-v));
   return v;
 }
-// v: conv result of out channel k; idx: its offset in the output tensor
+
+// ---- activation storage of the conv forward: fp32, or bf16 (inference of bf16 models).  Arithmetic stays fp32; a
+// bf16 value widens exactly and a result is rounded to bf16 once, when it is stored.
+__device__ __forceinline__ float act_ld(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float act_ld(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
+template <typename I> __device__ __forceinline__ void act_st(float* p, I i, float v) { p[i] = v; }
+template <typename I> __device__ __forceinline__ void act_st(__nv_bfloat16* p, I i, float v) { p[i] = __float2bfloat16_rn(v); }
+
+// v: conv result of out channel k; idx: its offset in the output tensor (and the residual, stored as T)
+template <typename T = float>
 __device__ __forceinline__ float conv_epilogue(float v, const ConvEpilogue& ep, int k, size_t idx) {
   v = fmaf(v, __ldg(ep.a + k), __ldg(ep.b + k));
-  if (ep.res) v += __ldg(ep.res + idx);
+  if (ep.res) v += act_ld(reinterpret_cast<const T*>(ep.res) + idx);
   return conv_act(v, ep.act);
 }
 
@@ -201,8 +210,9 @@ __device__ __forceinline__ float conv_epilogue(float v, const ConvEpilogue& ep, 
 int launch_wgrad_reduce(const float* partial, float* gw, int nparts, int K, int C, int ntaps, cudaStream_t st);
 // csrc/po2_conv_bwd.cu: fp32 cluster split-K GEMM for 1x1 convs on feature maps of <= 16 pixels
 bool pw_small_takes(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups);
-int launch_pw_small(const float* x, const float* w, float* out, int B, int C, int HW, int K, const ConvEpilogue& ep,
-                    cudaStream_t st);
+// x / out: fp32 (dtype PO2_F32) or bf16 (PO2_BF16) NCHW; w: fp32
+int launch_pw_small(const void* x, const float* w, void* out, int B, int C, int HW, int K, const ConvEpilogue& ep,
+                    int dtype, cudaStream_t st);
 // csrc/po2_conv_bwd.cu: the weight gradient of 1x1 stride-1 layers with B*H*W <= 8192 and B*H*W*C*K <= 2^26 -- fp32
 // split-reduction GEMM
 // + the fixed-order reduce kernel (two launches); the workspace holds the partials

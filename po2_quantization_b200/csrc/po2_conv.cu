@@ -16,6 +16,8 @@
 #include <limits.h>
 #include <stdlib.h>
 
+#include <type_traits>
+
 #include "po2_common.cuh"
 
 namespace po2 {
@@ -253,11 +255,15 @@ __device__ __forceinline__ bool elect_one() {
   return pred != 0;
 }
 
-template <int NTAPS, bool TF32>
-__global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const float* __restrict__ x,
+// XT: the activation storage of x, out and the residual -- float, or __nv_bfloat16 (a bf16 model at inference: its
+// values are exact bf16 operands, copied into the strips without conversion; the MMA is kind::f16, accumulation fp32)
+template <int NTAPS, bool TF32, typename XT>
+__global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const XT* __restrict__ x,
                                                                   const uint8_t* __restrict__ Bp,
                                                                   const float* __restrict__ scale,
-                                                                  float* __restrict__ out, ConvGeom g, ConvEpilogue ep) {
+                                                                  XT* __restrict__ out, ConvGeom g, ConvEpilogue ep) {
+  constexpr bool BF16X = sizeof(XT) == 2;
+  static_assert(!(BF16X && TF32), "bf16 activations are kind::f16 operands");
   extern __shared__ __align__(128) uint8_t smem[];
   uint8_t* sB = smem;
   uint8_t* sA = smem + g.b_slab_bytes;
@@ -392,7 +398,7 @@ __global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const float* _
       if (acc) aph1 ^= 1; else aph0 ^= 1;
     }
   } else if (warp < K3_EPI_WARPS) {
-    // =========================== epilogue: TMEM -> scale -> NCHW fp32 ===========================
+    // =========================== epilogue: TMEM -> scale -> NCHW fp32 / bf16 ===========================
     // `scale` may be written by the kernel this one was launched behind with programmatic dependent
     // launch (the fused quantize+pack kernel of po2_qconv2d_fwd): like the weight slab it must not be
     // read before that grid has completed.  The wait costs nothing here -- the first accumulator
@@ -424,29 +430,29 @@ __global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const float* _
         uint32_t r[16];
         tmem_ld16(trow + (uint32_t)cb * 16, r);
         if (valid) {
-          float* po = out + obase + cb * 16 * PQ;
+          XT* po = out + obase + cb * 16 * PQ;
           const int kleft = K - (kbase + cb * 16);
           if (ep.a) {                                            // folded BatchNorm (+ residual) (+ activation)
             float rs[16];
             if (ep.res) {
-              const float* pr = ep.res + obase + cb * 16 * PQ;
+              const XT* pr = reinterpret_cast<const XT*>(ep.res) + obase + cb * 16 * PQ;
 #pragma unroll
-              for (int j = 0; j < 16; ++j) rs[j] = j < kleft ? __ldg(pr + j * PQ) : 0.f;
+              for (int j = 0; j < 16; ++j) rs[j] = j < kleft ? act_ld(pr + j * PQ) : 0.f;
             }
 #pragma unroll
             for (int j = 0; j < 16; ++j)
               if (j < kleft) {
                 float t = fmaf(__uint_as_float(r[j]) * sc, s_ep[0][cb * 16 + j], s_ep[1][cb * 16 + j]);
                 if (ep.res) t += rs[j];
-                po[j * PQ] = conv_act(t, ep.act);
+                act_st(po, j * PQ, conv_act(t, ep.act));
               }
           } else if (kleft >= 16) {
 #pragma unroll
-            for (int j = 0; j < 16; ++j) po[j * PQ] = __uint_as_float(r[j]) * sc;
+            for (int j = 0; j < 16; ++j) act_st(po, j * PQ, __uint_as_float(r[j]) * sc);
           } else {
 #pragma unroll
             for (int j = 0; j < 16; ++j)
-              if (j < kleft) po[j * PQ] = __uint_as_float(r[j]) * sc;
+              if (j < kleft) act_st(po, j * PQ, __uint_as_float(r[j]) * sc);
           }
         }
       }
@@ -458,7 +464,7 @@ __global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const float* _
       aphase ^= (acc == 0);
     }
   } else {
-    // =========================== producers: fp32 NCHW -> bf16 flat K-major strips ===========================
+    // =========================== producers: fp32 / bf16 NCHW -> bf16 (tf32) flat K-major strips ===========================
     // The producer warps form K3_PROD_GROUPS independent groups; group q fills every stage `it` with
     // it % groups == q on its own, so that many stages are in flight against global-memory latency
     // at once (a thread cannot start its next stage before the loads of the current one return).
@@ -472,7 +478,7 @@ __global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const float* _
     const int nphase = g.nphase, nchunk = g.nchunk, nst = g.nst, m_step = g.m_step, nitems = g.nitems_m;
     const int halo = g.halo_before;
     const uint32_t a_stage_bytes = g.a_stage_bytes;
-    const bool hw1 = (HW == 1) && (C % 4 == 0);
+    const bool hw1 = (HW == 1) && (C % (BF16X ? 8 : 4) == 0);
     uint32_t it = 0, s = 0, sphase = 0;
     int turn = 0;                                         // which group owns stage `it`
     for (int m = m_first; m < nitems; m += m_step) {
@@ -490,19 +496,22 @@ __global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const float* _
         const int ngrp = min(CC, Cpad - cbase) / G;
         const int nitem = ngrp * strip;                    // (channel group, position) items per phase
         if (g.vec4) {
-          // ---- fast path (stride 1, W % 4 == 0): one item = 4 consecutive pixels of one image row x
-          // 8 channels = 8 x LDG.128 -> 4 x STS.128; the shared zero column is one extra item per row
-          const int pitch = g.pitch, W4 = W >> 2, ipr = g.items_per_row;     // W4 (+1 with a pad column)
+          // ---- fast path (stride 1, W % PX == 0): one item = PX consecutive pixels of one image row x
+          // 8 channels = 8 x LDG.128 -> PX x STS.128 (PX = 4 fp32 / 8 bf16 pixels per 16 bytes); the shared zero
+          // column is one extra item per row
+          constexpr int PX = BF16X ? 8 : 4, LPX = BF16X ? 3 : 2;
+          using VT = typename std::conditional<BF16X, uint4, float4>::type;
+          const int pitch = g.pitch, W4 = W >> LPX, ipr = g.items_per_row;     // W4 (+1 with a pad column)
           const int rowA = Ls >= 0 ? fdiv(Ls, g.div_pitch) : -((-Ls + pitch - 1) / pitch);
           const int rowB = fdiv(Ls + strip - 1, g.div_pitch);
           // only the row items that overlap the strip: [jA, jB] in the linearised (row, item) space
-          const int jA = min((Ls - rowA * pitch) >> 2, ipr - 1);
-          const int jB = (rowB - rowA) * ipr + min((Ls + strip - 1 - rowB * pitch) >> 2, ipr - 1);
+          const int jA = min((Ls - rowA * pitch) >> LPX, ipr - 1);
+          const int jB = (rowB - rowA) * ipr + min((Ls + strip - 1 - rowB * pitch) >> LPX, ipr - 1);
           const int nrow_items = jB - jA + 1;
           const int nall = ngrp * nrow_items;                 // (channel group, row item) pairs of this stage
           const float inv_items = 1.0f / (float)nrow_items;
           for (int i0 = gt; i0 < nall; i0 += 2 * NPG) {
-            float4 v[2][G];
+            VT v[2][G];
             int lbase[2], npos[2], gsel[2];
 #pragma unroll
             for (int u = 0; u < 2; ++u) {                // 16 x 128-bit loads in flight per thread
@@ -521,33 +530,44 @@ __global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const float* _
                 const int c0 = cbase + grp * G;
                 gsel[u] = grp;
                 cvalid = C - c0;
-                lbase[u] = row * pitch + q4 * 4 - Ls;                       // strip index of pixel 0 of the item
-                npos[u] = q4 < W4 ? 4 : pitch - W;                          // the pad item covers only the pad column
+                lbase[u] = row * pitch + q4 * PX - Ls;                      // strip index of pixel 0 of the item
+                npos[u] = q4 < W4 ? PX : pitch - W;                         // the pad item covers only the pad column
                 const int r0 = row - g.top;
                 if (q4 < W4 && r0 >= 0) {
                   const int img = fdiv(r0, g.div_rows);
                   const int a = r0 - img * g.rows_img;
-                  if (a < H && img < g.B) { ok = true; idx = ((img * C + c0) * H + a) * W + q4 * 4; }
+                  if (a < H && img < g.B) { ok = true; idx = ((img * C + c0) * H + a) * W + q4 * PX; }
                 }
               }
-              const float4* px = reinterpret_cast<const float4*>(x + idx);
+              const VT* px = reinterpret_cast<const VT*>(x + idx);
 #pragma unroll
               for (int c = 0; c < G; ++c)
-                v[u][c] = (ok && c < cvalid) ? __ldg(px + (size_t)c * (HW >> 2)) : make_float4(0.f, 0.f, 0.f, 0.f);
+                v[u][c] = (ok && c < cvalid) ? __ldg(px + (size_t)c * (HW >> LPX)) : VT{};
             }
 #pragma unroll
             for (int u = 0; u < 2; ++u) {
               uint8_t* sgrp = stage + (size_t)gsel[u] * strip * 16;
 #pragma unroll
-              for (int e = 0; e < 4; ++e) {
+              for (int e = 0; e < PX; ++e) {
                 const int lloc = lbase[u] + e;
                 if (e < npos[u] && lloc >= 0 && lloc < strip) {
 #define PO2_C4(q, e_) ((e_) == 0 ? (q).x : (e_) == 1 ? (q).y : (e_) == 2 ? (q).z : (q).w)
-                  float ch[G];                                    // pixel e of every channel of the item
+                  uint4 val;
+                  if constexpr (BF16X) {
+                    // pixel e of channels 2j, 2j+1: the low or high halves of word e / 2 of both loads
+                    const uint32_t sel = (e & 1) ? 0x7632u : 0x5410u;
+                    val = make_uint4(__byte_perm(PO2_C4(v[u][0], e >> 1), PO2_C4(v[u][1], e >> 1), sel),
+                                     __byte_perm(PO2_C4(v[u][2], e >> 1), PO2_C4(v[u][3], e >> 1), sel),
+                                     __byte_perm(PO2_C4(v[u][4], e >> 1), PO2_C4(v[u][5], e >> 1), sel),
+                                     __byte_perm(PO2_C4(v[u][6], e >> 1), PO2_C4(v[u][7], e >> 1), sel));
+                  } else {
+                    float ch[G];                                  // pixel e of every channel of the item
 #pragma unroll
-                  for (int c = 0; c < G; ++c) ch[c] = PO2_C4(v[u][c], e);
+                    for (int c = 0; c < G; ++c) ch[c] = PO2_C4(v[u][c], e);
+                    val = pack_channels<TF32>(ch);
+                  }
 #undef PO2_C4
-                  *reinterpret_cast<uint4*>(sgrp + (size_t)lloc * 16) = pack_channels<TF32>(ch);
+                  *reinterpret_cast<uint4*>(sgrp + (size_t)lloc * 16) = val;
                 }
               }
             }
@@ -558,7 +578,8 @@ __global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const float* _
           uint8_t* sph = stage + (size_t)ph * ngrpCC * strip * 16;
           for (int i0 = gt; i0 < nitem; i0 += PU * NPG) {
             // PU items (PU*G independent loads) in flight per thread before the first conversion
-            float v[PU][G];
+            // (bf16: the raw 16-bit patterns, stored without conversion)
+            typename std::conditional<BF16X, uint32_t, float>::type v[PU][G];
 #pragma unroll
             for (int u = 0; u < PU; ++u) {
               const int i = i0 + u * NPG;
@@ -576,8 +597,18 @@ __global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const float* _
                   }
                 }
               }
-              const float* px = x + idx;
-              if (hw1) {                                   // 1x1 feature map: the G channels are contiguous bytes
+              const XT* px = x + idx;
+              if constexpr (BF16X) {
+                if (hw1) {                                 // 1x1 feature map: the 8 channels are 16 contiguous bytes
+                  const uint4 q = cvalid > 0 ? __ldg(reinterpret_cast<const uint4*>(px)) : make_uint4(0u, 0u, 0u, 0u);
+                  const uint32_t w4[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+                  for (int j = 0; j < G; ++j) v[u][j] = (w4[j >> 1] >> (16 * (j & 1))) & 0xFFFFu;
+                } else {
+#pragma unroll
+                  for (int j = 0; j < G; ++j) v[u][j] = (j < cvalid) ? __bfloat16_as_ushort(__ldg(px + j * HW)) : 0u;
+                }
+              } else if (hw1) {                            // 1x1 feature map: the G channels are contiguous bytes
                 const float4 lo = cvalid > 0 ? __ldg(reinterpret_cast<const float4*>(px)) : make_float4(0.f, 0.f, 0.f, 0.f);
                 v[u][0] = lo.x; v[u][1] = lo.y; v[u][2] = lo.z; v[u][3] = lo.w;
                 if (G == 8) {
@@ -593,7 +624,13 @@ __global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const float* _
             for (int u = 0; u < PU; ++u) {
               const int i = i0 + u * NPG;
               if (i < nitem) {
-                *reinterpret_cast<uint4*>(sph + (size_t)i * 16) = pack_channels<TF32>(v[u]);   // i == grp*strip + lloc
+                uint4 val;
+                if constexpr (BF16X)
+                  val = make_uint4(v[u][0] | (v[u][1] << 16), v[u][2] | (v[u][3] << 16), v[u][4] | (v[u][5] << 16),
+                                   v[u][6] | (v[u][7] << 16));
+                else
+                  val = pack_channels<TF32>(v[u]);
+                *reinterpret_cast<uint4*>(sph + (size_t)i * 16) = val;   // i == grp*strip + lloc
               }
             }
           }
@@ -628,10 +665,11 @@ struct DwGeom {
   FastDiv div_q4, div_p, div_c;
 };
 
-template <int STRIDE>
-__global__ void __launch_bounds__(256) conv_depthwise_vec_kernel(const float* __restrict__ x,
+// XT: float, or __nv_bfloat16 (x, out and the residual of a bf16 model; fp32 arithmetic, 64-bit loads and stores)
+template <int STRIDE, typename XT>
+__global__ void __launch_bounds__(256) conv_depthwise_vec_kernel(const XT* __restrict__ x,
                                                                  const float* __restrict__ w,
-                                                                 float* __restrict__ out, DwGeom g, ConvEpilogue ep) {
+                                                                 XT* __restrict__ out, DwGeom g, ConvEpilogue ep) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < g.total; i += gridDim.x * blockDim.x) {
     int t = fdiv(i, g.div_q4);
     const int q0 = (i - t * g.Q4) * 4;
@@ -639,7 +677,7 @@ __global__ void __launch_bounds__(256) conv_depthwise_vec_kernel(const float* __
     const int p = t - u * g.P;
     const int plane = u;                                   // n * C + c
     const int c = plane - fdiv(plane, g.div_c) * g.C;
-    const float* px = x + (size_t)plane * g.H * g.W;
+    const XT* px = x + (size_t)plane * g.H * g.W;
     const float* pw = w + c * 9;
     float wk[9];
 #pragma unroll
@@ -651,17 +689,31 @@ __global__ void __launch_bounds__(256) conv_depthwise_vec_kernel(const float* __
     for (int r = 0; r < 3; ++r) {
       const int ih = p * STRIDE - 1 + r;
       if (ih < 0 || ih >= g.H) continue;
-      const float* row = px + ih * g.W;
+      const XT* row = px + ih * g.W;
       float in[NIN];
-      // columns iw0+1 .. iw0+4 (and +5..+8 for stride 2) are 16-byte aligned groups inside the row
-      const float4 a = __ldg(reinterpret_cast<const float4*>(row + iw0 + 1));
-      in[0] = iw0 >= 0 ? __ldg(row + iw0) : 0.f;
-      in[1] = a.x; in[2] = a.y; in[3] = a.z; in[4] = a.w;
-      if (STRIDE == 1) {
-        in[5] = (iw0 + 5 < g.W) ? __ldg(row + iw0 + 5) : 0.f;
+      // columns iw0+1 .. iw0+4 (and +5..+8 for stride 2) are 16-byte (bf16: 8-byte) aligned groups inside the row
+      if constexpr (sizeof(XT) == 2) {
+        const uint2 a = __ldg(reinterpret_cast<const uint2*>(row + iw0 + 1));
+        in[0] = iw0 >= 0 ? act_ld(row + iw0) : 0.f;
+        in[1] = __uint_as_float(a.x << 16); in[2] = __uint_as_float(a.x & 0xFFFF0000u);
+        in[3] = __uint_as_float(a.y << 16); in[4] = __uint_as_float(a.y & 0xFFFF0000u);
+        if (STRIDE == 1) {
+          in[5] = (iw0 + 5 < g.W) ? act_ld(row + iw0 + 5) : 0.f;
+        } else {
+          const uint2 b = __ldg(reinterpret_cast<const uint2*>(row + iw0 + 5));
+          in[5] = __uint_as_float(b.x << 16); in[6] = __uint_as_float(b.x & 0xFFFF0000u);
+          in[7] = __uint_as_float(b.y << 16); in[8] = __uint_as_float(b.y & 0xFFFF0000u);
+        }
       } else {
-        const float4 b = __ldg(reinterpret_cast<const float4*>(row + iw0 + 5));
-        in[5] = b.x; in[6] = b.y; in[7] = b.z; in[8] = b.w;
+        const float4 a = __ldg(reinterpret_cast<const float4*>(row + iw0 + 1));
+        in[0] = iw0 >= 0 ? __ldg(row + iw0) : 0.f;
+        in[1] = a.x; in[2] = a.y; in[3] = a.z; in[4] = a.w;
+        if (STRIDE == 1) {
+          in[5] = (iw0 + 5 < g.W) ? __ldg(row + iw0 + 5) : 0.f;
+        } else {
+          const float4 b = __ldg(reinterpret_cast<const float4*>(row + iw0 + 5));
+          in[5] = b.x; in[6] = b.y; in[7] = b.z; in[8] = b.w;
+        }
       }
 #pragma unroll
       for (int o = 0; o < 4; ++o)
@@ -671,16 +723,22 @@ __global__ void __launch_bounds__(256) conv_depthwise_vec_kernel(const float* __
     const size_t o = ((size_t)plane * g.P + p) * g.Q + q0;
     if (ep.a) {
 #pragma unroll
-      for (int e = 0; e < 4; ++e) acc[e] = conv_epilogue(acc[e], ep, c, o + e);
+      for (int e = 0; e < 4; ++e) acc[e] = conv_epilogue<XT>(acc[e], ep, c, o + e);
     }
-    *reinterpret_cast<float4*>(out + o) = make_float4(acc[0], acc[1], acc[2], acc[3]);
+    if constexpr (sizeof(XT) == 2) {
+      const __nv_bfloat162 lo = __floats2bfloat162_rn(acc[0], acc[1]), hi = __floats2bfloat162_rn(acc[2], acc[3]);
+      *reinterpret_cast<uint2*>(out + o) = make_uint2(*reinterpret_cast<const uint32_t*>(&lo), *reinterpret_cast<const uint32_t*>(&hi));
+    } else {
+      *reinterpret_cast<float4*>(out + o) = make_float4(acc[0], acc[1], acc[2], acc[3]);
+    }
   }
 }
 
 // any other depthwise shape: one thread per output element
-__global__ void __launch_bounds__(256) conv_depthwise_kernel(const float* __restrict__ x,
+template <typename XT>
+__global__ void __launch_bounds__(256) conv_depthwise_kernel(const XT* __restrict__ x,
                                                              const float* __restrict__ w,
-                                                             float* __restrict__ out, ConvGeom g,
+                                                             XT* __restrict__ out, ConvGeom g,
                                                              FastDiv div_q, FastDiv div_p, FastDiv div_c, ConvEpilogue ep) {
   const int total = g.B * g.C * g.P * g.Q;                 // < 2^31 (checked on the host)
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
@@ -689,7 +747,7 @@ __global__ void __launch_bounds__(256) conv_depthwise_kernel(const float* __rest
     const int plane = fdiv(t, div_p);
     const int p = t - plane * g.P;
     const int c = plane - fdiv(plane, div_c) * g.C;
-    const float* px = x + (size_t)plane * g.H * g.W;
+    const XT* px = x + (size_t)plane * g.H * g.W;
     const float* pw = w + (size_t)c * g.R * g.S;
     float acc = 0.0f;
     for (int r = 0; r < g.R; ++r) {
@@ -698,10 +756,10 @@ __global__ void __launch_bounds__(256) conv_depthwise_kernel(const float* __rest
       for (int s = 0; s < g.S; ++s) {
         const int iw = q * g.stride - g.pad + s;
         if (iw < 0 || iw >= g.W) continue;
-        acc = fmaf(__ldg(px + ih * g.W + iw), __ldg(pw + r * g.S + s), acc);
+        acc = fmaf(act_ld(px + ih * g.W + iw), __ldg(pw + r * g.S + s), acc);
       }
     }
-    out[i] = ep.a ? conv_epilogue(acc, ep, c, (size_t)i) : acc;
+    act_st(out, i, ep.a ? conv_epilogue<XT>(acc, ep, c, (size_t)i) : acc);
   }
 }
 
@@ -802,8 +860,9 @@ static size_t umma_smem_bytes(const ConvGeom& g) {
   return (size_t)g.b_slab_bytes + (size_t)g.nst * g.a_stage_bytes + (3 * K3_MAX_STAGES + 8) * 8 + 64;
 }
 
-// returns false if the shape does not fit the kernel's shared-memory plan
-static bool plan_umma(ConvGeom& g, bool tf32) {
+// returns false if the shape does not fit the kernel's shared-memory plan.  bf16x: x is bf16 (16 bytes = 8 pixels on
+// the producers' fast path)
+static bool plan_umma(ConvGeom& g, bool tf32, bool bf16x = false) {
   const bool k3 = (g.R == 3);
   g.tf32 = tf32 ? 1 : 0;
   g.G = tf32 ? 4 : 8;
@@ -878,8 +937,9 @@ static bool plan_umma(ConvGeom& g, bool tf32) {
   g.div_NT = make_fastdiv((uint32_t)g.NT);
   g.div_ncg = make_fastdiv((uint32_t)(g.Cpad / G));
   g.div_taps = make_fastdiv((uint32_t)g.ntaps);
-  g.vec4 = (g.stride == 1 && g.W % 4 == 0) ? 1 : 0;
-  g.items_per_row = g.W / 4 + (g.pitch > g.W ? 1 : 0);
+  const int px = bf16x ? 8 : 4;
+  g.vec4 = (g.stride == 1 && g.W % px == 0) ? 1 : 0;
+  g.items_per_row = g.W / px + (g.pitch > g.W ? 1 : 0);
   g.div_ipr = make_fastdiv((uint32_t)(g.items_per_row > 0 ? g.items_per_row : 1));
   return true;
 }
@@ -903,34 +963,40 @@ struct ConvPlan {
   size_t pack_bytes;     // the packed weight operand of kinds 2 / 3; 0 for the other kinds
   size_t workspace;      // what the launching entry point needs
   bool unpadded;         // kinds 2 / 3: the operand has no channel padding, so the fused quantizers can emit it
+  int dtype;             // storage of x / out / residual: PO2_F32, or PO2_BF16 (kinds 1, 2 and 4 only)
 };
 
 static size_t round256(size_t n) { return (n + 255) / 256 * 256; }
 
 // K3, or K3T where the TMA-fed kernel takes the planned geometry (it reads the 3x3 operand tap-minor); false: the
-// shape does not fit K3's shared-memory plan
+// shape does not fit K3's shared-memory plan.  A bf16 x runs on K3 with bf16 operands (exact, whatever the mode).
 static bool plan_tc(ConvPlan& p, bool tf32) {
-  if (!plan_umma(p.g, tf32)) return false;
-  p.kind = (tf32 && tma_enabled() && plan_tma(p.g, p.tp)) ? 3 : 2;
+  const bool bf16x = p.dtype == PO2_BF16;
+  if (!plan_umma(p.g, tf32 && !bf16x, bf16x)) return false;
+  p.kind = (tf32 && !bf16x && tma_enabled() && plan_tma(p.g, p.tp)) ? 3 : 2;
   p.g.tapminor = (p.kind == 3 && p.g.ntaps == 9) ? 1 : 0;
   p.pack_bytes = (size_t)p.g.ntiles_n * p.g.b_slab_bytes;
   p.unpadded = p.g.Cpad == p.g.C && p.g.ntiles_n * p.g.NT == p.g.K;
   return true;
 }
 
-// false: not a conv shape (PO2_E_SHAPE)
-static bool plan_fwd(ConvPlan& p, int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
-                     int compute) {
+// 0, PO2_E_SHAPE (not a conv shape), PO2_E_DTYPE, or PO2_E_UNSUPPORTED: a bf16 x on the fp32 CUDA cores (compute 1)
+// or on the direct kernel.  dtype: the storage of x / out / residual, PO2_F32 or PO2_BF16 (weights are fp32 either way)
+static int plan_fwd(ConvPlan& p, int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
+                    int compute, int dtype = PO2_F32) {
   p = ConvPlan{};
-  if (!fill_geom(p.g, B, C, H, W, K, R, S, stride, pad, groups)) return false;
+  if (dtype != PO2_F32 && dtype != PO2_BF16) return PO2_E_DTYPE;
+  p.dtype = dtype;
+  if (!fill_geom(p.g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
   // the pointwise layers on tiny feature maps go to the fp32 cluster GEMM of csrc/po2_conv_bwd.cu, not to K3 / K3T
   const bool pw_small = pw_small_takes(B, C, H, W, K, R, S, stride, pad, groups);
   if (compute == 1 || !umma_shape_ok(p.g) || pw_small || !plan_tc(p, compute == 2))
     p.kind = pw_small ? 4 : (groups == C && groups == K) ? 1 : 0;
+  if (dtype == PO2_BF16 && (compute == 1 || p.kind == 0)) return PO2_E_UNSUPPORTED;
   // the decoded fp32 weights (codes input), then the packed operand
   const size_t wbytes = (size_t)K * (C / groups) * R * S * sizeof(float);
   p.workspace = round256(wbytes + (p.pack_bytes ? p.pack_bytes + 256 : 0));
-  return true;
+  return 0;
 }
 
 // The data gradient of a stride-1 dense layer (x: B, C, H, W; w: K, C, R, S) is the forward conv of the output
@@ -971,11 +1037,13 @@ static bool pdl_chain_enabled() {
 }
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
-// K3's activation producers read x with 128-bit loads on the vec4 path (stride 1, W % 4 == 0) and on the hw1 path
-// (1x1 feature map, C % 4 == 0); K3T's tensor map needs a 16-byte-aligned base too, and every geometry plan_tma
-// takes is stride 1 with W % 4 == 0, i.e. has vec4 set.  PO2_E_ALIGN before any launch when x does not allow that.
-static int umma_check_x(const void* x, const ConvGeom& g) {
-  const bool wide_loads = g.vec4 || (g.H * g.W == 1 && g.C % 4 == 0);
+// K3's activation producers read x with 128-bit loads on the vec4 path (stride 1, W % 4 == 0; bf16: W % 8 == 0) and on
+// the hw1 path (1x1 feature map, C % 4 == 0; bf16: C % 8 == 0); K3T's tensor map needs a 16-byte-aligned base too, and
+// every geometry plan_tma takes is stride 1 with W % 4 == 0, i.e. has vec4 set.  PO2_E_ALIGN before any launch when x
+// does not allow that.
+static int umma_check_x(const void* x, const ConvPlan& p) {
+  const ConvGeom& g = p.g;
+  const bool wide_loads = g.vec4 || (g.H * g.W == 1 && g.C % (p.dtype == PO2_BF16 ? 8 : 4) == 0);
   return (wide_loads && !aligned16(x)) ? PO2_E_ALIGN : 0;
 }
 
@@ -1006,10 +1074,14 @@ static int launch_conv(const ConvPlan& p, const void* x, const void* Bp, const f
   static PerDeviceOnce attr_once;                       // the opt-in shared-memory size is a per-device attribute
   cudaError_t e = attr_once.run([]() -> cudaError_t {
     const int smax = (int)K3_SMEM_BUDGET + 1024;
-    cudaError_t a = cudaFuncSetAttribute(conv_umma_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
-    if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<9, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
-    if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
-    if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<9, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+    cudaError_t a = cudaFuncSetAttribute(conv_umma_kernel<1, false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+    if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<9, false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+    if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<1, true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+    if (a == cudaSuccess) a = cudaFuncSetAttribute(conv_umma_kernel<9, true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+    if (a == cudaSuccess)
+      a = cudaFuncSetAttribute(conv_umma_kernel<1, false, __nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+    if (a == cudaSuccess)
+      a = cudaFuncSetAttribute(conv_umma_kernel<9, false, __nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
     return a;
   });
   if (e != cudaSuccess) return (int)e;
@@ -1026,12 +1098,17 @@ static int launch_conv(const ConvPlan& p, const void* x, const void* Bp, const f
   const float* xf = (const float*)x;
   const uint8_t* bpc = (const uint8_t*)Bp;
   float* of = (float*)out;
-  if (g.tf32) {
-    if (g.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<1, true>, xf, bpc, scale, of, g, ep);
-    else e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<9, true>, xf, bpc, scale, of, g, ep);
+  if (p.dtype == PO2_BF16) {
+    const __nv_bfloat16* xb = (const __nv_bfloat16*)x;
+    __nv_bfloat16* ob = (__nv_bfloat16*)out;
+    if (g.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<1, false, __nv_bfloat16>, xb, bpc, scale, ob, g, ep);
+    else e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<9, false, __nv_bfloat16>, xb, bpc, scale, ob, g, ep);
+  } else if (g.tf32) {
+    if (g.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<1, true, float>, xf, bpc, scale, of, g, ep);
+    else e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<9, true, float>, xf, bpc, scale, of, g, ep);
   } else {
-    if (g.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<1, false>, xf, bpc, scale, of, g, ep);
-    else e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<9, false>, xf, bpc, scale, of, g, ep);
+    if (g.ntaps == 1) e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<1, false, float>, xf, bpc, scale, of, g, ep);
+    else e = cudaLaunchKernelEx(&cfg, conv_umma_kernel<9, false, float>, xf, bpc, scale, of, g, ep);
   }
   return (int)e;
 }
@@ -1439,8 +1516,13 @@ int po2_debug_set_trace(void* buf) {
 
 size_t po2_conv2d_workspace(int B, int C, int H, int W, int K, int R, int S, int stride, int pad,
                             int groups, int compute) {
+  return po2_conv2d_workspace_dt(B, C, H, W, K, R, S, stride, pad, groups, compute, PO2_F32);
+}
+
+size_t po2_conv2d_workspace_dt(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
+                               int compute, int dtype) {
   ConvPlan p;
-  return plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute) ? p.workspace : 0;
+  return plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute, dtype) ? 0 : p.workspace;
 }
 
 // which kernel po2_conv2d_fwd runs for this geometry: 0 direct fp32, 1 depthwise, 2 tcgen05 with the
@@ -1448,8 +1530,14 @@ size_t po2_conv2d_workspace(int B, int C, int H, int W, int K, int R, int S, int
 // pointwise layers on <= 16-pixel feature maps; < 0: PO2_E_*
 int po2_conv2d_kernel_kind(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
                            int compute) {
+  return po2_conv2d_kernel_kind_dt(B, C, H, W, K, R, S, stride, pad, groups, compute, PO2_F32);
+}
+
+int po2_conv2d_kernel_kind_dt(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
+                              int compute, int dtype) {
   ConvPlan p;
-  return plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute) ? p.kind : PO2_E_SHAPE;
+  const int e = plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute, dtype);
+  return e ? e : p.kind;
 }
 
 static int check_epilogue(const float* ep_a, const float* ep_b, int act) {
@@ -1472,12 +1560,20 @@ int po2_conv2d_fwd_ep(const void* x, const void* w, const float* scale, void* ou
                       int W, int K, int R, int S, int stride, int pad, int groups, int w_format,
                       int bits, int fsr, int compute, void* workspace, size_t workspace_bytes,
                       const float* ep_a, const float* ep_b, const void* residual, int act, void* stream) {
+  return po2_conv2d_fwd_ep_dt(x, w, scale, out, B, C, H, W, K, R, S, stride, pad, groups, w_format, bits, fsr, compute,
+                              workspace, workspace_bytes, ep_a, ep_b, residual, act, PO2_F32, stream);
+}
+
+int po2_conv2d_fwd_ep_dt(const void* x, const void* w, const float* scale, void* out, int B, int C, int H,
+                         int W, int K, int R, int S, int stride, int pad, int groups, int w_format,
+                         int bits, int fsr, int compute, void* workspace, size_t workspace_bytes,
+                         const float* ep_a, const float* ep_b, const void* residual, int act, int dtype, void* stream) {
   if (!x || !w || !out) return PO2_E_NULL;
   if (int e = check_epilogue(ep_a, ep_b, act)) return e;
   if (!ep_a && (residual || act)) return PO2_E_NULL;
   const ConvEpilogue ep{ep_a, ep_b, (const float*)residual, act};
   ConvPlan p;
-  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (int e = plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute, dtype)) return e;
   const ConvGeom& g = p.g;
   if (w_format != PO2_W_F32_PO2 && w_format != PO2_W_CODES) return PO2_E_UNSUPPORTED;
   if (w_format == PO2_W_CODES && (!scale || bits < 2 || bits > 8)) return PO2_E_BITS;
@@ -1488,7 +1584,7 @@ int po2_conv2d_fwd_ep(const void* x, const void* w, const float* scale, void* ou
 
   if (p.pack_bytes) {
     if (!workspace || workspace_bytes < p.workspace) return PO2_E_WORKSPACE;
-    if (int a = umma_check_x(x, g)) return a;
+    if (int a = umma_check_x(x, p)) return a;
     void* Bp = reinterpret_cast<char*>(workspace) + wbytes;
     if (int e = launch_pack(p, w, w_format, scale, bits, fsr, 0, Bp, st)) return e;
     return launch_conv(p, x, Bp, scale, out, 1, ep, st);
@@ -1505,7 +1601,7 @@ int po2_conv2d_fwd_ep(const void* x, const void* w, const float* scale, void* ou
     if (e != cudaSuccess) return (int)e;
     wf = (const float*)workspace;
   }
-  if (p.kind == 4) return launch_pw_small((const float*)x, wf, (float*)out, B, C, H * W, K, ep, st);
+  if (p.kind == 4) return launch_pw_small(x, wf, out, B, C, H * W, K, ep, dtype, st);
   if (p.kind == 1) {
     const int64_t total = (int64_t)B * C * g.P * g.Q;
     // vector kernel: 3x3 pad 1, stride 1 or 2, rows and outputs in whole 16-byte groups
@@ -1516,13 +1612,21 @@ int po2_conv2d_fwd_ep(const void* x, const void* w, const float* scale, void* ou
       d.total = (int)(total / 4);
       d.div_q4 = make_fastdiv((uint32_t)d.Q4); d.div_p = make_fastdiv((uint32_t)g.P); d.div_c = make_fastdiv((uint32_t)C);
       const int blocks = (int)((d.total + 255) / 256 < sm_count() * 16 ? (d.total + 255) / 256 : sm_count() * 16);
-      if (stride == 1) conv_depthwise_vec_kernel<1><<<blocks, 256, 0, st>>>((const float*)x, wf, (float*)out, d, ep);
-      else conv_depthwise_vec_kernel<2><<<blocks, 256, 0, st>>>((const float*)x, wf, (float*)out, d, ep);
+      const bool bf = dtype == PO2_BF16;
+      using BF = __nv_bfloat16;
+      if (stride == 1 && bf) conv_depthwise_vec_kernel<1, BF><<<blocks, 256, 0, st>>>((const BF*)x, wf, (BF*)out, d, ep);
+      else if (stride == 1) conv_depthwise_vec_kernel<1, float><<<blocks, 256, 0, st>>>((const float*)x, wf, (float*)out, d, ep);
+      else if (bf) conv_depthwise_vec_kernel<2, BF><<<blocks, 256, 0, st>>>((const BF*)x, wf, (BF*)out, d, ep);
+      else conv_depthwise_vec_kernel<2, float><<<blocks, 256, 0, st>>>((const float*)x, wf, (float*)out, d, ep);
       return (int)cudaGetLastError();
     }
     const int blocks = (int)((total + 255) / 256 < (int64_t)sm_count() * 16 ? (total + 255) / 256 : (int64_t)sm_count() * 16);
-    conv_depthwise_kernel<<<blocks, 256, 0, st>>>((const float*)x, wf, (float*)out, g, make_fastdiv((uint32_t)g.Q),
-                                                  make_fastdiv((uint32_t)g.P), make_fastdiv((uint32_t)C), ep);
+    const FastDiv dq = make_fastdiv((uint32_t)g.Q), dp = make_fastdiv((uint32_t)g.P), dc = make_fastdiv((uint32_t)C);
+    if (dtype == PO2_BF16)
+      conv_depthwise_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>((const __nv_bfloat16*)x, wf, (__nv_bfloat16*)out, g,
+                                                                   dq, dp, dc, ep);
+    else
+      conv_depthwise_kernel<float><<<blocks, 256, 0, st>>>((const float*)x, wf, (float*)out, g, dq, dp, dc, ep);
     return (int)cudaGetLastError();
   }
   const int Cg = C / groups, Kg = K / groups;
@@ -1552,7 +1656,7 @@ int po2_conv2d_dgrad(const void* g_out, const void* w, const float* scale, void*
   ConvPlan p;
   if (int e = plan_dgrad(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return e;
   if (!workspace || workspace_bytes < p.workspace) return PO2_E_WORKSPACE;
-  if (int a = umma_check_x(g_out, p.g)) return a;
+  if (int a = umma_check_x(g_out, p)) return a;
   cudaStream_t st = (cudaStream_t)stream;
   if (int e = launch_pack(p, w, w_format, scale, bits, fsr, 1, workspace, st)) return e;
   return launch_conv(p, g_out, workspace, scale, gx, 1, ConvEpilogue{}, st);
@@ -1562,18 +1666,30 @@ int po2_conv2d_dgrad(const void* g_out, const void* w, const float* scale, void*
 // po2_conv2d_pack_bytes == 0 means the shape does not run on the tensor-core kernel.
 size_t po2_conv2d_pack_bytes(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
                              int compute) {
+  return po2_conv2d_pack_bytes_dt(B, C, H, W, K, R, S, stride, pad, groups, compute, PO2_F32);
+}
+
+size_t po2_conv2d_pack_bytes_dt(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups,
+                                int compute, int dtype) {
   ConvPlan p;
-  return plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute) ? round256(p.pack_bytes) : 0;
+  return plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute, dtype) ? 0 : round256(p.pack_bytes);
 }
 
 int po2_conv2d_pack(const void* w, const float* scale, void* packed, size_t packed_bytes, int B, int C, int H,
                     int W, int K, int R, int S, int stride, int pad, int groups, int w_format, int bits,
                     int fsr, int compute, void* stream) {
+  return po2_conv2d_pack_dt(w, scale, packed, packed_bytes, B, C, H, W, K, R, S, stride, pad, groups, w_format, bits, fsr,
+                            compute, PO2_F32, stream);
+}
+
+int po2_conv2d_pack_dt(const void* w, const float* scale, void* packed, size_t packed_bytes, int B, int C, int H,
+                       int W, int K, int R, int S, int stride, int pad, int groups, int w_format, int bits,
+                       int fsr, int compute, int dtype, void* stream) {
   if (!w || !packed) return PO2_E_NULL;
   if (w_format != PO2_W_F32_PO2 && w_format != PO2_W_CODES) return PO2_E_UNSUPPORTED;
   if (w_format == PO2_W_CODES && (!scale || bits < 2 || bits > 8)) return PO2_E_BITS;
   ConvPlan p;
-  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (int e = plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute, dtype)) return e;
   if (!p.pack_bytes) return PO2_E_UNSUPPORTED;
   if (packed_bytes < p.pack_bytes) return PO2_E_WORKSPACE;
   return launch_pack(p, w, w_format, scale, bits, fsr, 0, packed, (cudaStream_t)stream);
@@ -1588,15 +1704,23 @@ int po2_conv2d_fwd_packed(const void* x, const void* packed, const float* scale,
 int po2_conv2d_fwd_packed_ep(const void* x, const void* packed, const float* scale, void* out, int B, int C, int H,
                              int W, int K, int R, int S, int stride, int pad, int groups, int compute,
                              const float* ep_a, const float* ep_b, const void* residual, int act, void* stream) {
+  return po2_conv2d_fwd_packed_ep_dt(x, packed, scale, out, B, C, H, W, K, R, S, stride, pad, groups, compute, ep_a, ep_b,
+                                     residual, act, PO2_F32, stream);
+}
+
+int po2_conv2d_fwd_packed_ep_dt(const void* x, const void* packed, const float* scale, void* out, int B, int C, int H,
+                                int W, int K, int R, int S, int stride, int pad, int groups, int compute,
+                                const float* ep_a, const float* ep_b, const void* residual, int act, int dtype,
+                                void* stream) {
   if (!x || !packed || !out) return PO2_E_NULL;
   if (int e = check_epilogue(ep_a, ep_b, act)) return e;
   if (!ep_a && (residual || act)) return PO2_E_NULL;
   const ConvEpilogue ep{ep_a, ep_b, (const float*)residual, act};
   ConvPlan p;
-  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (int e = plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute, dtype)) return e;
   if (!p.pack_bytes) return PO2_E_UNSUPPORTED;
   if (!index_fits(p.g)) return PO2_E_SIZE;
-  if (int a = umma_check_x(x, p.g)) return a;
+  if (int a = umma_check_x(x, p)) return a;
   return launch_conv(p, x, packed, scale, out, pdl_chain_enabled() ? 2 : 0, ep, (cudaStream_t)stream);
 }
 
@@ -1612,11 +1736,11 @@ int po2_qconv2d_fwd(const void* x, const void* w_master, void* qw_out, float* sc
   if (!x || !w_master || !qw_out || !scale_out || !out) return PO2_E_NULL;
   if (!quant_workspace) return PO2_E_WORKSPACE;
   ConvPlan p;
-  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (int e = plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return e;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t wn = (int64_t)K * (C / groups) * R * S;
   if (p.pack_bytes)
-    if (int a = umma_check_x(x, p.g)) return a;               // before the quantizer runs
+    if (int a = umma_check_x(x, p)) return a;                 // before the quantizer runs
   if (p.unpadded) {
     if (!workspace || workspace_bytes < p.workspace) return PO2_E_WORKSPACE;
     if (!index_fits(p.g)) return PO2_E_SIZE;
@@ -1640,7 +1764,7 @@ int po2_quantize_pack(const void* w_master, void* qw_out, float* scale_out, void
   if (!w_master || !qw_out || !scale_out || !packed) return PO2_E_NULL;
   if (!quant_workspace) return PO2_E_WORKSPACE;
   ConvPlan p;
-  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (int e = plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return e;
   if (!p.pack_bytes) return PO2_E_UNSUPPORTED;
   if (packed_bytes < p.pack_bytes) return PO2_E_WORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
@@ -1665,7 +1789,7 @@ int po2_multi_desc_fill(void* host_table, int index, const void* w_master, void*
   if (!host_table || index < 0 || !w_master || !qw_out || !scale_out || !packed) return PO2_E_NULL;
   if (int e = check_quant_args(bits, fsr, mode, flavor)) return e;
   ConvPlan p;
-  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (int e = plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return e;
   if (!p.unpadded) return PO2_E_UNSUPPORTED;             // no tensor-core operand, or one with channel padding
   if (packed_bytes < p.pack_bytes) return PO2_E_WORKSPACE;
   const int64_t wn = (int64_t)K * (C / groups) * R * S;
@@ -1716,7 +1840,7 @@ int po2_multi_desc_fill_dgrad(void* host_table, int index, void* packed_dgrad, s
 static int lin_pack_args(PackArgs& pk, ConvPlan& p, void* packed, size_t packed_bytes, void* packed_dgrad,
                          size_t dgrad_bytes, int B, int C, int H, int W, int K, int R, int S, int stride, int pad,
                          int groups, int bits, int num_iters, int compute) {
-  if (!plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return PO2_E_SHAPE;
+  if (int e = plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute)) return e;
   if (!p.pack_bytes) return PO2_E_UNSUPPORTED;
   if (num_iters < 1 || bits > (p.g.tf32 ? 12 : 9)) return PO2_E_UNSUPPORTED;    // step not a power of two / not exact
   if (packed_bytes < p.pack_bytes) return PO2_E_WORKSPACE;
@@ -1782,7 +1906,7 @@ int po2_conv2d_dgrad_packed(const void* g_out, const void* packed, const float* 
   if (!g_out || !packed || !gx) return PO2_E_NULL;
   ConvPlan p;
   if (plan_dgrad(p, B, C, H, W, K, R, S, 1, pad, 1, compute)) return PO2_E_UNSUPPORTED;
-  if (int a = umma_check_x(g_out, p.g)) return a;
+  if (int a = umma_check_x(g_out, p)) return a;
   return launch_conv(p, g_out, packed, scale, gx, pdl_chain_enabled() ? 2 : 0, ConvEpilogue{}, (cudaStream_t)stream);
 }
 

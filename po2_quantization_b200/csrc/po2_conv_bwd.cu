@@ -331,8 +331,10 @@ __device__ __forceinline__ float pw_ld_remote(const float* local, uint32_t rank)
   return v;
 }
 
-__global__ void __launch_bounds__(PW_THREADS) conv_pw_small_kernel(const float* __restrict__ x, const float* __restrict__ w,
-                                                                   float* __restrict__ out, PwGeom g, ConvEpilogue ep) {
+// XT: the activation storage (float, or __nv_bfloat16 for a bf16 conv; the arithmetic is fp32 either way)
+template <typename XT>
+__global__ void __launch_bounds__(PW_THREADS) conv_pw_small_kernel(const XT* __restrict__ x, const float* __restrict__ w,
+                                                                   XT* __restrict__ out, PwGeom g, ConvEpilogue ep) {
   __shared__ __align__(16) float As[PW_TK][PW_TM + 4];
   __shared__ __align__(16) float Bs[PW_TK][PW_TN + 4];
   __shared__ float red[PW_TM][PW_TN + 1];                  // this CTA's partial tile, read by cluster rank 0
@@ -357,7 +359,7 @@ __global__ void __launch_bounds__(PW_THREADS) conv_pw_small_kernel(const float* 
       float v = 0.f;
       if (m < M && c < C) {
         const int n = fdiv(m, g.div_hw);
-        v = __ldg(x + ((size_t)n * C + c) * HW + (m - n * HW));
+        v = act_ld(x + ((size_t)n * C + c) * HW + (m - n * HW));
       }
       av[e] = v;
     }
@@ -415,7 +417,7 @@ __global__ void __launch_bounds__(PW_THREADS) conv_pw_small_kernel(const float* 
         for (int r = 1; r < 8; ++r) v += t[r];
         if (k < K) {
           const size_t o = ((size_t)n * K + k) * HW + hw;
-          out[o] = ep.a ? conv_epilogue(v, ep, k, o) : v;
+          act_st(out, o, ep.a ? conv_epilogue<XT>(v, ep, k, o) : v);
         }
       }
     }
@@ -432,7 +434,7 @@ __global__ void __launch_bounds__(PW_THREADS) conv_pw_small_kernel(const float* 
       const int k = k0 + tx * 4 + j;
       if (k >= K) continue;
       const size_t o = ((size_t)n * K + k) * HW + hw;
-      out[o] = ep.a ? conv_epilogue(acc[i][j], ep, k, o) : acc[i][j];
+      act_st(out, o, ep.a ? conv_epilogue<XT>(acc[i][j], ep, k, o) : acc[i][j]);
     }
   }
 }
@@ -445,8 +447,8 @@ bool pw_small_takes(int B, int C, int H, int W, int K, int R, int S, int stride,
   return HW <= 16 && (int64_t)B * HW <= 16384;
 }
 
-int launch_pw_small(const float* x, const float* w, float* out, int B, int C, int HW, int K, const ConvEpilogue& ep,
-                    cudaStream_t st) {
+int launch_pw_small(const void* x, const float* w, void* out, int B, int C, int HW, int K, const ConvEpilogue& ep,
+                    int dtype, cudaStream_t st) {
   PwGeom g;
   g.M = B * HW; g.C = C; g.K = K; g.HW = HW;
   g.div_hw = make_fastdiv((uint32_t)HW);
@@ -467,7 +469,10 @@ int launch_pw_small(const float* x, const float* w, float* out, int B, int C, in
   attr[0].val.clusterDim.x = 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = (unsigned)KS;
   cfg.attrs = attr;
   cfg.numAttrs = KS > 1 ? 1 : 0;
-  return (int)cudaLaunchKernelEx(&cfg, conv_pw_small_kernel, x, w, out, g, ep);
+  if (dtype == PO2_BF16)
+    return (int)cudaLaunchKernelEx(&cfg, conv_pw_small_kernel<__nv_bfloat16>, (const __nv_bfloat16*)x, w,
+                                   (__nv_bfloat16*)out, g, ep);
+  return (int)cudaLaunchKernelEx(&cfg, conv_pw_small_kernel<float>, (const float*)x, w, (float*)out, g, ep);
 }
 
 // ------------------------------------------------------------------------------------------------

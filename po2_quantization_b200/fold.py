@@ -39,7 +39,8 @@ def _affine(bn: nn.modules.batchnorm._BatchNorm):
 
 def _foldable(conv, bn, x) -> bool:
     return (isinstance(conv, QuantizedConv2d) and isinstance(bn, nn.modules.batchnorm._BatchNorm) and not bn.training
-            and bn.running_mean is not None and bn.running_var is not None and x.is_cuda and x.dtype == torch.float32
+            and bn.running_mean is not None and bn.running_var is not None and x.is_cuda
+            and x.dtype in (torch.float32, torch.bfloat16)
             and not (torch.is_grad_enabled() and x.requires_grad))
 
 

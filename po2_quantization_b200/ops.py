@@ -259,7 +259,8 @@ def ste_backward(grad_output: torch.Tensor, grad_input: torch.Tensor, accumulate
 def conv2d_out(x, w, scale, out, stride, pad, groups, compute, w_format=_lib.W_F32_PO2, bits=4, fsr=1,
                wshape=None):
     """Raw launcher: out = conv2d(x, w).  w: fp32 (K, C/groups, R, S) on the grid +-scale*2^q, or the
-    packed codes of such a tensor (w_format=W_CODES, wshape=(K, C/groups, R, S))."""
+    packed codes of such a tensor (w_format=W_CODES, wshape=(K, C/groups, R, S)).  x / out: fp32, or bf16 (inference
+    of a bf16 model; w is then the exact fp32 widening of its bf16 weight)."""
     global LAUNCHES
     lib = _lib.load()
     check_conv_shapes(x.shape, w.shape if wshape is None else wshape, groups, pad)
@@ -267,13 +268,15 @@ def conv2d_out(x, w, scale, out, stride, pad, groups, compute, w_format=_lib.W_F
     K, _, R, S = w.shape if wshape is None else wshape
     if w_format == _lib.W_CODES and w.numel() < _code_bytes(K * (C // groups) * R * S, bits):
         raise RuntimeError(f"po2 conv2d: {w.numel()} code bytes for a weight of shape {list(wshape)} at {bits} bits")
-    need = lib.po2_conv2d_workspace(B, C, H, W_, K, R, S, stride, pad, groups, compute)
+    dt = _DT[x.dtype]
+    need = lib.po2_conv2d_workspace_dt(B, C, H, W_, K, R, S, stride, pad, groups, compute, dt)
     ws = torch.empty(max(int(need), 16), dtype=torch.uint8, device=x.device)
     fp32_w_bytes = (K * (C // groups) * R * S * 4 + 255) // 256 * 256
     LAUNCHES += (2 if need > fp32_w_bytes else 1) + (1 if w_format == _lib.W_CODES and need <= fp32_w_bytes else 0)
-    _lib.check(lib.po2_conv2d_fwd(x.data_ptr(), w.data_ptr(), scale.data_ptr() if scale is not None else None,
-                                  out.data_ptr(), B, C, H, W_, K, R, S, stride, pad, groups, w_format,
-                                  bits, fsr, compute, ws.data_ptr(), ws.numel(), _stream_ptr(x.device)),
+    _lib.check(lib.po2_conv2d_fwd_ep_dt(x.data_ptr(), w.data_ptr(), scale.data_ptr() if scale is not None else None,
+                                        out.data_ptr(), B, C, H, W_, K, R, S, stride, pad, groups, w_format,
+                                        bits, fsr, compute, ws.data_ptr(), ws.numel(), None, None, None, 0, dt,
+                                        _stream_ptr(x.device)),
                "po2_conv2d_fwd")
 
 
@@ -297,6 +300,26 @@ def check_conv_shapes(xshape, wshape, groups: int, pad: int) -> None:
                            f"({R} x {S}). Kernel size can't be greater than actual input size")
 
 
+def conv_kernel_kind(xshape, wshape, stride: int, pad: int, groups: int, compute: int,
+                     dtype: torch.dtype = torch.float32) -> int:
+    """Which kernel conv2d runs for an input of shape xshape and dtype `dtype` (po2_conv2d_kernel_kind_dt, a planning
+    query without a launch); negative: the PO2_E_* code the launch would return -- PO2_E_UNSUPPORTED for a bf16 shape
+    that no bf16 kernel takes."""
+    B, C, H, W_ = xshape
+    K, _, R, S = wshape
+    return int(_lib.load().po2_conv2d_kernel_kind_dt(B, C, H, W_, K, R, S, stride, pad, groups, compute, _DT[dtype]))
+
+
+def _conv_weight(x, w, what):
+    """w as the conv kernels take it: fp32 activations need fp32 weights; bf16 activations (a bf16 model at inference)
+    take bf16 or fp32 weights, handed to the library as their exact fp32 widening"""
+    if x.dtype == torch.float32 and w.dtype == torch.float32:
+        return w
+    if x.dtype == torch.bfloat16 and w.dtype in (torch.bfloat16, torch.float32):
+        return w.float()
+    raise TypeError(f"{what}: fp32 NCHW activations with fp32 weights, or bf16 NCHW activations (inference) only")
+
+
 def _conv_out_shape(x, w, stride, pad):
     B, _, H, W_ = x.shape
     K, _, R, S = w.shape
@@ -308,14 +331,13 @@ def conv2d(x: torch.Tensor, w: torch.Tensor, scale: Optional[torch.Tensor], stri
            groups: int, compute: int) -> torch.Tensor:
     """conv2d(x, w) with w on the PO2 grid +-scale*2^q (scale=None: plain fp32 weights).
     compute 0: tcgen05 bf16 tensor cores (weights exact, activations rounded to bf16, fp32 accumulate)
-    where the shape allows; 1: fp32 FMA everywhere."""
+    where the shape allows; 1: fp32 FMA everywhere.  A bf16 x (inference only) gives a bf16 output."""
     _require_cuda(x, "po2::conv2d")
-    if x.dtype != torch.float32 or w.dtype != torch.float32:
-        raise TypeError("po2::conv2d: fp32 NCHW activations and fp32 weights only")
+    w = _conv_weight(x, w, "po2::conv2d")
     check_conv_shapes(x.shape, w.shape, groups, pad)
     x = _aligned16(x.contiguous())
     w = _aligned16(w.contiguous())
-    out = torch.empty(_conv_out_shape(x, w, stride, pad), dtype=torch.float32, device=x.device)
+    out = torch.empty(_conv_out_shape(x, w, stride, pad), dtype=x.dtype, device=x.device)
     with torch.cuda.device(x.device):
         conv2d_out(x, w, scale, out, stride, pad, groups, compute)
     return out
@@ -588,8 +610,15 @@ def _conv_backward(g, x, w, scale, stride, pad, groups, compute, need_x, need_w,
     return gx, gw
 
 
+def _no_bf16_backward(x, what):
+    if x.dtype == torch.bfloat16:
+        raise RuntimeError(f"{what}: a bf16 convolution runs at inference only -- there is no bf16 backward; run it under "
+                           "torch.no_grad() / torch.inference_mode(), or train in fp32")
+
+
 def _conv2d_setup(ctx, inputs, output):
     x, w, scale, stride, pad, groups, compute = inputs
+    _no_bf16_backward(x, "po2::conv2d")
     ctx.save_for_backward(x, w, scale) if scale is not None else ctx.save_for_backward(x, w)
     ctx.has_scale = scale is not None
     ctx.cfg = (stride, pad, groups, compute)
@@ -790,49 +819,53 @@ lin_qconv2d.register_autograd(_lin_qconv2d_bwd, setup_context=_lin_qconv2d_setup
 # static weights: pack once, then one launch per forward
 # ------------------------------------------------------------------------------------------------
 def conv2d_pack(w: torch.Tensor, scale: Optional[torch.Tensor], xshape, stride: int, pad: int, groups: int,
-                compute: int = 0):
-    """Packed bf16 tensor-core operand for conv2d(x of shape xshape, w), or None if that shape does not
-    run on the tensor-core kernel."""
+                compute: int = 0, xdtype: torch.dtype = torch.float32):
+    """Packed bf16 tensor-core operand for conv2d(x of shape xshape and dtype xdtype, w), or None if that shape does not
+    run on the tensor-core kernel.  w: fp32, or (bf16 x) the model's bf16 weight, packed from its exact fp32 widening."""
     global LAUNCHES
     lib = _lib.load()
     check_conv_shapes(xshape, w.shape, groups, pad)
     B, C, H, W_ = xshape
     K, _, R, S = w.shape
-    nbytes = lib.po2_conv2d_pack_bytes(B, C, H, W_, K, R, S, stride, pad, groups, compute)
+    dt = _DT[xdtype]
+    nbytes = lib.po2_conv2d_pack_bytes_dt(B, C, H, W_, K, R, S, stride, pad, groups, compute, dt)
     if nbytes == 0:
         return None
+    w = w.float().contiguous()
     packed = torch.empty(int(nbytes), dtype=torch.uint8, device=w.device)
     with torch.cuda.device(w.device):
         LAUNCHES += 1
-        _lib.check(lib.po2_conv2d_pack(w.data_ptr(), scale.data_ptr() if scale is not None else None, packed.data_ptr(),
-                                       packed.numel(), B, C, H, W_, K, R, S, stride, pad, groups, _lib.W_F32_PO2, 4, 1,
-                                       compute, _stream_ptr(w.device)), "po2_conv2d_pack")
+        _lib.check(lib.po2_conv2d_pack_dt(w.data_ptr(), scale.data_ptr() if scale is not None else None, packed.data_ptr(),
+                                          packed.numel(), B, C, H, W_, K, R, S, stride, pad, groups, _lib.W_F32_PO2, 4, 1,
+                                          compute, dt, _stream_ptr(w.device)), "po2_conv2d_pack")
     return packed
 
 
 @torch.library.custom_op("po2::conv2d_packed", mutates_args=(), device_types="cuda")
 def conv2d_packed(x: torch.Tensor, packed: torch.Tensor, scale: Optional[torch.Tensor], K: int, R: int, S: int,
                   stride: int, pad: int, groups: int, compute: int) -> torch.Tensor:
-    """conv2d from a pre-packed weight operand (inference with static weights): one kernel launch."""
+    """conv2d from a pre-packed weight operand (inference with static weights): one kernel launch.  x: fp32, or bf16
+    (the operand packed for a bf16 x); the output has x's dtype."""
     global LAUNCHES
     _require_cuda(x, "po2::conv2d_packed")
     if x.dim() != 4:
         raise RuntimeError(f"Expected 4D (batched) input to conv2d, but got input of size: {list(x.shape)}")
     x = _aligned16(x.contiguous())
     B, C, H, W_ = x.shape
+    dt = _act_dt(x, "po2::conv2d_packed")
     # the packed operand was laid out for ONE (input shape, weight shape): re-validate it against this input
-    need = int(_lib.load().po2_conv2d_pack_bytes(B, C, H, W_, K, R, S, stride, pad, groups, compute))
+    need = int(_lib.load().po2_conv2d_pack_bytes_dt(B, C, H, W_, K, R, S, stride, pad, groups, compute, dt))
     if need == 0 or packed.numel() != need:
         raise RuntimeError(f"po2::conv2d_packed: the packed operand ({packed.numel()} bytes) was not built for input "
                            f"{list(x.shape)} / weight [{K}, {C // max(groups, 1)}, {R}, {S}] (needs {need} bytes)")
     out = torch.empty((B, K, (H + 2 * pad - R) // stride + 1, (W_ + 2 * pad - S) // stride + 1),
-                      dtype=torch.float32, device=x.device)
+                      dtype=x.dtype, device=x.device)
     with torch.cuda.device(x.device):
         LAUNCHES += 1
-        _lib.check(_lib.load().po2_conv2d_fwd_packed(x.data_ptr(), packed.data_ptr(),
-                                                     scale.data_ptr() if scale is not None else None, out.data_ptr(),
-                                                     B, C, H, W_, K, R, S, stride, pad, groups, compute,
-                                                     _stream_ptr(x.device)),
+        _lib.check(_lib.load().po2_conv2d_fwd_packed_ep_dt(x.data_ptr(), packed.data_ptr(),
+                                                           scale.data_ptr() if scale is not None else None, out.data_ptr(),
+                                                           B, C, H, W_, K, R, S, stride, pad, groups, compute,
+                                                           None, None, None, 0, dt, _stream_ptr(x.device)),
                    "po2_conv2d_fwd_packed")
     return out
 
@@ -846,10 +879,18 @@ def _(x, packed, scale, K, R, S, stride, pad, groups, compute):
 # ------------------------------------------------------------------------------------------------
 # inference with eval-mode BatchNorm (+ residual add) (+ activation) folded into the conv's epilogue
 # ------------------------------------------------------------------------------------------------
-def _ep_check(out_shape, K, ep_a, ep_b, residual):
+def _act_dt(x, what):
+    """the C ABI dtype of a conv's activations: fp32, or bf16 (inference)"""
+    if x.dtype not in (torch.float32, torch.bfloat16):
+        raise TypeError(f"{what}: fp32 or bf16 NCHW activations only, got {x.dtype}")
+    return _DT[x.dtype]
+
+
+def _ep_check(out, K, ep_a, ep_b, residual):
+    out_shape = out.shape
     if ep_a.numel() != K or ep_b.numel() != K or ep_a.dtype != torch.float32 or ep_b.dtype != torch.float32:
         raise RuntimeError(f"po2 conv epilogue: scale/shift must be fp32 vectors of {K} out channels")
-    if residual is not None and (tuple(residual.shape) != tuple(out_shape) or residual.dtype != torch.float32):
+    if residual is not None and (tuple(residual.shape) != tuple(out_shape) or residual.dtype != out.dtype):
         raise RuntimeError(f"po2 conv epilogue: residual {list(residual.shape)} does not match the output {list(out_shape)}")
 
 
@@ -862,21 +903,22 @@ def conv2d_packed_ep(x: torch.Tensor, packed: torch.Tensor, scale: Optional[torc
     _require_cuda(x, "po2::conv2d_packed_ep")
     x = _aligned16(x.contiguous())
     B, C, H, W_ = x.shape
-    need = int(_lib.load().po2_conv2d_pack_bytes(B, C, H, W_, K, R, S, stride, pad, groups, compute))
+    dt = _act_dt(x, "po2::conv2d_packed_ep")
+    need = int(_lib.load().po2_conv2d_pack_bytes_dt(B, C, H, W_, K, R, S, stride, pad, groups, compute, dt))
     if need == 0 or packed.numel() != need:
         raise RuntimeError(f"po2::conv2d_packed_ep: the packed operand ({packed.numel()} bytes) was not built for input "
                            f"{list(x.shape)} / weight [{K}, {C // max(groups, 1)}, {R}, {S}] (needs {need} bytes)")
     out = torch.empty((B, K, (H + 2 * pad - R) // stride + 1, (W_ + 2 * pad - S) // stride + 1),
-                      dtype=torch.float32, device=x.device)
-    _ep_check(out.shape, K, ep_a, ep_b, residual)
+                      dtype=x.dtype, device=x.device)
+    _ep_check(out, K, ep_a, ep_b, residual)
     if residual is not None:
         residual = residual.contiguous()
     with torch.cuda.device(x.device):
         LAUNCHES += 1
-        _lib.check(_lib.load().po2_conv2d_fwd_packed_ep(
+        _lib.check(_lib.load().po2_conv2d_fwd_packed_ep_dt(
             x.data_ptr(), packed.data_ptr(), scale.data_ptr() if scale is not None else None, out.data_ptr(),
             B, C, H, W_, K, R, S, stride, pad, groups, compute, ep_a.data_ptr(), ep_b.data_ptr(),
-            residual.data_ptr() if residual is not None else None, int(act), _stream_ptr(x.device)),
+            residual.data_ptr() if residual is not None else None, int(act), dt, _stream_ptr(x.device)),
             "po2_conv2d_fwd_packed_ep")
     return out
 
@@ -892,31 +934,31 @@ def conv2d_ep(x: torch.Tensor, w: torch.Tensor, scale: Optional[torch.Tensor], s
               compute: int, ep_a: torch.Tensor, ep_b: torch.Tensor, residual: Optional[torch.Tensor],
               act: int) -> torch.Tensor:
     """act(conv2d(x, w) * ep_a[k] + ep_b[k] + residual) for any layer kind (depthwise, direct, tensor-core with an
-    inline pack): inference only."""
+    inline pack): inference only.  A bf16 x (with a bf16 residual) gives a bf16 output."""
     global LAUNCHES
     _require_cuda(x, "po2::conv2d_ep")
-    if x.dtype != torch.float32 or w.dtype != torch.float32:
-        raise TypeError("po2::conv2d_ep: fp32 NCHW activations and fp32 weights only")
+    w = _conv_weight(x, w, "po2::conv2d_ep")
     check_conv_shapes(x.shape, w.shape, groups, pad)
     x = _aligned16(x.contiguous())
     w = _aligned16(w.contiguous())
     lib = _lib.load()
     B, C, H, W_ = x.shape
     K, _, R, S = w.shape
-    out = torch.empty(_conv_out_shape(x, w, stride, pad), dtype=torch.float32, device=x.device)
-    _ep_check(out.shape, K, ep_a, ep_b, residual)
+    dt = _DT[x.dtype]
+    out = torch.empty(_conv_out_shape(x, w, stride, pad), dtype=x.dtype, device=x.device)
+    _ep_check(out, K, ep_a, ep_b, residual)
     if residual is not None:
         residual = residual.contiguous()
     with torch.cuda.device(x.device):
-        need = lib.po2_conv2d_workspace(B, C, H, W_, K, R, S, stride, pad, groups, compute)
+        need = lib.po2_conv2d_workspace_dt(B, C, H, W_, K, R, S, stride, pad, groups, compute, dt)
         ws = torch.empty(max(int(need), 16), dtype=torch.uint8, device=x.device)
         fp32_w_bytes = (K * (C // groups) * R * S * 4 + 255) // 256 * 256
         LAUNCHES += 2 if need > fp32_w_bytes else 1
-        _lib.check(lib.po2_conv2d_fwd_ep(x.data_ptr(), w.data_ptr(), scale.data_ptr() if scale is not None else None,
-                                         out.data_ptr(), B, C, H, W_, K, R, S, stride, pad, groups, _lib.W_F32_PO2, 4, 1,
-                                         compute, ws.data_ptr(), ws.numel(), ep_a.data_ptr(), ep_b.data_ptr(),
-                                         residual.data_ptr() if residual is not None else None, int(act),
-                                         _stream_ptr(x.device)), "po2_conv2d_fwd_ep")
+        _lib.check(lib.po2_conv2d_fwd_ep_dt(x.data_ptr(), w.data_ptr(), scale.data_ptr() if scale is not None else None,
+                                            out.data_ptr(), B, C, H, W_, K, R, S, stride, pad, groups, _lib.W_F32_PO2, 4,
+                                            1, compute, ws.data_ptr(), ws.numel(), ep_a.data_ptr(), ep_b.data_ptr(),
+                                            residual.data_ptr() if residual is not None else None, int(act), dt,
+                                            _stream_ptr(x.device)), "po2_conv2d_fwd_ep")
     return out
 
 

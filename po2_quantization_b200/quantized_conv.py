@@ -38,13 +38,20 @@ class QuantizedConv2d(nn.Conv2d):
     # ---- which inputs the sm_100a conv kernels take.  Anything else goes to nn.Conv2d's own path
     # (cuDNN) -- never silently: _why_not() names the reason and forward() reports it once per reason
     # (ops.note_library_path; an error under PO2_STRICT=1).  Every QuantizedConv2d the reference's model
-    # files construct (bias=False, dilation 1, square stride/padding, fp32) is taken.
+    # files construct (bias=False, dilation 1, square stride/padding, fp32) is taken, and so is a bf16 model's layer
+    # at inference (no gradient, mode tc / tf32) on the kernels that have a bf16 form.
+    def _bf16_inference(self, input) -> bool:
+        return (input.dtype == torch.bfloat16 and self.weight.dtype == torch.bfloat16
+                and ops.get_conv_mode() in ("tc", "tf32")
+                and not (torch.is_grad_enabled() and (input.requires_grad or self.weight.requires_grad)))
+
     def _why_not(self, input):
         if ops.get_conv_mode() == "cudnn":
             return None                                       # the caller asked for cuDNN: not a fallback
         if not input.is_cuda:
             return "CPU input"
-        if input.dtype != torch.float32 or self.weight.dtype != torch.float32:
+        bf16 = self._bf16_inference(input)
+        if (input.dtype != torch.float32 or self.weight.dtype != torch.float32) and not bf16:
             return f"dtype {input.dtype}/{self.weight.dtype} (fp32 NCHW only)"
         if input.dim() != 4:
             return f"{input.dim()}-D input (batched NCHW only)"
@@ -56,6 +63,9 @@ class QuantizedConv2d(nn.Conv2d):
             return f"padding {self.padding!r} / padding_mode {self.padding_mode!r}"
         if self.stride[0] != self.stride[1] or self.padding[0] != self.padding[1]:
             return f"non-square stride {self.stride} / padding {self.padding}"
+        if bf16 and ops.conv_kernel_kind(input.shape, self.weight.shape, self.stride[0], self.padding[0], self.groups,
+                                         ops.COMPUTE[ops.get_conv_mode()], input.dtype) < 0:
+            return f"bf16 layer {list(self.weight.shape)} groups {self.groups} (no bf16 kernel for this shape)"
         return ""
 
     def _po2_conv_ok(self, input) -> bool:
@@ -67,6 +77,8 @@ class QuantizedConv2d(nn.Conv2d):
         why = self._why_not(input)
         if why != "":
             return why
+        if input.dtype != torch.float32:
+            return f"dtype {input.dtype}/{self.weight.dtype} (fp32 NCHW only)"
         mode = ops.get_conv_mode()
         if not 2 <= bits <= ops.LIN_EXACT_BITS[mode]:
             return f"lin weights of {bits} bits are not exact as {mode} operands (at most {ops.LIN_EXACT_BITS[mode]} bits)"
@@ -128,6 +140,48 @@ class QuantizedConv2d(nn.Conv2d):
             self.__dict__["_po2_pack_cache"] = cache
         return cache[1]
 
+    def _bf16_forward(self, input, ep=None):
+        """forward of a bf16 PO2 / PO2+ layer at inference (PTQ weights, or a QAT layer in eval), ep = (ep_a, ep_b,
+        residual, act) for the folded form.  Cached in _po2_pack_cache per (weight version, input shape, device, mode,
+        dtype): the packed operand, or the fp32 widening of the bf16 weight for the depthwise / small-pointwise kernels.
+        A QAT layer's weight is quantized in bf16 first (quantize_full), as the quantizer itself does on a bf16 model."""
+        mode = ops.get_conv_mode()
+        compute, w = ops.COMPUTE[mode], self.weight
+        stride, pad, groups = self.stride[0], self.padding[0], self.groups
+        fam = _quantizers.quantizer_family(self.quantize_fn) if self.quantize_fn is not None else None
+        qat = (int(self.bits), fam[1]) if fam is not None else ()
+        key = (w._version, tuple(input.shape), input.device, mode, input.dtype) + qat
+        cache = self.__dict__.get("_po2_pack_cache")
+        if cache is None or cache[0] != key:
+            if qat:
+                y, _codes, scale, _zc, _sse = ops.quantize_full(w.detach(), int(self.bits), 1, bool(fam[1]))
+            else:
+                y, scale = w.detach(), self._po2_ptq[1]
+            packed = ops.conv2d_pack(y, scale, tuple(input.shape), stride, pad, groups, compute, input.dtype)
+            cache = (key, packed, y.float() if packed is None else None, scale)
+            self.__dict__["_po2_pack_cache"] = cache
+        _, packed, wf, scale = cache
+        K, _, R, S = w.shape
+        if ep is None:
+            if packed is not None:
+                return ops.conv2d_packed(input, packed, scale, K, R, S, stride, pad, groups, compute)
+            return ops.conv2d(input, wf, scale, stride, pad, groups, compute)
+        ep_a, ep_b, residual, act = ep
+        if packed is not None:
+            return ops.conv2d_packed_ep(input, packed, scale, K, R, S, stride, pad, groups, compute, ep_a, ep_b, residual,
+                                        int(act))
+        return ops.conv2d_ep(input, wf, scale, stride, pad, groups, compute, ep_a, ep_b, residual, int(act))
+
+    def _bf16_po2_layer(self, input) -> bool:
+        """a PO2 / PO2+ layer (QAT quantizer or current PTQ tag) whose bf16 call the kernels take"""
+        if self.quantize_fn is not None:
+            fam = _quantizers.quantizer_family(self.quantize_fn)
+            po2 = fam is not None and fam[0] == "po2"
+        else:
+            tag = getattr(self, "_po2_ptq", None)
+            po2 = tag is not None and tag[0] == self.weight._version
+        return po2 and input.dtype == torch.bfloat16 and self._why_not(input) == ""
+
     def _library_conv(self, input, weight, why):
         if why:
             ops.note_library_path("qconv:" + why, f"QuantizedConv2d runs nn.Conv2d's own convolution (cuDNN) for this "
@@ -142,6 +196,8 @@ class QuantizedConv2d(nn.Conv2d):
 
     def forward(self, input):
         # models/quantized_conv.py:32-38: quantize the weight on every forward (QAT), then conv
+        if input.dtype == torch.bfloat16 and input.is_cuda and self._bf16_po2_layer(input):
+            return self._bf16_forward(input)
         if self.quantize_fn is not None:
             fam = _quantizers.quantizer_family(self.quantize_fn)
             if fam is not None and fam[0] == "lin":
@@ -208,6 +264,8 @@ class QuantizedConv2d(nn.Conv2d):
         mode = ops.get_conv_mode()
         if mode == "cudnn" or self._why_not(input) != "":
             return None
+        if input.dtype == torch.bfloat16:
+            return self._bf16_forward(input, (ep_a, ep_b, residual, act)) if self._bf16_po2_layer(input) else None
         compute = ops.COMPUTE[mode]
         K, _, R, S = self.weight.shape
         if self.quantize_fn is not None:
