@@ -238,11 +238,17 @@ int po2_conv2d_dgrad(const void* g, const void* w, const float* scale, void* gx,
 /* Backward of the layer kinds the tensor-core kernels do not take directly (csrc/po2_conv_bwd.cu):
  * po2_dilate2: g (planes, P, Q) -> g_up (planes, 2P, 2Q) with g_up[2p][2q] = g[p][q], zero elsewhere -- both
  * gradients of a STRIDE-2 dense conv are the stride-1 gradients (po2_conv2d_dgrad / po2_conv2d_wgrad) taken with
- * g_up (models/resnet.py:25-50, the four stride-2 layers of ResNet-20/56).
+ * g_up (models/resnet.py:25-50, the four stride-2 layers of ResNet-20/56).  Q must be even, g 8-byte and g_up
+ * 16-byte aligned (PO2_E_UNSUPPORTED otherwise).
+ * po2_dilate2_into: the same for any size, g (planes, P, Q) -> g_up (planes, H, W) with P == (H - 1) / 2 + 1 and
+ * Q == (W - 1) / 2 + 1 (the output of a 3x3 pad 1 or 1x1 pad 0 stride-2 conv on H x W, odd H, W or Q included),
+ * any 4-byte alignment; writes every element of g_up.  PO2_E_SHAPE for non-positive or mismatched sizes,
+ * PO2_E_SIZE from 2^31 elements of g_up.
  * Depthwise 3x3 pad 1 (models/mobilenet.py:64-74): the data gradient and the deterministic weight gradient;
- * `g` is the output gradient at the INPUT resolution (stride 2: zero-inserted with po2_dilate2); the
+ * `g` is the output gradient at the INPUT resolution (stride 2: zero-inserted with po2_dilate2 / _into); the
  * workspace's first 16 KB (tickets) must be zero before the first call and are left zero. */
 int po2_dilate2(const void* g, void* g_up, int planes, int P, int Q, void* stream);
+int po2_dilate2_into(const void* g, void* g_up, int planes, int P, int Q, int H, int W, void* stream);
 int po2_conv2d_depthwise_dgrad(const void* g, const void* w, void* gx, int B, int C, int H, int W, void* stream);
 size_t po2_conv2d_depthwise_wgrad_workspace(int C);
 int po2_conv2d_depthwise_wgrad(const void* g, const void* x, void* gw, int B, int C, int H, int W, void* workspace,

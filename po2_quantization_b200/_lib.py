@@ -55,6 +55,7 @@ SIGNATURES = {
     "po2_conv2d_dgrad_workspace": (_sz, [_i] * 9),
     "po2_conv2d_dgrad": (_i, [_vp, _vp, _vp, _vp] + [_i] * 14 + [_vp, _sz, _vp]),
     "po2_dilate2": (_i, [_vp, _vp, _i, _i, _i, _vp]),
+    "po2_dilate2_into": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "po2_conv2d_stem_wgrad_workspace": (_sz, [_i] * 10),
     "po2_conv2d_stem_wgrad": (_i, [_vp, _vp, _vp] + [_i] * 10 + [_vp, _sz, _vp]),
     "po2_sgd_step": (_i, [_vp, _vp, _vp, _vp, _i, _c.c_float, _c.c_float, _c.c_float, _i, _vp]),

@@ -5,7 +5,9 @@
 //   * stride 2, dense: both gradients of conv(x, W, stride 2) equal the gradients of the STRIDE-1 conv whose
 //     output gradient is the zero-inserted one, g_up[2p][2q] = g[p][q]:
 //         gx = conv_transpose(g, W, 2) = dgrad_stride1(g_up, W),   gw = wgrad_stride1(g_up, x)
-//     so one small kernel (dilate2_kernel) puts these layers on the TMA-fed tcgen05 kernels (K3T / K5T).
+//     so one small kernel (dilate2_kernel; dilate2_into_kernel for odd sizes) puts these layers on the stride-1
+//     kernels (K3T / K5T where they take the shape).  For 3x3 pad 1 and 1x1 pad 0 this holds for any H x W: output
+//     row p reads input rows 2p - 1 .. 2p + 1, as row 2p of the stride-1 conv does, and 2(P - 1) <= H - 1.
 //   * depthwise 3x3 pad 1 (groups == C == K): data gradient = the depthwise forward kernel's arithmetic with
 //     the filter rotated by 180 degrees (on g, or on g_up for stride 2); weight gradient = nine per-channel
 //     inner products over the batch, a two-stage fixed-order reduction (deterministic).
@@ -27,6 +29,17 @@ __global__ void __launch_bounds__(256) dilate2_kernel(const float* __restrict__ 
     float4* o = reinterpret_cast<float4*>(up + (size_t)row * 4 * Q) + c2;        // output row 2*row has 2Q floats
     o[0] = make_float4(v.x, 0.f, v.y, 0.f);
     o[Q2] = make_float4(0.f, 0.f, 0.f, 0.f);                                      // output row 2*row + 1
+  }
+}
+
+// The same zero-insertion for any H x W with P = (H - 1) / 2 + 1, Q = (W - 1) / 2 + 1 (odd H or W, odd Q), at any
+// 4-byte alignment: g (planes, P, Q) -> g_up (planes, H, W).  One thread = one output element, scalar accesses.
+__global__ void __launch_bounds__(256) dilate2_into_kernel(const float* __restrict__ g, float* __restrict__ up, int P,
+                                                           int Q, int H, int W, int total) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+    const int row = i / W, w = i - row * W;                                       // row = plane * H + h
+    const int plane = row / H, h = row - plane * H;
+    up[i] = ((h | w) & 1) ? 0.f : __ldg(g + ((size_t)plane * P + (h >> 1)) * Q + (w >> 1));
   }
 }
 
@@ -259,7 +272,17 @@ int po2_dilate2(const void* g, void* g_up, int planes, int P, int Q, void* strea
   return (int)cudaGetLastError();
 }
 
-// g: (B, C, H, W) -- the output gradient at the INPUT resolution (stride 2: zero-inserted with po2_dilate2)
+int po2_dilate2_into(const void* g, void* g_up, int planes, int P, int Q, int H, int W, void* stream) {
+  if (!g || !g_up) return PO2_E_NULL;
+  if (planes <= 0 || H <= 0 || W <= 0 || P != (H - 1) / 2 + 1 || Q != (W - 1) / 2 + 1) return PO2_E_SHAPE;
+  if ((int64_t)planes * H * W >= (1ll << 31)) return PO2_E_SIZE;
+  const int total = planes * H * W;
+  const int blocks = (total + 255) / 256 < device_sm_count() * 16 ? (total + 255) / 256 : device_sm_count() * 16;
+  dilate2_into_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>((const float*)g, (float*)g_up, P, Q, H, W, total);
+  return (int)cudaGetLastError();
+}
+
+// g: (B, C, H, W) -- the output gradient at the INPUT resolution (stride 2: zero-inserted with po2_dilate2 / _into)
 int po2_conv2d_depthwise_dgrad(const void* g, const void* w, void* gx, int B, int C, int H, int W, void* stream) {
   if (!g || !w || !gx) return PO2_E_NULL;
   if (B <= 0 || C <= 0 || H <= 0 || W <= 0) return PO2_E_SHAPE;

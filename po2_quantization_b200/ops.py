@@ -447,6 +447,16 @@ def dilate2_out(g, g_up) -> None:
     _lib.check(_lib.load().po2_dilate2(g.data_ptr(), g_up.data_ptr(), B * K, P, Q, _stream_ptr(g.device)), "po2_dilate2")
 
 
+def dilate2_into_out(g, g_up) -> None:
+    """dilate2_out for any H x W of g_up with g's P x Q == ((H - 1) // 2 + 1, (W - 1) // 2 + 1): odd H or W, odd Q"""
+    global LAUNCHES
+    B, K, P, Q = g.shape
+    H, W_ = g_up.shape[2:]
+    LAUNCHES += 1
+    _lib.check(_lib.load().po2_dilate2_into(g.data_ptr(), g_up.data_ptr(), B * K, P, Q, H, W_, _stream_ptr(g.device)),
+               "po2_dilate2_into")
+
+
 _dw_workspaces = {}
 _wgrad_tickets = {}
 
@@ -561,13 +571,17 @@ def _conv_backward(g, x, w, scale, stride, pad, groups, compute, need_x, need_w,
     ours = compute != 1 and groups == 1 and fp32 and stride in (1, 2)
     depthwise = (fp32 and _dgrad_mode == "tc" and groups == C == K and R == 3 and S == 3 and pad == 1 and stride in (1, 2)
                  and C <= 4096)
-    s2_ok = stride == 2 and H % 2 == 0 and W_ % 2 == 0 and ((R == 3 and pad == 1) or (R == 1 and pad == 0)) and \
-        g.shape[2] * 2 == H and g.shape[3] * 2 == W_ and g.shape[3] % 2 == 0
+    # 3x3 pad 1 / 1x1 pad 0 at stride 2 is the stride-1 problem on the zero-inserted output gradient, at any H x W
+    s2_ok = stride == 2 and ((R == 3 and pad == 1) or (R == 1 and pad == 0)) and \
+        tuple(g.shape[2:]) == ((H - 1) // 2 + 1, (W_ - 1) // 2 + 1)
     with torch.cuda.device(x.device):
         g_s1 = g
         if stride == 2 and (ours or depthwise) and s2_ok and (need_x or need_w):
             g_s1 = torch.empty(B, K, H, W_, dtype=torch.float32, device=g.device)
-            dilate2_out(g, g_s1)
+            if H % 2 == 0 and W_ % 2 == 0 and g.shape[3] % 2 == 0:
+                dilate2_out(g, g_s1)
+            else:
+                dilate2_into_out(g, g_s1)
         elif stride == 2:
             ours = depthwise = False
         if depthwise:
