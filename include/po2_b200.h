@@ -284,10 +284,16 @@ int po2_conv2d_wgrad(const void* g, const void* x, void* gw, int B, int C, int H
 /* lin / lin+ quantizers (SURVEY.md section 8f "next" #1) -- utils/quantizers.py:59-96 (plus = 0), :99-136
  * (plus = 1): per-input-channel uniform quantizer with a power-of-two step refined by num_iters rounds.
  * w, y: fp32 (K, C, R*S) contiguous; one launch.  PO2_E_UNSUPPORTED when K*R*S exceeds
- * po2_lin_max_channel_elems() (the caller keeps the op-by-op form). */
+ * po2_lin_max_channel_elems() (the caller keeps the op-by-op form).
+ * po2_lin_quantize_dt: the same for w, y of storage `dtype`.  PO2_F32 is exactly po2_lin_quantize; PO2_BF16 (a bf16
+ * model's weights) evaluates every op of the reference in fp32 and rounds its result to bf16, as torch does for bf16
+ * tensors, and writes a bf16 y.  PO2_E_DTYPE for any other dtype; otherwise the errors of po2_lin_quantize, all
+ * before any launch. */
 int po2_lin_max_channel_elems(void);
 int po2_lin_quantize(const void* w, void* y, int K, int C, int RS, int bits, int num_iters, int plus, int flavor,
                      void* stream);
+int po2_lin_quantize_dt(const void* w, void* y, int K, int C, int RS, int bits, int num_iters, int plus, int flavor,
+                        int dtype, void* stream);
 
 /* lin / lin+ weights on the tensor-core conv: after num_iters >= 1 rounds every weight is n * 2^k (one power-of-two
  * step per input channel, |n| <= 2^(bits-1) - 1), which is exact as a bf16 operand for bits <= 9 (compute 0) and as

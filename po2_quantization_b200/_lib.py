@@ -69,6 +69,7 @@ SIGNATURES = {
     "po2_conv2d_wgrad": (_i, [_vp, _vp, _vp] + [_i] * 11 + [_vp, _sz, _vp]),
     "po2_lin_max_channel_elems": (_i, []),
     "po2_lin_quantize": (_i, [_vp, _vp] + [_i] * 7 + [_vp]),
+    "po2_lin_quantize_dt": (_i, [_vp, _vp] + [_i] * 8 + [_vp]),
     "po2_lin_quantize_pack": (_i, [_vp, _vp, _vp, _sz, _vp, _sz] + [_i] * 15 + [_vp]),
     "po2_lin_multi_desc_bytes": (_sz, []),
     "po2_lin_multi_desc_fill": (_i, [_vp, _i, _vp, _vp, _vp, _sz, _vp, _sz] + [_i] * 15),

@@ -17,6 +17,7 @@ namespace po2 {
 template <int DT> struct Tr;
 
 template <> struct Tr<PO2_F32> {
+  using T = float;                  // the storage type
   static constexpr int EB = 4;      // bytes per element
   static constexpr int MB = 23;     // mantissa bits (binade index = magnitude >> MB)
   static constexpr int EPV = 4;     // elements per 16-byte vector
@@ -26,6 +27,7 @@ template <> struct Tr<PO2_F32> {
   static __device__ __forceinline__ uint32_t pat(float f) { return __float_as_uint(f); }
 };
 template <> struct Tr<PO2_BF16> {
+  using T = __nv_bfloat16;
   static constexpr int EB = 2, MB = 7, EPV = 8, NBIN = 256;
   static constexpr uint32_t MAG = 0x7FFFu, SGN = 0x8000u, QNAN = 0x7FC0u, INF = 0x7F80u;
   static __device__ __forceinline__ float val(uint32_t p) { return __uint_as_float(p << 16); }
@@ -34,6 +36,7 @@ template <> struct Tr<PO2_BF16> {
   }
 };
 template <> struct Tr<PO2_F16> {
+  using T = __half;
   static constexpr int EB = 2, MB = 10, EPV = 8, NBIN = 32;
   static constexpr uint32_t MAG = 0x7FFFu, SGN = 0x8000u, QNAN = 0x7E00u, INF = 0x7C00u;
   static __device__ __forceinline__ float val(uint32_t p) {

@@ -28,7 +28,8 @@ __device__ __forceinline__ double lin_warp_sum(double v) {
 
 __device__ __forceinline__ float lin_clamp(float t, float lim) { return t != t ? t : fminf(fmaxf(t, -lim), lim); }
 
-// 2 ** round(log2(step)) as torch evaluates it in fp32
+// 2 ** round(log2(step)) as torch evaluates it in the storage type DT (fp32 or bf16)
+template <int DT>
 __device__ __forceinline__ float lin_pow2_round_log2(float step, int flavor) {
   const uint32_t pat = __float_as_uint(step);
   if (step > 0.0f && step <= 1.0f) {
@@ -36,19 +37,22 @@ __device__ __forceinline__ float lin_pow2_round_log2(float step, int flavor) {
     int e = (int)(pat >> 23) - 127;
     if ((pat >> 23) == 0) e = -127 - (__clz(pat) - 9);           // subnormal: position of the leading bit
     int k = e;
-    if (e + 1 <= PO2_KMAX && e + 1 >= PO2_KMIN && pat >= PO2_BOUNDS[flavor][0][0][e + 1 - PO2_KMIN]) k = e + 1;
+    if (e + 1 <= PO2_KMAX && e + 1 >= PO2_KMIN && pat >= PO2_BOUNDS[flavor][DT][0][e + 1 - PO2_KMIN]) k = e + 1;
     if (k < PO2_KMIN) k = PO2_KMIN;                               // round(log2) of the smallest subnormals
     return exp2_int(k);
   }
   // step > 1, zero, negative, inf, NaN: the float ops themselves (NaN / inf propagate as in torch)
-  return exp2f(rintf(log2f(step)));
+  return exp2f(rintf(round_storage<DT>(log2f(step))));
 }
 
 // input channel c of w (K, C, RS) -> y; with pk.Bp set, also the channel's entries of the conv's packed operand(s)
 // (the operand value is y itself: n * 2^k with |n| <= 2^(bits-1) - 1 -- exact in bf16 for bits <= 9, in tf32 for
-// bits <= 12 -- once at least one refinement round has made the step a power of two)
-__device__ __forceinline__ void lin_channel(const float* __restrict__ w, float* __restrict__ y, int K, int C, int RS,
-                                            int bits, int iters, int plus, int flavor, int c, const PackArgs& pk) {
+// bits <= 12 -- once at least one refinement round has made the step a power of two).  w, y: float (PO2_F32) or
+// __nv_bfloat16 (PO2_BF16)
+template <int DT>
+__device__ __forceinline__ void lin_channel(const typename Tr<DT>::T* __restrict__ w,
+                                            typename Tr<DT>::T* __restrict__ y, int K, int C, int RS, int bits,
+                                            int iters, int plus, int flavor, int c, const PackArgs& pk) {
   extern __shared__ float sw[];
   __shared__ double red[LIN_THREADS / 32][2];
   __shared__ float bc[2];
@@ -59,7 +63,9 @@ __device__ __forceinline__ void lin_channel(const float* __restrict__ w, float* 
   bool nan = false;
   for (int i = tid; i < n; i += LIN_THREADS) {
     const int k = i / RS, j = i - k * RS;
-    const float v = __ldg(w + ((size_t)k * C + c) * RS + j);
+    float v;
+    if constexpr (DT == PO2_F32) v = __ldg(w + ((size_t)k * C + c) * RS + j);
+    else v = __bfloat162float(__ldg(w + ((size_t)k * C + c) * RS + j));     // exact widening
     sw[i] = v;
     nan |= (v != v);
     hi = fmaxf(hi, v);
@@ -82,22 +88,23 @@ __device__ __forceinline__ void lin_channel(const float* __restrict__ w, float* 
       if (l != l) anynan = true; else L = fminf(L, (float)l);
     }
     const float levels = (float)((1 << bits) - 1);
-    bc[0] = anynan ? NAN : __fdiv_rn(H - L, levels);             // utils/quantizers.py: (max - min) / (2**bits - 1)
+    bc[0] = anynan ? NAN : round_storage<DT>(__fdiv_rn(round_storage<DT>(H - L), levels));  // (max - min) / (2**bits - 1)
   }
   __syncthreads();
   float step = bc[0];
   const float lim = (float)((1 << (bits - 1)) - 1);
   const float c89 = __fsqrt_rn(8.0f / 9.0f);                       // torch.sqrt(torch.tensor(8/9))
   // q = uniform_quantize(w, step) / step = (step * clamp(round(w / step), -lim, lim)) / step
-  // (torch.clamp propagates NaN, fminf / fmaxf would swallow it)
-#define LIN_Q(v, s) __fdiv_rn(__fmul_rn((s), lin_clamp(rintf(__fdiv_rn((v), (s))), lim)), (s))
+  // (torch.clamp propagates NaN, fminf / fmaxf would swallow it); in bf16 each op's result is rounded to bf16
+#define LIN_R(t) round_storage<DT>(t)
+#define LIN_Q(v, s) LIN_R(__fdiv_rn(LIN_R(__fmul_rn((s), LIN_R(lin_clamp(rintf(LIN_R(__fdiv_rn((v), (s)))), lim)))), (s)))
   for (int it = 0; it < iters; ++it) {
     double num = 0.0, den = 0.0;
     for (int i = tid; i < n; i += LIN_THREADS) {
       const float v = sw[i];
       const float q = LIN_Q(v, step);
-      num += (double)__fmul_rn(q, v);
-      den += (double)__fmul_rn(q, q);
+      num += (double)LIN_R(__fmul_rn(q, v));
+      den += (double)LIN_R(__fmul_rn(q, q));
     }
     num = lin_warp_sum(num);
     den = lin_warp_sum(den);
@@ -107,9 +114,9 @@ __device__ __forceinline__ void lin_channel(const float* __restrict__ w, float* 
     if (tid == 0) {
       double a = 0.0, b = 0.0;
       for (int q = 0; q < LIN_THREADS / 32; ++q) { a += red[q][0]; b += red[q][1]; }
-      float s = __fdiv_rn((float)a, (float)b);
-      if (plus) s = __fmul_rn(c89, s);
-      bc[0] = lin_pow2_round_log2(s, flavor);
+      float s = LIN_R(__fdiv_rn(LIN_R((float)a), LIN_R((float)b)));
+      if (plus) s = LIN_R(__fmul_rn(c89, s));                     // the fp32 constant, as torch uses it for bf16 too
+      bc[0] = lin_pow2_round_log2<DT>(s, flavor);
     }
     __syncthreads();
     step = bc[0];
@@ -117,17 +124,21 @@ __device__ __forceinline__ void lin_channel(const float* __restrict__ w, float* 
   for (int i = tid; i < n; i += LIN_THREADS) {
     const int k = i / RS, j = i - k * RS;
     const float q = LIN_Q(sw[i], step);
-    const float yv = __fmul_rn(q, step);
-    y[((size_t)k * C + c) * RS + j] = yv;
+    const float yv = LIN_R(__fmul_rn(q, step));
+    if constexpr (DT == PO2_F32) y[((size_t)k * C + c) * RS + j] = yv;
+    else y[((size_t)k * C + c) * RS + j] = __float2bfloat16_rn(yv);     // exact: yv is on the bf16 grid
     if (pk.Bp) pack_store(pk, k, c, j, yv);
   }
 #undef LIN_Q
+#undef LIN_R
 }
 
-__global__ void __launch_bounds__(LIN_THREADS) lin_quantize_kernel(const float* __restrict__ w, float* __restrict__ y,
-                                                                   int K, int C, int RS, int bits, int iters,
-                                                                   int plus, int flavor, PackArgs pk) {
-  lin_channel(w, y, K, C, RS, bits, iters, plus, flavor, blockIdx.x, pk);
+template <int DT>
+__global__ void __launch_bounds__(LIN_THREADS) lin_quantize_kernel(const typename Tr<DT>::T* __restrict__ w,
+                                                                   typename Tr<DT>::T* __restrict__ y, int K, int C,
+                                                                   int RS, int bits, int iters, int plus, int flavor,
+                                                                   PackArgs pk) {
+  lin_channel<DT>(w, y, K, C, RS, bits, iters, plus, flavor, blockIdx.x, pk);
 }
 
 // Multi-tensor form: ONE launch for the lin layers of a model, one CTA per (tensor, input channel).  The tensor of a
@@ -140,7 +151,7 @@ __global__ void __launch_bounds__(LIN_THREADS) lin_multi_kernel(const LinDesc* _
     if (descs[mid].cta0 <= b) lo = mid; else hi = mid - 1;
   }
   const LinDesc& d = descs[lo];
-  lin_channel(d.w, d.y, d.K, d.C, d.RS, d.bits, d.iters, d.plus, d.flavor, b - d.cta0, d.pk);
+  lin_channel<PO2_F32>(d.w, d.y, d.K, d.C, d.RS, d.bits, d.iters, d.plus, d.flavor, b - d.cta0, d.pk);
 }
 
 int lin_check_args(int K, int C, int RS, int bits, int num_iters, int flavor) {
@@ -155,7 +166,7 @@ int lin_check_args(int K, int C, int RS, int bits, int num_iters, int flavor) {
 int lin_launch(const float* w, float* y, int K, int C, int RS, int bits, int iters, int plus, int flavor,
                const PackArgs& pk, cudaStream_t st) {
   const size_t smem = (size_t)K * RS * sizeof(float);
-  lin_quantize_kernel<<<C, LIN_THREADS, smem, st>>>(w, y, K, C, RS, bits, iters, plus, flavor, pk);
+  lin_quantize_kernel<PO2_F32><<<C, LIN_THREADS, smem, st>>>(w, y, K, C, RS, bits, iters, plus, flavor, pk);
   return (int)cudaGetLastError();
 }
 
@@ -167,12 +178,23 @@ extern "C" {
 
 int po2_lin_max_channel_elems(void) { return LIN_MAX_ELEMS; }
 
+int po2_lin_quantize_dt(const void* w, void* y, int K, int C, int RS, int bits, int num_iters, int plus, int flavor,
+                        int dtype, void* stream) {
+  if (!w || !y) return PO2_E_NULL;
+  if (dtype != PO2_F32 && dtype != PO2_BF16) return PO2_E_DTYPE;
+  if (int e = lin_check_args(K, C, RS, bits, num_iters, flavor)) return e;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == PO2_F32)
+    return lin_launch((const float*)w, (float*)y, K, C, RS, bits, num_iters, plus, flavor, PackArgs{}, st);
+  const size_t smem = (size_t)K * RS * sizeof(float);           // the channel's fp32 widening
+  lin_quantize_kernel<PO2_BF16><<<C, LIN_THREADS, smem, st>>>((const __nv_bfloat16*)w, (__nv_bfloat16*)y, K, C, RS, bits,
+                                                              num_iters, plus, flavor, PackArgs{});
+  return (int)cudaGetLastError();
+}
+
 int po2_lin_quantize(const void* w, void* y, int K, int C, int RS, int bits, int num_iters, int plus, int flavor,
                      void* stream) {
-  if (!w || !y) return PO2_E_NULL;
-  if (int e = lin_check_args(K, C, RS, bits, num_iters, flavor)) return e;
-  return lin_launch((const float*)w, (float*)y, K, C, RS, bits, num_iters, plus, flavor, PackArgs{},
-                    (cudaStream_t)stream);
+  return po2_lin_quantize_dt(w, y, K, C, RS, bits, num_iters, plus, flavor, PO2_F32, stream);
 }
 
 size_t po2_lin_multi_desc_bytes(void) { return sizeof(LinDesc); }

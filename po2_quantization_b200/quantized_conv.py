@@ -140,20 +140,26 @@ class QuantizedConv2d(nn.Conv2d):
             self.__dict__["_po2_pack_cache"] = cache
         return cache[1]
 
-    def _bf16_forward(self, input, ep=None):
-        """forward of a bf16 PO2 / PO2+ layer at inference (PTQ weights, or a QAT layer in eval), ep = (ep_a, ep_b,
-        residual, act) for the folded form.  Cached in _po2_pack_cache per (weight version, input shape, device, mode,
-        dtype): the packed operand, or the fp32 widening of the bf16 weight for the depthwise / small-pointwise kernels.
-        A QAT layer's weight is quantized in bf16 first (quantize_full), as the quantizer itself does on a bf16 model."""
+    def _bf16_forward(self, input, family, ep=None):
+        """forward of a bf16 PO2 / PO2+ / lin / lin+ layer at inference (PTQ weights, or a QAT layer in eval); family:
+        what _bf16_layer returned; ep = (ep_a, ep_b, residual, act) for the folded form.  Cached in _po2_pack_cache per
+        (weight version, input shape, device, mode, dtype, family): the packed operand, or the fp32 widening of the bf16
+        weight for the depthwise / small-pointwise kernels.  A QAT layer's weight is quantized in bf16 first
+        (quantize_full, or the bf16 lin kernel), as the quantizer itself does on a bf16 model.  A lin weight y is a bf16
+        tensor, so it is its own exact operand at any bit width, with scale 1.0 (ops.lin_scale)."""
         mode = ops.get_conv_mode()
         compute, w = ops.COMPUTE[mode], self.weight
         stride, pad, groups = self.stride[0], self.padding[0], self.groups
         fam = _quantizers.quantizer_family(self.quantize_fn) if self.quantize_fn is not None else None
         qat = (int(self.bits), fam[1]) if fam is not None else ()
-        key = (w._version, tuple(input.shape), input.device, mode, input.dtype) + qat
+        key = (w._version, tuple(input.shape), input.device, mode, input.dtype, family) + qat
         cache = self.__dict__.get("_po2_pack_cache")
         if cache is None or cache[0] != key:
-            if qat:
+            if family == "lin":
+                y = (_quantizers._lin_forward_cuda(w.detach(), int(self.bits), ops.LIN_ITERS, fam[1]) if qat
+                     else w.detach())
+                scale = ops.lin_scale(input.device)
+            elif qat:
                 y, _codes, scale, _zc, _sse = ops.quantize_full(w.detach(), int(self.bits), 1, bool(fam[1]))
             else:
                 y, scale = w.detach(), self._po2_ptq[1]
@@ -172,15 +178,29 @@ class QuantizedConv2d(nn.Conv2d):
                                         int(act))
         return ops.conv2d_ep(input, wf, scale, stride, pad, groups, compute, ep_a, ep_b, residual, int(act))
 
-    def _bf16_po2_layer(self, input) -> bool:
-        """a PO2 / PO2+ layer (QAT quantizer or current PTQ tag) whose bf16 call the kernels take"""
+    def _bf16_layer(self, input):
+        """"po2" / "lin": the quantizer family of a layer whose bf16 call the kernels take at inference (a PO2 / lin QAT
+        quantizer, or a current PTQ tag); None for any other layer or call.  A lin QAT layer also needs the bf16 lin
+        quantizer kernel to take its weight."""
         if self.quantize_fn is not None:
             fam = _quantizers.quantizer_family(self.quantize_fn)
-            po2 = fam is not None and fam[0] == "po2"
+            family = fam[0] if fam is not None else None
+            if family == "lin":
+                from . import _lib
+                K, _, R, S = self.weight.shape
+                if (os.environ.get("PO2_LIN", "cuda") != "cuda" or not 2 <= int(self.bits) <= 16
+                        or K * R * S > _lib.load().po2_lin_max_channel_elems()):
+                    family = None
         else:
-            tag = getattr(self, "_po2_ptq", None)
-            po2 = tag is not None and tag[0] == self.weight._version
-        return po2 and input.dtype == torch.bfloat16 and self._why_not(input) == ""
+            family = None
+            for name, tagged in (("_po2_ptq", "po2"), ("_po2_lin_ptq", "lin")):
+                tag = self.__dict__.get(name)
+                if tag is not None and tag[0] == self.weight._version:
+                    family = tagged
+                    break
+        if family is None or input.dtype != torch.bfloat16 or self._why_not(input) != "":
+            return None
+        return family
 
     def _library_conv(self, input, weight, why):
         if why:
@@ -196,8 +216,10 @@ class QuantizedConv2d(nn.Conv2d):
 
     def forward(self, input):
         # models/quantized_conv.py:32-38: quantize the weight on every forward (QAT), then conv
-        if input.dtype == torch.bfloat16 and input.is_cuda and self._bf16_po2_layer(input):
-            return self._bf16_forward(input)
+        if input.dtype == torch.bfloat16 and input.is_cuda:
+            family = self._bf16_layer(input)
+            if family is not None:
+                return self._bf16_forward(input, family)
         if self.quantize_fn is not None:
             fam = _quantizers.quantizer_family(self.quantize_fn)
             if fam is not None and fam[0] == "lin":
@@ -265,7 +287,8 @@ class QuantizedConv2d(nn.Conv2d):
         if mode == "cudnn" or self._why_not(input) != "":
             return None
         if input.dtype == torch.bfloat16:
-            return self._bf16_forward(input, (ep_a, ep_b, residual, act)) if self._bf16_po2_layer(input) else None
+            family = self._bf16_layer(input)
+            return self._bf16_forward(input, family, (ep_a, ep_b, residual, act)) if family is not None else None
         compute = ops.COMPUTE[mode]
         K, _, R, S = self.weight.shape
         if self.quantize_fn is not None:

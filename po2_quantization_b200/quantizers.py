@@ -54,8 +54,9 @@ class PowerOfTwoPlusQuantizer(_Po2Base):
 
 # ------------------------------------------------------------------------------------------------
 # lin / lin+ (SURVEY.md section 8f "next" #1): per-input-channel uniform quantizer whose step is
-# constrained to a power of two (utils/quantizers.py:8-16, 59-136).  CUDA fp32 4-D weights take the
-# single-launch kernel of csrc/po2_lin.cu; everything else the op-by-op form below.
+# constrained to a power of two (utils/quantizers.py:8-16, 59-136).  CUDA fp32 or bf16 4-D weights take the
+# single-launch kernel of csrc/po2_lin.cu (bf16: each op rounded to bf16, as the op-by-op form does on bf16 tensors);
+# everything else the op-by-op form below.
 # ------------------------------------------------------------------------------------------------
 def _uniform_per_in_channel(w: torch.Tensor, step: torch.Tensor, bits: int) -> torch.Tensor:
     s = step.view(-1, 1, 1)
@@ -64,7 +65,8 @@ def _uniform_per_in_channel(w: torch.Tensor, step: torch.Tensor, bits: int) -> t
 
 
 def _lin_forward_cuda(w: torch.Tensor, bits: int, num_iters: int, plus: bool):
-    """one launch of csrc/po2_lin.cu (one CTA per input channel), or None if the shape is not taken"""
+    """one launch of csrc/po2_lin.cu (one CTA per input channel) for an fp32 or bf16 w, or None if the shape is not
+    taken"""
     from . import _lib
     lib = _lib.load()
     K, C = w.shape[0], w.shape[1]
@@ -74,23 +76,24 @@ def _lin_forward_cuda(w: torch.Tensor, bits: int, num_iters: int, plus: bool):
     x = w.contiguous()
     y = torch.empty_like(x)
     with torch.cuda.device(x.device):
-        rc = lib.po2_lin_quantize(x.data_ptr(), y.data_ptr(), K, C, RS, int(bits), int(num_iters), int(plus), ops._flavor,
-                                  ops._stream_ptr(x.device))
+        rc = lib.po2_lin_quantize_dt(x.data_ptr(), y.data_ptr(), K, C, RS, int(bits), int(num_iters), int(plus),
+                                     ops._flavor, ops._DT[x.dtype], ops._stream_ptr(x.device))
     if rc == -10:
         return None
-    _lib.check(rc, "po2_lin_quantize")
+    _lib.check(rc, "po2_lin_quantize_dt")
     ops.LAUNCHES += 1
     return y
 
 
 def _lin_forward(w: torch.Tensor, bits: int, num_iters: int, plus: bool) -> torch.Tensor:
-    if w.is_cuda and w.dtype == torch.float32 and w.dim() == 4 and w.numel() > 0 and os.environ.get("PO2_LIN", "cuda") == "cuda":
+    kernel_dtype = w.dtype in (torch.float32, torch.bfloat16)
+    if w.is_cuda and kernel_dtype and w.dim() == 4 and w.numel() > 0 and os.environ.get("PO2_LIN", "cuda") == "cuda":
         y = _lin_forward_cuda(w.detach(), bits, num_iters, plus)
         if y is not None:
             return y
         why = "a channel exceeds the kernel's shared-memory capacity or bits is outside 2..16"
     else:
-        why = ("CPU tensor" if not w.is_cuda else f"dtype {w.dtype}" if w.dtype != torch.float32 else
+        why = ("CPU tensor" if not w.is_cuda else f"dtype {w.dtype}" if not kernel_dtype else
                f"{w.dim()}-D tensor" if w.dim() != 4 else "empty tensor" if w.numel() == 0 else "PO2_LIN != cuda")
     # op-by-op ATen form in the reference's order (utils/quantizers.py:59-136) -- a library path, so it is
     # reported (once per reason; an error under PO2_STRICT=1).  lin / lin+ are SURVEY section 8f "next" rows:
