@@ -83,6 +83,7 @@ int po2_absmax(const void* x, int64_t n, int dtype, float* scale_out, void* work
  *   nibble), else one per byte; code = signbit<<(bits-1) | ((fsr-1)-q).
  * zero_count (optional, caller-zeroed u32): number of inputs equal to +-0; those produce y = +0
  *   (the reference's sign() is 0) but have no code of their own and are emitted as (+, min level).
+ *   A u32: an input with 2^32 or more zeros wraps it (the count is modulo 2^32).
  * sse (optional, caller-zeroed double): accumulates sum((y-x)^2) -- models/quantized_conv.py:43,
  *   utils/quantizers.py:149.
  * bits in [2, 8].  x, y 16-byte aligned for the vector path (any alignment is accepted). */

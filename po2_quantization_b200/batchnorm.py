@@ -366,8 +366,13 @@ def _route_skip_gradient(residual: torch.Tensor) -> torch.Tensor:
     return _SkipGrad.apply(residual, node)
 
 
+# the norm kernels index x in 32 bits: po2_bn_* refuse 2^31 or more elements (PO2_E_SIZE)
+BN_MAX_NUMEL = 2**31 - 1
+
+
 def _kernel_ok(x: torch.Tensor) -> bool:
-    return x.is_cuda and x.dtype == torch.float32 and x.dim() >= 2 and x.numel() > 0 and x.shape[1] <= 4096
+    return (x.is_cuda and x.dtype == torch.float32 and x.dim() >= 2 and 0 < x.numel() <= BN_MAX_NUMEL
+            and x.shape[1] <= 4096)
 
 
 ACT = {None: 0, "none": 0, "relu": 1, "relu6": 2, "silu": 3}
@@ -438,6 +443,7 @@ class FusedSyncBatchNorm(nn.SyncBatchNorm):
         # stock path (CPU tensors, other dtypes, eval mode under autograd, cumulative-average momentum):
         # a library path, reported once per reason (an error under PO2_STRICT=1)
         why = ("CPU tensor" if not input.is_cuda else f"dtype {input.dtype}" if input.dtype != torch.float32 else
+               f"{input.numel()} elements (the kernels take up to 2^31 - 1)" if input.numel() > BN_MAX_NUMEL else
                "residual of another shape/dtype" if not fast else
                "eval mode under autograd" if not use_batch_stats else "momentum=None (cumulative average)")
         ops.note_library_path("bn:" + why, f"FusedSyncBatchNorm runs nn.SyncBatchNorm's own forward: {why}")

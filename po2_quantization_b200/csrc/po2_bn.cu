@@ -23,6 +23,8 @@
 // sums go to a workspace and the last CTA of a channel to finish (ticket counter, self-resetting)
 // combines them in double precision.  Sums are shifted by the channel's first element so that
 // E[x^2]-E[x]^2 cancellation stays harmless when |mean| >> std.
+#include <type_traits>
+
 #include "po2_common.cuh"
 
 namespace po2 {
@@ -228,6 +230,11 @@ __device__ unsigned long long* g_bn_trace = nullptr;
 #define BN_STAMP(i) do {} while (0)
 #endif
 
+// Index of the element loops.  The VEC forms count float4s, so their counts stay below 2^29 and a 32-bit index never
+// nears 2^31.  The scalar forms count floats: a count below 2^31 may lie within one step of 2^31, so they step in
+// 64 bits.
+template <bool VEC> using BnIdx = typename std::conditional<VEC, int, int64_t>::type;
+
 // MODE 0: forward statistics (p = x - shift, q = p);  1: backward sums (p = dy, q = x - mean);
 // MODE 2: backward sums behind a ReLU (p = y > 0 ? dy : 0).
 template <bool VEC, int MODE>
@@ -267,7 +274,7 @@ __global__ void __launch_bounds__(BN_THREADS) bn_reduce_kernel(const float* __re
   if (threadIdx.x == 0 && peers.world > 1)
     s_epoch = *reinterpret_cast<volatile uint32_t*>(&peers.box[peers.rank]->epoch) + 1;
   float s1 = 0.f, s2 = 0.f;
-  for (int i0 = threadIdx.x; i0 < n; i0 += BN_UNROLL * BN_THREADS) {
+  for (BnIdx<VEC> i0 = threadIdx.x; i0 < n; i0 += BN_UNROLL * BN_THREADS) {
     if (VEC) {
       float4 vx[BN_UNROLL], vd[BN_UNROLL], vy[BN_UNROLL];
 #pragma unroll
@@ -306,8 +313,8 @@ __global__ void __launch_bounds__(BN_THREADS) bn_reduce_kernel(const float* __re
     } else {
 #pragma unroll
       for (int u = 0; u < BN_UNROLL; ++u) {
-        const int i = i0 + u * BN_THREADS;
-        if (i < n) {
+        if (i0 + u * BN_THREADS < n) {
+          const int i = (int)(i0 + u * BN_THREADS);
           const int k = fdiv(i, g.div_l);
           const size_t off = ((size_t)(s + k * g.S) * C + c) * L + (i - k * L);
           const float xv = __ldg(x + off);
@@ -441,7 +448,7 @@ __global__ void __launch_bounds__(BN_THREADS, 4) bn_apply_kernel(const float* __
   if (blockIdx.x == 0 && threadIdx.x == 0 && !use_running && num_batches_tracked) *num_batches_tracked += 1;
   __syncthreads();
   const int L = g.L;
-  for (int i0 = blockIdx.x * (BN_UNROLL * BN_THREADS) + threadIdx.x; i0 < g.total;
+  for (BnIdx<VEC> i0 = blockIdx.x * (BN_UNROLL * BN_THREADS) + threadIdx.x; i0 < g.total;
        i0 += gridDim.x * (BN_UNROLL * BN_THREADS)) {
     if (VEC) {
       float4 vx[BN_UNROLL], vr[BN_UNROLL];
@@ -471,8 +478,8 @@ __global__ void __launch_bounds__(BN_THREADS, 4) bn_apply_kernel(const float* __
     } else {
 #pragma unroll
       for (int u = 0; u < BN_UNROLL; ++u) {
-        const int i = i0 + u * BN_THREADS;
-        if (i < g.total) {
+        if (i0 + u * BN_THREADS < g.total) {
+          const int i = (int)(i0 + u * BN_THREADS);
           const int slab = fdiv(i, g.div_l);
           const int c = slab - fdiv(slab, g.div_c) * C;
           const float4 p = prm[c];
@@ -527,7 +534,7 @@ __global__ void __launch_bounds__(BN_THREADS, 4) bn_bwd_apply_kernel(const float
   __syncthreads();
   const bool silu = act == 3;
   const bool relu = act != 0 && !silu;                         // masked by the activation's open interval
-  for (int i0 = blockIdx.x * (BN_UNROLL * BN_THREADS) + threadIdx.x; i0 < g.total;
+  for (BnIdx<VEC> i0 = blockIdx.x * (BN_UNROLL * BN_THREADS) + threadIdx.x; i0 < g.total;
        i0 += gridDim.x * (BN_UNROLL * BN_THREADS)) {
     if (VEC) {
       float4 vd[BN_UNROLL], vx[BN_UNROLL], vy[BN_UNROLL];
@@ -570,8 +577,8 @@ __global__ void __launch_bounds__(BN_THREADS, 4) bn_bwd_apply_kernel(const float
     } else {
 #pragma unroll
       for (int u = 0; u < BN_UNROLL; ++u) {
-        const int i = i0 + u * BN_THREADS;
-        if (i < g.total) {
+        if (i0 + u * BN_THREADS < g.total) {
+          const int i = (int)(i0 + u * BN_THREADS);
           const int slab = fdiv(i, g.div_l);
           const int c = slab - fdiv(slab, g.div_c) * C;
           const float4 p = prm[c];

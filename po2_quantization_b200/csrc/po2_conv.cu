@@ -138,7 +138,8 @@ struct ConvGeom {
   int tf32, G;           // operand kind: bf16 (G = 8 channels per 16-byte plane entry) or tf32 (G = 4)
   int Cpad, CC, nchunk;  // channels padded to 2G (one MMA k-step); channels per pipeline stage; stages per item
   int NT, ntiles_n;      // out-channel tile (multiple of 16, <= 256) and their count
-  int nitems_m, m_step;  // 128-position items; items advance by m_step per CTA iteration
+  int nitems_m, m_step;  // 128-position items; items advance by m_step per CTA iteration (nitems_m < 2^24 and
+                         // m_step <= 148: the 32-bit item loops stay far below 2^31)
   int nst;               // A pipeline stages
   uint32_t a_stage_bytes, b_slab_bytes;
   FastDiv div_pitch, div_rows, div_strip, div_ipr, div_NT, div_ncg, div_taps;
@@ -163,7 +164,7 @@ __global__ void pack_weights_kernel(const float* __restrict__ w, const uint8_t* 
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   const int G = g.G, lgG = (G == 8) ? 3 : 2;
   const int taps = g.ntaps, ncg = g.Cpad / G;
-  const int total = g.ntiles_n * taps * ncg * g.NT * G;           // < 2^31 (weights)
+  const int total = g.ntiles_n * taps * ncg * g.NT * G;           // < 2^30 (plan_tc): i + stride cannot wrap
   const float s = scale ? *scale : 1.0f;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     // i = (((nt * taps + tap) * ncg + cg) * NT + n) * G + j, decoded with mul-hi divisions
@@ -661,7 +662,7 @@ __global__ void __launch_bounds__(K3_THREADS, 1) conv_umma_kernel(const XT* __re
 // ------------------------------------------------------------------------------------------------
 struct DwGeom {
   int C, H, W, P, Q, Q4, stride;
-  int total;                 // B*C*P*Q4 threads' worth of work
+  int total;                 // B*C*P*Q4 threads' worth of work: < 2^29, so the 32-bit loop never nears 2^31
   FastDiv div_q4, div_p, div_c;
 };
 
@@ -741,7 +742,9 @@ __global__ void __launch_bounds__(256) conv_depthwise_kernel(const XT* __restric
                                                              XT* __restrict__ out, ConvGeom g,
                                                              FastDiv div_q, FastDiv div_p, FastDiv div_c, ConvEpilogue ep) {
   const int total = g.B * g.C * g.P * g.Q;                 // < 2^31 (checked on the host)
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+  // total may lie within one grid stride of 2^31: a 32-bit i would wrap on its last step
+  for (int64_t i64 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i64 < total; i64 += (int64_t)gridDim.x * blockDim.x) {
+    const int i = (int)i64;
     int t = fdiv(i, div_q);
     const int q = i - t * g.Q;
     const int plane = fdiv(t, div_p);
@@ -973,6 +976,9 @@ static size_t round256(size_t n) { return (n + 255) / 256 * 256; }
 static bool plan_tc(ConvPlan& p, bool tf32) {
   const bool bf16x = p.dtype == PO2_BF16;
   if (!plan_umma(p.g, tf32 && !bf16x, bf16x)) return false;
+  // pack_weights_kernel's 32-bit grid-stride loop runs over the operand's elements: keep it a stride below 2^31
+  // (checked before the plan is filled in: a refused shape keeps kind, tapminor and pack_bytes of a CUDA-core plan)
+  if ((int64_t)p.g.ntiles_n * p.g.NT * p.g.ntaps * p.g.Cpad >= (1ll << 30)) return false;
   p.kind = (tf32 && !bf16x && tma_enabled() && plan_tma(p.g, p.tp)) ? 3 : 2;
   p.g.tapminor = (p.kind == 3 && p.g.ntaps == 9) ? 1 : 0;
   p.pack_bytes = (size_t)p.g.ntiles_n * p.g.b_slab_bytes;
@@ -988,6 +994,7 @@ static int plan_fwd(ConvPlan& p, int B, int C, int H, int W, int K, int R, int S
   if (dtype != PO2_F32 && dtype != PO2_BF16) return PO2_E_DTYPE;
   p.dtype = dtype;
   if (!fill_geom(p.g, B, C, H, W, K, R, S, stride, pad, groups)) return PO2_E_SHAPE;
+  if (!index_fits(p.g)) return PO2_E_SIZE;
   // the pointwise layers on tiny feature maps go to the fp32 cluster GEMM of csrc/po2_conv_bwd.cu, not to K3 / K3T
   const bool pw_small = pw_small_takes(B, C, H, W, K, R, S, stride, pad, groups);
   if (compute == 1 || !umma_shape_ok(p.g) || pw_small || !plan_tc(p, compute == 2))
@@ -1577,7 +1584,6 @@ int po2_conv2d_fwd_ep_dt(const void* x, const void* w, const float* scale, void*
   const ConvGeom& g = p.g;
   if (w_format != PO2_W_F32_PO2 && w_format != PO2_W_CODES) return PO2_E_UNSUPPORTED;
   if (w_format == PO2_W_CODES && (!scale || bits < 2 || bits > 8)) return PO2_E_BITS;
-  if (!index_fits(g)) return PO2_E_SIZE;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t wn = (int64_t)K * (C / groups) * R * S;
   const size_t wbytes = round256((size_t)wn * sizeof(float));
@@ -1719,7 +1725,6 @@ int po2_conv2d_fwd_packed_ep_dt(const void* x, const void* packed, const float* 
   ConvPlan p;
   if (int e = plan_fwd(p, B, C, H, W, K, R, S, stride, pad, groups, compute, dtype)) return e;
   if (!p.pack_bytes) return PO2_E_UNSUPPORTED;
-  if (!index_fits(p.g)) return PO2_E_SIZE;
   if (int a = umma_check_x(x, p)) return a;
   return launch_conv(p, x, packed, scale, out, pdl_chain_enabled() ? 2 : 0, ep, (cudaStream_t)stream);
 }
@@ -1743,7 +1748,6 @@ int po2_qconv2d_fwd(const void* x, const void* w_master, void* qw_out, float* sc
     if (int a = umma_check_x(x, p)) return a;                 // before the quantizer runs
   if (p.unpadded) {
     if (!workspace || workspace_bytes < p.workspace) return PO2_E_WORKSPACE;
-    if (!index_fits(p.g)) return PO2_E_SIZE;
     const PackArgs pk = pack_args(p.g, reinterpret_cast<char*>(workspace) + round256((size_t)wn * sizeof(float)));
     const int rc = fused_quantize_pack(w_master, qw_out, scale_out, wn, bits, fsr, mode, flavor, quant_workspace, pk, st);
     if (rc == 0) return launch_conv(p, x, pk.Bp, scale_out, out, 1, ConvEpilogue{}, st);

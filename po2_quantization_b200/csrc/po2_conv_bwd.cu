@@ -36,7 +36,9 @@ __global__ void __launch_bounds__(256) dilate2_kernel(const float* __restrict__ 
 // 4-byte alignment: g (planes, P, Q) -> g_up (planes, H, W).  One thread = one output element, scalar accesses.
 __global__ void __launch_bounds__(256) dilate2_into_kernel(const float* __restrict__ g, float* __restrict__ up, int P,
                                                            int Q, int H, int W, int total) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+  // total < 2^31 may lie within one grid stride of 2^31: a 32-bit i would wrap on its last step
+  for (int64_t i64 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i64 < total; i64 += (int64_t)gridDim.x * blockDim.x) {
+    const int i = (int)i64;
     const int row = i / W, w = i - row * W;                                       // row = plane * H + h
     const int plane = row / H, h = row - plane * H;
     up[i] = ((h | w) & 1) ? 0.f : __ldg(g + ((size_t)plane * P + (h >> 1)) * Q + (w >> 1));
@@ -47,7 +49,8 @@ __global__ void __launch_bounds__(256) dilate2_into_kernel(const float* __restri
 //   gx[h][w] = sum_{r,s} g[h + 1 - r][w + 1 - s] * w[c][r][s]
 __global__ void __launch_bounds__(256) dw_dgrad_kernel(const float* __restrict__ g, const float* __restrict__ w,
                                                        float* __restrict__ gx, int C, int H, int W, int total) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+  for (int64_t i64 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i64 < total; i64 += (int64_t)gridDim.x * blockDim.x) {
+    const int i = (int)i64;                                     // 64-bit step: total may lie within a stride of 2^31
     const int x = i % W;
     const int t = i / W;
     const int y = t % H;
@@ -86,10 +89,12 @@ __global__ void __launch_bounds__(DWG_THREADS) dw_wgrad_kernel(const float* __re
   float acc[9];
 #pragma unroll
   for (int k = 0; k < 9; ++k) acc[k] = 0.f;
-  for (int n = split; n < B; n += S) {
+  // 64-bit steps: B and HW may each lie within one step of 2^31 (B * C * H * W < 2^31 is all the host checks)
+  for (int64_t n = split; n < B; n += S) {
     const float* pg = g + ((size_t)n * C + c) * HW;
     const float* px = x + ((size_t)n * C + c) * HW;
-    for (int i = threadIdx.x; i < HW; i += DWG_THREADS) {
+    for (int64_t i64 = threadIdx.x; i64 < HW; i64 += DWG_THREADS) {
+      const int i = (int)i64;
       const float gv = __ldg(pg + i);
       if (gv == 0.f) continue;                                  // zero-inserted gradients: 3 of 4 positions
       const int y = i / W, xx = i - y * W;
@@ -222,11 +227,19 @@ static size_t stem_wgrad_smem(int C, int H, int W, int K) {
 static bool stem_wgrad_takes(int B, int C, int H, int W, int K, int R, int S, int stride, int pad, int groups) {
   if (R != 3 || S != 3 || stride != 1 || pad != 1 || groups != 1 || B < 1) return false;
   if (C < 1 || C > 4 || K < 1 || K * C > SW_THREADS || H < 1 || W < 1) return false;
-  return stem_wgrad_smem(C, H, W, K) <= 200 * 1024 && (int64_t)B * K * H * W < (1ll << 31);
+  // B < 2^30 keeps the image loop's 32-bit n += gridDim.x (<= 148) from wrapping; the other loops stay in shared memory
+  return stem_wgrad_smem(C, H, W, K) <= 200 * 1024 && (int64_t)B * K * H * W < (1ll << 31) && B < (1 << 30);
 }
 static int stem_wgrad_ctas(int B) {
   const int sms = device_sm_count();
   return B < sms ? B : sms;
+}
+
+// blocks of 256 threads for a grid-stride loop over total < 2^31 elements, at most 16 per SM (64-bit: total + 255
+// must not wrap)
+static int grid_blocks(int total) {
+  const int64_t need = ((int64_t)total + 255) / 256, cap = (int64_t)device_sm_count() * 16;
+  return (int)(need < cap ? need : cap);
 }
 
 constexpr int DWG_MAX_C = 4096;
@@ -266,8 +279,8 @@ int po2_dilate2(const void* g, void* g_up, int planes, int P, int Q, void* strea
   if (planes <= 0 || P <= 0 || Q <= 0) return PO2_E_SHAPE;
   if (Q % 2 || (reinterpret_cast<uintptr_t>(g) & 7) || (reinterpret_cast<uintptr_t>(g_up) & 15)) return PO2_E_UNSUPPORTED;
   if ((int64_t)planes * P * Q * 4 >= (1ll << 31)) return PO2_E_SIZE;
-  const int rows = planes * P, total = rows * (Q / 2);
-  const int blocks = (total + 255) / 256 < device_sm_count() * 16 ? (total + 255) / 256 : device_sm_count() * 16;
+  const int rows = planes * P, total = rows * (Q / 2);          // < 2^28: dilate2_kernel's 32-bit i never nears 2^31
+  const int blocks = grid_blocks(total);
   dilate2_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>((const float*)g, (float*)g_up, Q / 2, rows, Q);
   return (int)cudaGetLastError();
 }
@@ -277,7 +290,7 @@ int po2_dilate2_into(const void* g, void* g_up, int planes, int P, int Q, int H,
   if (planes <= 0 || H <= 0 || W <= 0 || P != (H - 1) / 2 + 1 || Q != (W - 1) / 2 + 1) return PO2_E_SHAPE;
   if ((int64_t)planes * H * W >= (1ll << 31)) return PO2_E_SIZE;
   const int total = planes * H * W;
-  const int blocks = (total + 255) / 256 < device_sm_count() * 16 ? (total + 255) / 256 : device_sm_count() * 16;
+  const int blocks = grid_blocks(total);
   dilate2_into_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>((const float*)g, (float*)g_up, P, Q, H, W, total);
   return (int)cudaGetLastError();
 }
@@ -288,7 +301,7 @@ int po2_conv2d_depthwise_dgrad(const void* g, const void* w, void* gx, int B, in
   if (B <= 0 || C <= 0 || H <= 0 || W <= 0) return PO2_E_SHAPE;
   if ((int64_t)B * C * H * W >= (1ll << 31)) return PO2_E_SIZE;
   const int total = B * C * H * W;
-  const int blocks = (total + 255) / 256 < device_sm_count() * 16 ? (total + 255) / 256 : device_sm_count() * 16;
+  const int blocks = grid_blocks(total);
   dw_dgrad_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>((const float*)g, (const float*)w, (float*)gx, C, H, W, total);
   return (int)cudaGetLastError();
 }

@@ -51,7 +51,7 @@ __global__ void __launch_bounds__(SGD_THREADS) sgd_multi_kernel(const __grid_con
   for (int u = 0; u < 4; ++u) {
     const int e = e0 + (u * SGD_THREADS + (int)threadIdx.x) * 4;
     if (e >= n) break;
-    if (vec && e + 4 <= n) {
+    if (vec && e <= n - 4) {                        // n < 2^31 may be within 4 of 2^31: e + 4 would wrap
       float4 pv = *reinterpret_cast<const float4*>(p + e);
       const float4 gv = __ldg(reinterpret_cast<const float4*>(g + e));
       float4 bv = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -63,7 +63,7 @@ __global__ void __launch_bounds__(SGD_THREADS) sgd_multi_kernel(const __grid_con
       *reinterpret_cast<float4*>(p + e) = pv;
       if (mom != 0.f) *reinterpret_cast<float4*>(buf + e) = bv;
     } else {
-      for (int i = e; i < min(e + 4, n); ++i) {
+      for (int i = e; i < e + min(4, n - e); ++i) {
         float b = (mom != 0.f && !first) ? buf[i] : 0.f;
         const float pn = sgd_one(p[i], g[i], &b, lr, mom, wd, first);
         p[i] = pn;

@@ -84,6 +84,7 @@ LAUNCHES = 0
 # "fp32": CUDA-core fp32 FMA everywhere (the fp32-accumulate parity mode); "cudnn": leave the convolution
 # to F.conv2d.
 COMPUTE = {"tc": 0, "fp32": 1, "tf32": 2}
+E_SIZE = -4                    # PO2_E_SIZE: a tensor of 2^31 or more elements
 DEFAULT_CONV_MODE = os.environ.get("PO2_CONV", "tf32")      # the mode of a fresh process (tests restore it)
 _conv_mode = DEFAULT_CONV_MODE
 
@@ -557,6 +558,15 @@ def _depthwise_backward(g_full, x, w, need_x, need_w):
     return gx, gw
 
 
+def _stride1_taken(B, C, H, W_, K, R, pad, compute, need_x, need_w) -> bool:
+    """whether a kernel takes either gradient of the stride-1 problem on the zero-inserted output gradient (B, K, H, W)
+    of a dense stride-2 layer.  The planner refuses it, among other reasons, when that gradient has 2^31 or more
+    elements, which po2_dilate2 would refuse too: the layer then leaves the kernels before anything is dilated."""
+    lib = _lib.load()
+    return bool((need_x and lib.po2_conv2d_dgrad_workspace(B, C, H, W_, K, R, R, pad, compute) > 0) or
+                (need_w and lib.po2_conv2d_wgrad_kernel_kind(B, C, H, W_, K, R, R, 1, pad, 1, compute) != 0))
+
+
 def _conv_backward(g, x, w, scale, stride, pad, groups, compute, need_x, need_w, packed_d=None, defer_w=False):
     """(gx, gw) of conv2d(x, w) on our kernels: dense layers on the tcgen05 kernels (data gradient: the forward
     kernel with transposed weights; weight gradient: K5T / K5, or the fp32 GEMM for small wide 1x1 layers) --
@@ -576,7 +586,8 @@ def _conv_backward(g, x, w, scale, stride, pad, groups, compute, need_x, need_w,
         tuple(g.shape[2:]) == ((H - 1) // 2 + 1, (W_ - 1) // 2 + 1)
     with torch.cuda.device(x.device):
         g_s1 = g
-        if stride == 2 and (ours or depthwise) and s2_ok and (need_x or need_w):
+        if stride == 2 and (ours or depthwise) and s2_ok and (need_x or need_w) and \
+                (depthwise or _stride1_taken(B, C, H, W_, K, R, pad, compute, need_x, need_w)):
             g_s1 = torch.empty(B, K, H, W_, dtype=torch.float32, device=g.device)
             if H % 2 == 0 and W_ % 2 == 0 and g.shape[3] % 2 == 0:
                 dilate2_out(g, g_s1)

@@ -5,13 +5,17 @@ weight_decay)``, train.py:92 ``optimizer.step()``) as ONE launch per 96 paramete
 ``state_dict`` and LR-scheduler behaviour; only ``step()`` differs for parameters that are fp32 CUDA tensors --
 torch's foreach path issues 14 launches for ResNet-56's 171 parameters, ``po2_sgd_step`` two, with the same
 roundings (bit-identical parameters, tests/test_models_gpu.py).  Everything else (CPU tensors, other dtypes,
-Nesterov, dampening, maximize, sparse gradients) is handed to ``torch.optim.SGD.step``.  CUDA-graph capturable like the
+Nesterov, dampening, maximize, sparse gradients, tensors of 2^31 or more elements) is handed to
+``torch.optim.SGD.step``.  CUDA-graph capturable like the
 stock optimizer with a float ``lr`` (the value is baked into the captured launch)."""
 import ctypes
 
 import torch
 
 from . import _lib, ops
+
+
+SGD_MAX_NUMEL = 2**31 - 1     # po2_sgd_step indexes a tensor in 32 bits and refuses larger ones (PO2_E_SIZE)
 
 
 class SGD(torch.optim.SGD):
@@ -30,8 +34,12 @@ class SGD(torch.optim.SGD):
                 g = p.grad
                 if g is None:
                     continue
-                if not (ours and p.is_cuda and p.dtype == torch.float32 and g.dtype == torch.float32 and not g.is_sparse
-                        and p.is_contiguous() and g.is_contiguous() and g.device == p.device):
+                taken = (ours and p.is_cuda and p.dtype == torch.float32 and g.dtype == torch.float32 and not g.is_sparse
+                         and p.is_contiguous() and g.is_contiguous() and g.device == p.device)
+                if not (taken and p.numel() <= SGD_MAX_NUMEL):
+                    if taken:                     # the size is the only reason: a kernel-eligible tensor leaves it
+                        ops.note_library_path("sgd:size", f"optim.SGD hands a parameter of {p.numel()} elements to "
+                                              "torch.optim.SGD.step (po2_sgd_step takes up to 2^31 - 1)")
                     rest.append(p)
                     continue
                 first = "momentum_buffer" not in self.state[p] or self.state[p]["momentum_buffer"] is None

@@ -63,8 +63,17 @@ class QuantizedConv2d(nn.Conv2d):
             return f"padding {self.padding!r} / padding_mode {self.padding_mode!r}"
         if self.stride[0] != self.stride[1] or self.padding[0] != self.padding[1]:
             return f"non-square stride {self.stride} / padding {self.padding}"
-        if bf16 and ops.conv_kernel_kind(input.shape, self.weight.shape, self.stride[0], self.padding[0], self.groups,
-                                         ops.COMPUTE[ops.get_conv_mode()], input.dtype) < 0:
+        # the planner's answer for this input shape, asked once per shape: PO2_E_SIZE when x or the output has 2^31 or
+        # more elements (the kernels index them in 32 bits), PO2_E_UNSUPPORTED for a bf16 shape no bf16 kernel takes
+        key = (tuple(input.shape), tuple(self.weight.shape), input.dtype, ops.get_conv_mode())
+        kind = self.__dict__.get("_po2_kind")
+        if kind is None or kind[0] != key:
+            kind = (key, ops.conv_kernel_kind(input.shape, self.weight.shape, self.stride[0], self.padding[0], self.groups,
+                                              ops.COMPUTE[key[3]], input.dtype))
+            self.__dict__["_po2_kind"] = kind
+        if kind[1] == ops.E_SIZE:
+            return f"input {list(input.shape)} (x and the output must each have fewer than 2^31 elements)"
+        if bf16 and kind[1] < 0:
             return f"bf16 layer {list(self.weight.shape)} groups {self.groups} (no bf16 kernel for this shape)"
         return ""
 
